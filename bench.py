@@ -2,6 +2,7 @@
 """Headline benchmark: enhanced audio-seconds per wall-second of the CRN_ELU streaming path (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--streams B] [--precision fp32|tf32]
+                    [--dump-outputs DIR]
 
 A step advances every concurrent stream by one 3200-sample chunk at hop 1600 (0.1 s of new audio per stream):
 STFT -> features -> preconv/encoder -> GRU -> decoder -> cIRM mask -> iSTFT -> overlap-add, with the per-stream causal
@@ -36,6 +37,7 @@ _REAL_STDOUT = sys.stdout
 METRIC = "enhanced audio-sec/sec (CRN_ELU streaming)"
 UNIT = "audio-s/s"
 RING = 16  # distinct hops of input per stream kept in HBM (input ring 1024*3*27200*4 B = 334 MB > 126 MB L2)
+DUMP_BYTES = 64 << 20  # --dump-outputs keeps a dump at most this large
 
 
 def parse():
@@ -58,7 +60,15 @@ def parse():
     ap.add_argument("--profile-step", action="store_true",
                     help="warm up, then run ONE chunk step inside cudaProfilerStart/Stop (for ncu --profile-from-start off) "
                          "and write the kernel labels of that step to gpurun_out/kernel_labels.json")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned to DIR/enhanced.npy "
+                         "([streams, 1600] float32 enhanced samples), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -157,6 +167,15 @@ def synthetic_signal(n_streams, n_samples):
     gains = 0.5 + 0.5 * synth.uniform01(2021, n_streams, stream=7).astype(np.float32)
     sig *= gains[:, None, None]
     return sig
+
+
+def dump_outputs(path, enhanced):
+    """Writes the enhanced samples of the last timed step as path/enhanced.npy (float32).  Above DUMP_BYTES every k-th
+    stream is kept: a fixed sample, so that the dumps of two builds line up stream for stream."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    stride = -(-enhanced.nbytes // DUMP_BYTES)
+    np.save(os.path.join(path, "enhanced.npy"), np.ascontiguousarray(enhanced[::stride], dtype=np.float32))
 
 
 def build_model(args, max_streams):
@@ -258,8 +277,7 @@ def run_reference(args):
     if rank != 0:
         return
     n = args.cpu_streams
-    steps = min(args.steps, 20)
-    value, ms, steps, kind, cores, what = _cpu_run(args, n, steps=steps, warmup=max(args.warmup, 1))
+    value, ms, steps, kind, cores, what = _cpu_run(args, n, steps=args.steps, warmup=max(args.warmup, 1))
     sample = f"{n} of the {args.streams} streams per step, {steps} steps, fp32 torch CPU ops with {cores} threads: {what}"
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
@@ -354,6 +372,8 @@ def main():
         events[k + 1].record()
     barrier()
     sampler.window[1] = time.time()
+    if args.dump_outputs and rank == 0:  # every rank runs the same streams
+        dump_outputs(args.dump_outputs, out.cpu().numpy())
     total_ms = events[0].elapsed_time(events[K])
     lat = sorted(events[k].elapsed_time(events[k + 1]) for k in range(K))
     clocks = sampler.stop()

@@ -1,5 +1,6 @@
-import sys, numpy as np, torch
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests')
+import os, sys, numpy as np, torch
+REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, REPO); sys.path.insert(0, os.path.join(REPO, "tests"))
 from common import make_model, load_golden, si_sdr_db, rel_err
 from oracle import synth
 for tag in ("crn_small","crn_teacher","crn_student"):

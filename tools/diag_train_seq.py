@@ -1,5 +1,5 @@
 import sys, os, json
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from tools import bench_parts
 dev = torch.device("cuda", 0)
