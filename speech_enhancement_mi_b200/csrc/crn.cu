@@ -242,7 +242,8 @@ struct se_ctx {
     // mma.sync with the stream resident in shared memory (front_mma.cu).  SE_B200_FRONT_MMA=0 / SE_B200_ENC_MMA=0 keep the
     // round-1 kernels (preconv_tc.cu per layer; back-to-back tcgen05 GEMM + separate GlobalLayerNorm pass).
     bool front_mma = true, enc_mma = true;
-    bool enc_tc = true;  // SE_B200_ENC_TC=0: the 16 -> 32 / 32 -> 64 encoder levels on their round-2a kernels (mma.sync / b2b GEMM)
+    int enc_tc = 1;  // SE_B200_ENC_TC=0: the 16 -> 32 / 32 -> 64 encoder levels on their round-2a kernels (mma.sync / b2b GEMM);
+                     // 1: 32 -> 64 on the implicit-GEMM kernel (enc_tc.cu); 2: 16 -> 32 there too
     int bwd_mode = BWD_3XTF32;  // arithmetic of the backward contractions (train_kernels.cu), SE_B200_BWD_MMA
     bool dec_mma = true;  // SE_B200_DEC_MMA=0: small-channel decoder blocks as deconv GEMM + skip-pair kernel + blend kernel
     bool use_tma = true;  // SE_B200_TMA=0: every tcgen05 GEMM keeps the cp.async gather producers
@@ -526,7 +527,7 @@ struct Builder {
         const bool enc_shape = stage == ST_ENCODER && !residual && KF == 5 && KT == 3 && strideF == 2 && dilF == 1 &&
                                Cp_out == Cout_real && in.padF0 == 2 && in.padT0 == 2 * dilT && c->half && !c->train;
         // ... as an implicit GEMM on tcgen05 over the resident input where the channel counts allow it (enc_tc.cu)
-        const bool use_tc = c->enc_tc && enc_shape && enc_tc_supported(Cp_in, Cout_real, in.Tp, in.Fp, Fo);
+        const bool use_tc = enc_shape && enc_tc_supported(c->enc_tc, Cp_in, Cout_real, in.Tp, in.Fp, Fo);
         const bool use_mma = use_tc || (c->enc_mma && enc_shape && enc_mma_supported(Cp_in, Cout_real, in.Tp, in.Fp, Fo));
         const bool fuse_gate = use_mma || (tc_stage(stage) && !c->train &&
                                (Cp_out <= 16 || (c->half && c->b2b_gate && (Cout_real == 32 || Cout_real == 64))));
@@ -1020,7 +1021,8 @@ int build_ctx(se_ctx* c) {
     c->use_tma = c->use_tma && c->half && !c->train;
     if (const char* e = getenv("SE_B200_FRONT_MMA")) c->front_mma = atoi(e) != 0;
     if (const char* e = getenv("SE_B200_ENC_MMA")) c->enc_mma = atoi(e) != 0;
-    if (const char* e = getenv("SE_B200_ENC_TC")) c->enc_tc = atoi(e) != 0;
+    if (const char* e = getenv("SE_B200_ENC_TC")) c->enc_tc = atoi(e);
+    SE_REQUIRE(c->enc_tc >= 0 && c->enc_tc <= 2, "SE_B200_ENC_TC must be 0, 1 or 2");
     c->front_mma = c->front_mma && c->preconv_tc;  // replaces the per-layer tensor-core kernels
     c->enc_mma = c->enc_mma && c->half && !c->train;
     if (const char* e = getenv("SE_B200_DEC_MMA")) c->dec_mma = atoi(e) != 0;

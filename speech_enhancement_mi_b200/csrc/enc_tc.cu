@@ -477,14 +477,14 @@ int launch_enc_tc_t(EncMmaParams p, cudaStream_t st) {
 
 }  // namespace
 
-bool enc_tc_supported(int Cin, int Cout, int Tp, int Fp, int Fo) {
+bool enc_tc_supported(int mode, int Cin, int Cout, int Tp, int Fp, int Fo) {
+    if (mode == 0) return false;
     const int Jp = (Fp + 1) / 2;
     if (Fo > Jp || (Tp - T) % 2 != 0) return false;
     // 16 -> 32 runs too (SE_B200_ENC_TC=2) but only measures 117 us against 122 us for the mma.sync kernel, so it stays
     // there by default.  Measured with -DSE_ENC_PROFILE=1: a no-swizzle A operand is read at ~64 B/clk (65 cycles per
     // K = 16 MMA whatever N <= 64 is, twice the SWIZZLE_128B rate), so the conv phase costs 1,000 (16 ch) / 1,950 (32 ch)
     // cycles per 128-row tile, and the gate phase is paced by the ~900-cycle accumulator round trip per tile.
-    static const int mode = getenv("SE_B200_ENC_TC") ? atoi(getenv("SE_B200_ENC_TC")) : 1;
     if (Cin == 16 && Cout == 32) return mode == 2 && enc_tc_bytes<16, 32>(Tp, Fp) <= 227 * 1024;
     if (Cin == 32 && Cout == 64) return enc_tc_bytes<32, 64>(Tp, Fp) <= 227 * 1024;
     return false;
@@ -492,7 +492,7 @@ bool enc_tc_supported(int Cin, int Cout, int Tp, int Fp, int Fo) {
 
 int launch_enc_tc(const EncMmaParams& p, int Cin, int Cout, cudaStream_t st) {
     if (p.B <= 0) return 0;
-    SE_REQUIRE(enc_tc_supported(Cin, Cout, p.Tp, p.Fp, p.Fo), "enc_tc: unsupported shape");
+    SE_REQUIRE(enc_tc_supported(2, Cin, Cout, p.Tp, p.Fp, p.Fo), "enc_tc: unsupported shape");  // 2: every shape it has
     if (Cin == 16) return launch_enc_tc_t<16, 32>(p, st);
     return launch_enc_tc_t<32, 64>(p, st);
 }

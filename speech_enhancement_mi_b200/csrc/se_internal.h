@@ -260,8 +260,9 @@ struct EncMmaParams {
     const __half *w1c, *w2c;  // enc_tc: conv / gate weights as fp16 UMMA operands in shared-memory order (crn.cu packs them)
 };
 bool enc_mma_supported(int Cin, int Cout, int Tp, int Fp, int Fo);
-// the same block as an implicit GEMM on tcgen05 over the resident input (enc_tc.cu): 16 -> 32 and 32 -> 64 channels
-bool enc_tc_supported(int Cin, int Cout, int Tp, int Fp, int Fo);
+// the same block as an implicit GEMM on tcgen05 over the resident input (enc_tc.cu): 16 -> 32 and 32 -> 64 channels.
+// mode is the context's SE_B200_ENC_TC: 0 never, 1 (default) 32 -> 64 only, 2 also 16 -> 32
+bool enc_tc_supported(int mode, int Cin, int Cout, int Tp, int Fp, int Fo);
 int launch_enc_tc(const EncMmaParams& p, int Cin, int Cout, cudaStream_t st);
 int launch_enc_mma(const EncMmaParams& p, int Cin, int Cout, cudaStream_t st);
 

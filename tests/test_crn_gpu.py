@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from common import CONFIGS, TOL, load_golden, make_model, make_oracle, rel_err, si_sdr_db
+from common import CONFIGS, TOL, load_golden, make_model, make_oracle, oracle_stream_steps, rel_err, si_sdr_db
 from oracle import crn_oracle, synth
 
 pytestmark = pytest.mark.gpu
@@ -235,31 +235,9 @@ def test_full_size_1024_streams_replicas_match_oracle_checked_streams(precision)
     D, B, N = 8, 1024, 4
     mix, _ = synth.make_mixture(D, 1600 * (N + 1))
     chunks = [torch.from_numpy(mix[:, :, 1600 * n:1600 * n + 3200].copy()) for n in range(N)]
-    with torch.no_grad():
-        oracle.reset()
-        state = None
-        want = []
-        on_cut = torch.zeros(D, dtype=torch.bool)
-        for c in chunks:
-            # The reference's phase feature is an UNWRAPPED atan2 (CRN_ELU.py:370-371): a bin on the negative real axis
-            # whose imaginary part is rounding noise (here 1.8e-7 vs -8.5e-8 next to a spectrum peak of 48) gets +pi or
-            # -pi depending on the last bit of the FFT, and the feature jumps by 2 pi.  Both results are valid roundings
-            # of the same signal, but such a stream cannot be compared at the fp32 tolerance: streams whose two spectra
-            # (both within 2e-7 of the peak of each other, asserted) land on different sides of the cut are left out of
-            # the tight check and held to the fp16 tolerance instead.
-            xo = oracle.stft_trans(c)
-            xc = model.stft_trans(c.cuda()).cpu()
-            assert (xo - xc).abs().max() < 1e-6 * xo.abs().max()
-            jump = (torch.atan2(xo[..., 1], xo[..., 0]) - torch.atan2(xc[..., 1], xc[..., 0])).abs() > 3.0
-            on_cut |= jump.flatten(1).any(1)
-            y, state = oracle.stream_step(c, state)
-            want.append(y.numpy())
-    want = np.concatenate(want, axis=-1)
-    keep = (~on_cut).numpy()
-    # at most ONE of the 8 streams may sit on the branch cut (observed: one, stream-dependent on the FFT's last bit); more
-    # would mean the transform itself has drifted, not the cut
-    print(f"streams on the atan2 branch cut (held to the fp16 tolerance): {np.flatnonzero(on_cut.numpy()).tolist()}")
-    assert int(on_cut.sum()) <= 1
+    # streams on the atan2 branch cut of the phase feature are left out of the tight check (common.oracle_stream_steps)
+    want, on_cut = oracle_stream_steps(oracle, chunks, model)
+    keep = ~on_cut
     model.reset()
     small = np.concatenate([model.process_chunk(c.cuda()).cpu().numpy() for c in chunks], axis=-1)
     tol = TOL[precision]
@@ -279,14 +257,18 @@ def test_full_size_1024_streams_replicas_match_oracle_checked_streams(precision)
 @pytest.mark.parametrize("switch,value", [("SE_B200_FRONT_MMA", "0"), ("SE_B200_ENC_MMA", "0"), ("SE_B200_TMA", "0"),
                                           ("SE_B200_DEC_MMA", "0"), ("SE_B200_TMA_PAIR", "0"), ("SE_B200_TMA_PAIR", "2"),
                                           ("SE_B200_GRU_WAVE", "0"), ("SE_B200_GRU_WAVE", "2"), ("SE_B200_ENC_TC", "0"),
-                                          ("SE_B200_ENC_TC", "2")])
+                                          ("SE_B200_ENC_TC", "2"), ("SE_B200_GRU_PERSIST", "0"), ("SE_B200_B2B", "0")])
 def test_fp16_round2_kernel_switches_match_reference(monkeypatch, switch, value):
     """Round-2 kernels against the kernels they replace: the fused pre-convolutions / small-channel encoder and decoder
     blocks (front_mma.cu, back_mma.cu: warp-level mma.sync on SMEM-resident streams), the TMA operand delivery and the
-    CTA-pair mode of the tcgen05 GEMM, the wavefront GRU (gru_wave.cu) and the implicit-GEMM encoder block (enc_tc.cu).
+    CTA-pair mode of the tcgen05 GEMM, the wavefront GRU (gru_wave.cu) and the implicit-GEMM encoder block (enc_tc.cu),
+    plus two earlier fallbacks: the GRU recurrence as one GEMM launch per step instead of a persistent kernel and the
+    32- / 64-channel gates as separate GEMMs instead of the back-to-back one.
     The default path is covered by every other test; here each switch is turned OFF (0) or to its opt-in alternative (2:
     pair mode for every TMA GEMM, the one-layer form of the wavefront kernel, enc_tc for 16 -> 32 channels too) and that
-    path must still meet the fixtures (all three configurations, incl. the carried state of a flag=True continuation)."""
+    path must still meet the fixtures (all three configurations, incl. the carried state of a flag=True continuation).
+    Every switch is read when a context is created, so it takes effect whatever contexts earlier tests built
+    (test_stream_counts_gpu.py counts the enc_tc launches per setting)."""
     monkeypatch.setenv(switch, value)
     for tag in CONFIGS:
         g = load_golden(tag)
@@ -307,8 +289,9 @@ def test_fp16_round2_kernel_switches_match_reference(monkeypatch, switch, value)
 def test_full_size_2048_student_streams_replicas_match_oracle_checked_streams():
     """BASELINE configs[2] per-GPU size (distilled student, 16384 streams over 8 GPUs = 2048 per GPU, fp16 operands): 8
     distinct streams are checked against the oracle over 3 chunk steps, the 2048-stream batch holds 256 shuffled replicas
-    of each and every replica must reproduce its original (all waves of the persistent GRU kernel, all stream-CTAs of the
-    front-end kernels, all tiles of the TMA GEMMs)."""
+    of each and every replica must reproduce its original (all 16 m-tiles of the two-layer wavefront GRU kernel, all
+    stream-CTAs of the front-end kernels, all tiles of the TMA GEMMs).  On a 148-SM B200 the 16 m-tiles fit ONE launch
+    of that kernel; batches that need a second wave are in test_stream_counts_gpu.py."""
     oracle, _ = make_oracle("crn_student")
     model = make_model("crn_student", "fp16")
     D, B, N = 8, 2048, 3
