@@ -86,10 +86,10 @@ struct se_fsn {
     bool weights_bound = false;
     std::map<int, cudaGraphExec_t> graphs;
     cudaStream_t own_stream = nullptr;
-    // scratch of se_fsn_realtime_process (grown on demand; sized by chunks x streams)
+    // scratch of se_fsn_realtime_process (grown on demand; see there for which buffer scales with what)
     float *rt_spec = nullptr, *rt_xin = nullptr, *rt_x0 = nullptr, *rt_crm = nullptr, *rt_s = nullptr, *rt_enh = nullptr,
           *rt_chunks = nullptr, *rt_pline = nullptr, *rt_fbout = nullptr;
-    size_t rt_rows = 0, rt_rows_train = 0;
+    size_t rt_rows = 0, rt_rows_train = 0, rt_xin_rows = 0;
     IoDesc* rt_io = nullptr;
     const float* cur_x = nullptr;  // indirection cell for graph replay
     const float** x_cell = nullptr;
@@ -784,9 +784,17 @@ int se_fsn_realtime_process(se_fsn* c, const float* mixture, const float* source
     const size_t R = (size_t)N * B;
     const size_t per = (size_t)F * T;
     const int Fp = round_up(F, 4), Pp = round_up(F + 2 * c->cfg.sb_num_neighbors, 4);
+    // Scratch, kept across calls.  The buffers of one chunk of every stream (the spectrum rt_spec, and with train=False
+    // the network input rt_xin) scale with the streams B; they are sized for the context's capacity maxB, since a later
+    // call may bring more streams in fewer chunks.  The buffers of every chunk of every stream (rt_x0, rt_crm, rt_s,
+    // rt_enh, rt_chunks; with train=True also rt_xin, rt_pline and rt_fbout) scale with the rows R = N * B and grow with R.
+    if (!c->rt_spec && dev_alloc(c, &c->rt_spec, (size_t)c->maxB * M * per * 2)) return 1;
+    const size_t xin_rows = train ? R : (size_t)B;
+    if (xin_rows > c->rt_xin_rows) {
+        c->rt_xin_rows = xin_rows > (size_t)c->maxB ? xin_rows : (size_t)c->maxB;
+        if (regrow(c, &c->rt_xin, c->rt_xin_rows * 2 * M * per)) return 1;
+    }
     if (R > c->rt_rows) {
-        if (regrow(c, &c->rt_spec, (size_t)B * M * per * 2)) return 1;
-        if (regrow(c, &c->rt_xin, (size_t)B * 2 * M * per)) return 1;
         if (regrow(c, &c->rt_x0, R * 2 * per)) return 1;
         if (regrow(c, &c->rt_crm, R * 2 * per)) return 1;
         if (regrow(c, &c->rt_s, R * 2 * per)) return 1;
@@ -794,10 +802,8 @@ int se_fsn_realtime_process(se_fsn* c, const float* mixture, const float* source
         if (regrow(c, &c->rt_chunks, R * K)) return 1;
         if (!c->rt_io && dev_alloc(c, &c->rt_io, 1)) return 1;
         c->rt_rows = R;
-        c->rt_rows_train = 0;
     }
-    if (train && R > c->rt_rows_train) {  // train=True keeps every chunk's network input and full-band results
-        if (regrow(c, &c->rt_xin, R * 2 * M * per)) return 1;
+    if (train && R > c->rt_rows_train) {  // train=True keeps every chunk's full-band results
         if (regrow(c, &c->rt_pline, R * T * Pp)) return 1;
         if (regrow(c, &c->rt_fbout, R * T * Fp)) return 1;
         c->rt_rows_train = R;

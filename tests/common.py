@@ -34,6 +34,30 @@ TOL = {
 }
 
 
+FSN_SMALL = dict(num_freqs=201, num_mics=3, fb_hidden=64, sb_hidden=32, sb_num_neighbors=15, fb_num_neighbors=0,
+                 num_layers=2)
+FSN_FULL = dict(num_freqs=201, num_mics=3, fb_hidden=512, sb_hidden=384, sb_num_neighbors=15, fb_num_neighbors=0,
+                num_layers=2)
+# FullSubNet against the reference / oracle, tf32 and fp16: max-abs error on mask and waveform relative to the peak, and
+# SI-SDR against the reference waveform
+FSN_TOL_REL, FSN_TOL_DB = 2e-2, 40.0
+
+
+def make_fsn(cfg, seed, **kw):
+    """The product FullSubNet with the deterministic synthetic weights of (cfg, seed) loaded through load_state_dict."""
+    from speech_enhancement_mi_b200 import fullsubnet
+    m = fullsubnet.FullSubNet(
+        num_freqs=cfg["num_freqs"], look_ahead=0, sequence_model="LSTM", fb_num_neighbors=cfg["fb_num_neighbors"],
+        sb_num_neighbors=cfg["sb_num_neighbors"], fb_output_activate_function="ReLU", sb_output_activate_function=False,
+        fb_model_hidden_size=cfg["fb_hidden"], sb_model_hidden_size=cfg["sb_hidden"], num_mics=cfg["num_mics"],
+        num_layers=cfg["num_layers"], weight_init=False, sample_rate=16000, segment_length=3200, win_length=25,
+        hop_length=10, n_fft=400, **kw)
+    w = synth.make_fsn_weights(seed=seed, **cfg)
+    missing, unexpected = m.load_state_dict({k: torch.from_numpy(v) for k, v in w.items()}, strict=True)
+    assert not missing and not unexpected
+    return m.eval()
+
+
 def load_golden(tag):
     z = np.load(os.path.join(GOLDEN, f"{tag}.npz"))
     return {k: z[k] for k in z.files}

@@ -8,36 +8,19 @@ import numpy as np
 import pytest
 import torch
 
-from common import GOLDEN, rel_err, si_sdr_db
+from common import FSN_FULL, FSN_SMALL, FSN_TOL_DB, FSN_TOL_REL, GOLDEN, rel_err, si_sdr_db
+from common import make_fsn as make
 from oracle import synth
 from oracle.fsn_oracle import FSNOracle, unfold
 
 pytestmark = pytest.mark.gpu
 
-FSN_SMALL = dict(num_freqs=201, num_mics=3, fb_hidden=64, sb_hidden=32, sb_num_neighbors=15, fb_num_neighbors=0,
-                 num_layers=2)
-FSN_FULL = dict(num_freqs=201, num_mics=3, fb_hidden=512, sb_hidden=384, sb_num_neighbors=15, fb_num_neighbors=0,
-                num_layers=2)
-TOL_REL, TOL_DB = 2e-2, 40.0
+TOL_REL, TOL_DB = FSN_TOL_REL, FSN_TOL_DB
 
 
 def load(tag):
     z = np.load(os.path.join(GOLDEN, f"{tag}.npz"))
     return {k: z[k] for k in z.files}
-
-
-def make(cfg, seed, **kw):
-    from speech_enhancement_mi_b200 import fullsubnet
-    m = fullsubnet.FullSubNet(
-        num_freqs=cfg["num_freqs"], look_ahead=0, sequence_model="LSTM", fb_num_neighbors=cfg["fb_num_neighbors"],
-        sb_num_neighbors=cfg["sb_num_neighbors"], fb_output_activate_function="ReLU", sb_output_activate_function=False,
-        fb_model_hidden_size=cfg["fb_hidden"], sb_model_hidden_size=cfg["sb_hidden"], num_mics=cfg["num_mics"],
-        num_layers=cfg["num_layers"], weight_init=False, sample_rate=16000, segment_length=3200, win_length=25,
-        hop_length=10, n_fft=400, **kw)
-    w = synth.make_fsn_weights(seed=seed, **cfg)
-    missing, unexpected = m.load_state_dict({k: torch.from_numpy(v) for k, v in w.items()}, strict=True)
-    assert not missing and not unexpected
-    return m.eval()
 
 
 def test_unfold_bit_exact():
@@ -151,33 +134,36 @@ def test_full_config_realtime_process_matches_reference(precision):
     assert si_sdr_db(pred, g["out"]) > TOL_DB
 
 
-@pytest.mark.parametrize("precision", ["tf32", "fp16"])
-def test_partial_state_reset_touches_only_the_given_streams(precision):
+@pytest.mark.parametrize("precision,B,first,count,max_streams",
+                         [("tf32", 4, 1, 2, None), ("fp16", 4, 1, 2, None),
+                          ("tf32", 300, 100, 130, 512), ("fp16", 300, 100, 130, 512)],
+                         ids=["tf32", "fp16", "tf32-B300-of-512", "fp16-B300-of-512"])
+def test_partial_state_reset_touches_only_the_given_streams(precision, B, first, count, max_streams):
     """se_fsn_reset_state(first, count) (fullsubnet.py:826-832 for a sub-range of the streams): the LSTM cell states are
-    stored unit-major ([H][streams x bins], gemm_tc.cu EPI_LSTM), so a stream range is a strided block of every unit row.
-    Streams 1..2 are reset between two calls, streams 0 and 3 continue: the reset streams must reproduce a run from a
-    fully reset model bit for bit, the others the uninterrupted continuation."""
+    stored unit-major ([H][capacity x bins], gemm_tc.cu EPI_LSTM), so a stream range is a strided block of every unit
+    row.  Streams first .. first+count-1 are reset between two calls, the others continue: the reset streams must
+    reproduce a run from a fully reset model bit for bit, the others the uninterrupted continuation.  300 streams on a
+    context of 512: the pitch of the unit rows is the capacity, not the batch."""
     from speech_enhancement_mi_b200._native import check, lib
-    mix1, _ = synth.make_mixture(4, 6400)
-    mix2, _ = synth.make_mixture(4, 6400, first_stream=50)
+    mix1, _ = synth.make_mixture(B, 6400)
+    mix2, _ = synth.make_mixture(B, 6400, first_stream=50)
     x1, x2 = torch.from_numpy(mix1).cuda(), torch.from_numpy(mix2).cuda()
     # fp16 operands need 64-unit tiles (the TMA / CTA-pair path of the LSTM steps): sb_hidden 64 there
     FSN_SMALL = dict(globals()["FSN_SMALL"], sb_hidden=64) if precision == "fp16" else globals()["FSN_SMALL"]
 
-    cont = make(FSN_SMALL, 11, precision=precision)
-    cont.realtime_process(x1, None, flag=False, train=False)
-    y_cont = cont.realtime_process(x2, None, flag=True, train=False).cpu().numpy()
+    def run(between):
+        m = make(FSN_SMALL, 11, precision=precision, max_streams=max_streams)
+        m.realtime_process(x1, None, flag=False, train=False)
+        assert m._ctx_capacity == (max_streams or B)
+        between(m)
+        return m.realtime_process(x2, None, flag=True, train=False).cpu().numpy()
 
-    fresh = make(FSN_SMALL, 11, precision=precision)
-    fresh.realtime_process(x1, None, flag=False, train=False)  # builds the context; state discarded below
-    fresh.reset_state(4)
-    y_fresh = fresh.realtime_process(x2, None, flag=True, train=False).cpu().numpy()
-
-    part = make(FSN_SMALL, 11, precision=precision)
-    part.realtime_process(x1, None, flag=False, train=False)
-    check(lib().se_fsn_reset_state(part._ctx, 1, 2, None), "se_fsn_reset_state")
-    y = part.realtime_process(x2, None, flag=True, train=False).cpu().numpy()
-
-    assert np.array_equal(y[[0, 3]], y_cont[[0, 3]])
-    assert np.array_equal(y[[1, 2]], y_fresh[[1, 2]])
-    assert np.abs(y_cont[1] - y_fresh[1]).max() > 1e-4  # the carried state matters, or this test would prove nothing
+    y_cont = run(lambda m: None)
+    y_fresh = run(lambda m: m.reset_state(B))
+    y = run(lambda m: check(lib().se_fsn_reset_state(m._ctx, first, count, None), "se_fsn_reset_state"))
+    sel = np.zeros(B, dtype=bool)
+    sel[first:first + count] = True
+    assert np.array_equal(y[~sel], y_cont[~sel])
+    assert np.array_equal(y[sel], y_fresh[sel])
+    # the carried state matters for every reset stream, or this test would prove nothing
+    assert np.abs(y_cont[sel] - y_fresh[sel]).max(axis=1).min() > 1e-4
