@@ -31,6 +31,8 @@ extern "C" {
 #define SE_PRECISION_TF32 1 /* tcgen05.mma kind::tf32, fp32 accumulate in TMEM (fast)  */
 #define SE_PRECISION_FP16 2 /* tcgen05.mma kind::f16: GEMM operands (activations between layers, weights) stored as
                                fp16 (same 11-bit significand as tf32), fp32 accumulate, fp32 statistics / state / I/O */
+#define SE_PRECISION_3XTF32 3 /* tcgen05.mma kind::tf32 on split operands (x = tf32 head + tf32 tail, three products
+                                 per step), exact-mode epilogues: fp32-accurate at tensor-core speed */
 
 /* Mirrors the kwargs of CRN_ELU.TemporalCRN.__init__ (CRN_ELU.py:321-323; config.yaml:205-217), with
  * win_length / hop_length already converted from milliseconds to samples (speechbrain STFT: round(sr/1000*ms)). */
@@ -124,9 +126,9 @@ typedef struct se_fsn_config {
     int32_t sb_num_neighbors; /* 15                                    */
     int32_t fb_num_neighbors; /* 0                                     */
     int32_t max_streams;      /* capacity of the per-stream LSTM state */
-    int32_t precision;        /* SE_PRECISION_TF32, or SE_PRECISION_FP16: sub-band LSTM operands (98.7 % of the
-                                 FLOPs) stored as fp16 -- the reference itself runs this model under fp16 autocast
-                                 on CUDA (fullsubnet.py:943) */
+    int32_t precision;        /* SE_PRECISION_TF32, SE_PRECISION_3XTF32 (fp32-accurate products and cells), or
+                                 SE_PRECISION_FP16: sub-band LSTM operands (98.7 % of the FLOPs) stored as fp16 -- the
+                                 reference itself runs this model under fp16 autocast on CUDA (fullsubnet.py:943) */
 } se_fsn_config;
 typedef struct se_fsn se_fsn;
 

@@ -146,7 +146,9 @@ class TemporalCRN(nn.Module):
     """B200-native ``CRN_ELU.TemporalCRN`` (reference CRN_ELU.py:314-535).
 
     Extra keyword arguments (not in the reference, all optional): ``precision`` ("fp32" exact CUDA-core arithmetic,
-    "tf32" tcgen05 tensor cores on fp32 storage, "fp16" tcgen05 tensor cores with fp16 operand storage and fp32 accumulation), ``max_streams`` (capacity of the per-stream state arena; grows on demand),
+    "3xtf32" tcgen05 tensor cores on split fp32 operands (tf32 head + tail, three products) with exact-mode epilogues,
+    accurate to fp32, "tf32" tcgen05 tensor cores on fp32 storage, "fp16" tcgen05 tensor cores with fp16 operand
+    storage and fp32 accumulation), ``max_streams`` (capacity of the per-stream state arena; grows on demand),
     ``device`` (CUDA device index used when tensors arrive on the CPU, as in predict.py:48).
     """
 
@@ -199,8 +201,8 @@ class TemporalCRN(nn.Module):
         # ---- native side -----------------------------------------------------------------------------------
         if precision is None:
             precision = os.environ.get("SE_B200_PRECISION", "fp32")
-        if precision not in ("fp32", "tf32", "fp16"):
-            raise ValueError(f"precision must be 'fp32', 'tf32' or 'fp16', got {precision!r}")
+        if precision not in ("fp32", "3xtf32", "tf32", "fp16"):
+            raise ValueError(f"precision must be 'fp32', '3xtf32', 'tf32' or 'fp16', got {precision!r}")
         self.precision = precision
         self._max_streams = int(max_streams) if max_streams else 0
         self._device_index = device
@@ -241,8 +243,8 @@ class TemporalCRN(nn.Module):
         cfg.win_length = self.win_samples
         cfg.hop_length = self.hop_samples
         cfg.variant = self._variant
-        cfg.precision = {"fp32": _native.SE_PRECISION_FP32, "tf32": _native.SE_PRECISION_TF32,
-                         "fp16": _native.SE_PRECISION_FP16}[self.precision]
+        cfg.precision = {"fp32": _native.SE_PRECISION_FP32, "3xtf32": _native.SE_PRECISION_3XTF32,
+                         "tf32": _native.SE_PRECISION_TF32, "fp16": _native.SE_PRECISION_FP16}[self.precision]
         if training and self.precision == "fp16":
             cfg.precision = _native.SE_PRECISION_TF32  # training keeps fp32 activations (tensor cores on fp32 storage)
         cfg.max_streams = capacity

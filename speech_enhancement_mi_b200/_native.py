@@ -16,6 +16,7 @@ SE_VARIANT_DISTILLED = 1
 SE_PRECISION_FP32 = 0
 SE_PRECISION_TF32 = 1
 SE_PRECISION_FP16 = 2
+SE_PRECISION_3XTF32 = 3
 
 
 class SeCrnConfig(C.Structure):

@@ -220,6 +220,7 @@ struct se_ctx {
     bool use_graph = true;
     bool tf32 = false;  // tensor-core path (tf32 or fp16 operands)
     bool half = false;  // operands of the tensor-core GEMMs are stored as fp16 (SE_PRECISION_FP16)
+    bool split = false;  // tensor-core GEMMs in the 3xTF32 form, exact-mode epilogues (SE_PRECISION_3XTF32)
     int esz = 4;        // element size of the GEMM-operand activations
     int ue = 4;         // elements per 16-byte gather unit
     int kblock = 32;    // elements per k-block
@@ -995,7 +996,8 @@ int build_ctx(se_ctx* c) {
     SE_REQUIRE(g.num_layers == 2, "num_layers must be 2 (config.yaml:210)");
     SE_REQUIRE(g.hidden % 16 == 0 && g.hidden > 0, "hidden must be a positive multiple of 16");
     SE_REQUIRE(g.max_streams > 0, "max_streams must be positive");
-    SE_REQUIRE(g.precision == SE_PRECISION_FP32 || g.precision == SE_PRECISION_TF32 || g.precision == SE_PRECISION_FP16,
+    SE_REQUIRE(g.precision == SE_PRECISION_FP32 || g.precision == SE_PRECISION_TF32 || g.precision == SE_PRECISION_FP16 ||
+                   g.precision == SE_PRECISION_3XTF32,
                "unknown precision");
     SE_REQUIRE(g.variant == SE_VARIANT_CRN_ELU || g.variant == SE_VARIANT_DISTILLED, "unknown variant");
     c->maxB = g.max_streams;
@@ -1005,8 +1007,9 @@ int build_ctx(se_ctx* c) {
     c->H = g.hidden;
     c->tf32 = g.precision != SE_PRECISION_FP32;
     c->half = g.precision == SE_PRECISION_FP16;
+    c->split = g.precision == SE_PRECISION_3XTF32;
     c->train = g.training != 0;
-    SE_REQUIRE(!(c->train && c->half), "training keeps fp32 activations: use precision fp32 or tf32");
+    SE_REQUIRE(!(c->train && c->half), "training keeps fp32 activations: use precision fp32, 3xtf32 or tf32");
     c->esz = c->half ? 2 : 4;
     c->ue = 16 / c->esz;
     c->kblock = 128 / c->esz;
@@ -1027,9 +1030,9 @@ int build_ctx(se_ctx* c) {
     c->enc_mma = c->enc_mma && c->half && !c->train;
     if (const char* e = getenv("SE_B200_DEC_MMA")) c->dec_mma = atoi(e) != 0;
     c->dec_mma = c->dec_mma && c->half && !c->train;
-    // backward contractions of the training step: fp32-accurate 3xTF32 beside the exact forward, one tf32 pass beside
-    // the tf32 forward; SE_B200_BWD_MMA=0 keeps them on the CUDA cores (1 / 2 force a tensor-core form)
-    c->bwd_mode = c->tf32 ? BWD_TF32 : BWD_3XTF32;
+    // backward contractions of the training step: fp32-accurate 3xTF32 beside the exact and the 3xTF32 forward, one
+    // tf32 pass beside the tf32 forward; SE_B200_BWD_MMA=0 keeps them on the CUDA cores (1 / 2 force a tensor-core form)
+    c->bwd_mode = c->tf32 && !c->split ? BWD_TF32 : BWD_3XTF32;
     if (const char* e = getenv("SE_B200_BWD_MMA")) c->bwd_mode = atoi(e);
     SE_REQUIRE(c->bwd_mode >= 0 && c->bwd_mode <= 2, "SE_B200_BWD_MMA must be 0, 1 or 2");
     if (const char* e = getenv("SE_B200_GRU_PIPE")) c->gru_pipe = atoi(e);
@@ -1832,8 +1835,9 @@ int run_gemm(const se_ctx* c, const GemmParams& g, int stage, const std::string&
     return 0;
 }
 int run_gemm_impl(const se_ctx* c, const GemmParams& g, int stage, const std::string& label, cudaStream_t st) {
-    if (g.epi == EPI_GRU || g.epi == EPI_ELU_GATE) return launch_gemm_tf32(g, st);
-    if (c->tf32 && (c->half || ((c->tc_mask >> stage) & 1u)) && gemm_tf32_supported(g)) return launch_gemm_tf32(g, st);
+    if (g.epi == EPI_GRU || g.epi == EPI_ELU_GATE) return launch_gemm_tf32(g, st, c->split);
+    if (c->tf32 && (c->half || ((c->tc_mask >> stage) & 1u)) && gemm_tf32_supported(g))
+        return launch_gemm_tf32(g, st, c->split);
     SE_REQUIRE(!c->half, "internal: fp16 operands need the tensor-core GEMM (" + label + ")");
     return launch_gemm_fp32(g, st);
 }
@@ -1984,7 +1988,7 @@ int enqueue_stream_step(se_ctx* c, int B, cudaStream_t st, int stage_filter = -1
         mp.b = c->b_last;
         mp.noisy = c->noisy;
         mp.carry = c->carry;
-        mp.fast = (c->half || c->tf32) ? 1 : 0;
+        mp.fast = (c->half || c->tf32) && !c->split ? 1 : 0;  // 3xtf32 keeps the exact cIRM decompression
         if (launch_mask_istft(mp, st)) return 1;
     }
     if (want(ST_ROLL)) {
@@ -2148,7 +2152,7 @@ int train_forward(se_ctx* c, const float* mixture, int nb, long long L, int flag
                 const bool tc = c->tf32 && ((c->tc_mask >> proj.stage) & 1u) && gemm_tf32_supported(g);
                 if (tc) {
                     g.b0 = s0;
-                    if (launch_gemm_tf32(g, c->pipe_stream)) return 1;
+                    if (launch_gemm_tf32(g, c->pipe_stream, c->split)) return 1;
                 } else {
                     g.A = reinterpret_cast<const float*>(g.A) + (long long)s0 * g.sB;
                     g.out += (long long)s0 * g.oB;

@@ -69,6 +69,7 @@ struct se_fsn {
     // SE_PRECISION_FP16: the sub-band records (x_t and the h histories, 98.7 % of the FLOPs read them) and the sub-band
     // weights are stored as fp16 (tcgen05 kind::f16, fp32 accumulate; cell state c and all statistics stay fp32)
     bool half = false;
+    bool split = false;  // SE_PRECISION_3XTF32: every GEMM in the 3xTF32 form (fp32-accurate products, exact cells)
     bool wide_tiles = true;  // 256-column LSTM tiles where the hidden size allows (SE_B200_FSN_WIDE=0: 128-column tiles)
     int sesz = 4;   // element size of the sub-band records
     int Ksp = 0;    // sub-band input size padded to whole k-blocks (32 floats / 64 halves)
@@ -330,7 +331,8 @@ void build_lstm(se_fsn* c, const std::string& prefix, int layer, int Kin, int Ki
                 bool half = false) {
     const int U = half ? 8 : 4;    // elements per 16-byte gather unit
     const int esz = half ? 2 : 4;
-    const int U_tile = (H % 64 == 0 && c->wide_tiles) ? 64 : 32;  // hidden units per output tile
+    // hidden units per output tile (the 3xTF32 form has 128-column tiles: 32 units)
+    const int U_tile = (H % 64 == 0 && c->wide_tiles && !c->split) ? 64 : 32;
     const int K = Kin_pad + H;
     const int N = 4 * H;
     const size_t w_off = c->reserve_w((size_t)N * K), b_off = c->reserve_w(N);
@@ -441,9 +443,10 @@ int build(se_fsn* c) {
     c->NB = 2 * g.sb_num_neighbors + 1;
     c->Ks = c->NB + 1;
     c->Kf = round_up(c->F * c->M, 32) ;  // whole k-blocks, so that [x | h] stays k-block aligned
-    SE_REQUIRE(g.precision == SE_PRECISION_TF32 || g.precision == SE_PRECISION_FP16,
-               "FullSubNet: precision must be SE_PRECISION_TF32 or SE_PRECISION_FP16");
+    SE_REQUIRE(g.precision == SE_PRECISION_TF32 || g.precision == SE_PRECISION_FP16 || g.precision == SE_PRECISION_3XTF32,
+               "FullSubNet: precision must be SE_PRECISION_TF32, SE_PRECISION_3XTF32 or SE_PRECISION_FP16");
     c->half = g.precision == SE_PRECISION_FP16;
+    c->split = g.precision == SE_PRECISION_3XTF32;
     if (const char* e = getenv("SE_B200_FSN_WIDE")) c->wide_tiles = atoi(e) != 0;
     c->sesz = c->half ? 2 : 4;
     SE_REQUIRE(round_up(c->Ks, 32) == c->Ks, "FullSubNet: sub-band input size must be a multiple of 32 (31 neighbours + 1)");
@@ -536,7 +539,7 @@ int run_gemm(se_fsn* c, int i, int B, cudaStream_t st) {
     GemmParams g = c->gemms[i];
     g.M = B * c->g_rows[i];
     if (c->g_tma_ok[i]) return launch_gemm_tma(g, c->g_tma[i], st);
-    return launch_gemm_tf32(g, st);
+    return launch_gemm_tf32(g, st, c->split);
 }
 
 // The chunk step in four phases.  whole = 0: the streaming chunk step (fullsubnet.py:932-945), both CumLayerNorms advance
@@ -567,7 +570,7 @@ int phase_fullband(se_fsn* c, int B, cudaStream_t st) {  // scale, reflect-padde
         g.M = B * c->g_rows[gi];
         g.stats = c->sums + 2;
         g.stats_stride = 4;  // sums holds 4 doubles per stream
-        if (launch_gemm_tf32(g, st)) return 1;
+        if (launch_gemm_tf32(g, st, c->split)) return 1;
     }
     fsn_roll_kernel<float><<<dim3(B, (c->Hf + 255) / 256), 256, 0, st>>>(c->fbrec, c->recF, c->f_h0, c->f_h1, c->Hf);
     SE_CUDA_OK(cudaGetLastError());

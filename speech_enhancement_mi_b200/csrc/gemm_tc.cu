@@ -227,6 +227,40 @@ __device__ __forceinline__ float fast_tanh(float x) {
 }
 __device__ __forceinline__ float fast_sigmoid(float x) { return fmaf(0.5f, fast_tanh(0.5f * x), 0.5f); }
 __device__ __forceinline__ float fast_elu(float x) { return x > 0.f ? x : ex2_ftz(1.4426950408889634f * x) - 1.0f; }
+// Epilogue math by form: X = true (3xTF32 split form, fp32-accurate products) keeps the exact-mode functions of
+// gemm_fp32.cu -- the MUFU versions above are accurate to 2^-11 only and would bound the whole result there.
+template <bool X>
+__device__ __forceinline__ float epi_sigmoid(float x) { return X ? 1.f / (1.f + expf(-x)) : fast_sigmoid(x); }
+template <bool X>
+__device__ __forceinline__ float epi_tanh(float x) { return X ? tanhf(x) : fast_tanh(x); }
+template <bool X>
+__device__ __forceinline__ float epi_elu(float x) { return X ? (x > 0.f ? x : expm1f(x)) : fast_elu(x); }
+
+// 3xTF32 operand split: x = hi + lo with hi = tf32(x), lo = tf32(x - hi) (|x - hi - lo| <= 2^-22 |x|).  Both halves are
+// written as tf32 values (low 13 mantissa bits zero), so the products do not depend on how the tensor core reads the
+// low bits of an fp32 word.
+__device__ __forceinline__ uint32_t to_tf32(float x) {
+    uint32_t r;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+    return r;
+}
+__device__ __forceinline__ void split16(unsigned char* head, unsigned char* tail) {  // one 16-byte chunk in place
+    const float4 v = *reinterpret_cast<const float4*>(head);
+    uint4 h, l;
+    h.x = to_tf32(v.x);
+    h.y = to_tf32(v.y);
+    h.z = to_tf32(v.z);
+    h.w = to_tf32(v.w);
+    l.x = to_tf32(v.x - __uint_as_float(h.x));
+    l.y = to_tf32(v.y - __uint_as_float(h.y));
+    l.z = to_tf32(v.z - __uint_as_float(h.z));
+    l.w = to_tf32(v.w - __uint_as_float(h.w));
+    *reinterpret_cast<uint4*>(head) = h;
+    *reinterpret_cast<uint4*>(tail) = l;
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // per-stream (sum, sum of squares) of the rows a warp owns: rows are ordered by stream, so the warp holds a short
 // monotone run of stream indices; one shuffle reduction and one pair of double atomics per distinct stream
@@ -272,24 +306,33 @@ constexpr int kW2Floats = 32 * 16 + 32;  // fused small gate: W2 [2*C2][16] + bi
 // TMA: 0 = cp.async gather producers, 1 = TMA tile loads, 2 = TMA + CTA pair (cta_group::2: the two CTAs of a cluster run
 // one M256 x BN MMA; each holds its own 128 rows of A and HALF of the weight tile, which halves the shared-memory reads of
 // the tensor core and the fill traffic per SM -- these GEMMs run at the shared-memory bandwidth of their operand tiles)
-template <int BN, bool B2B = (BN == 16), int TMA = 0>
+// SPLIT: the 3xTF32 form (gemm_tc3x_kernel; gathered fp32 operands only).  A stage holds two operand planes, the tf32
+// heads and the tf32 tails, so it is twice the size of a tf32 stage: the tile is capped at BN = 128 (two 64 KB stages
+// beside the 72 KB of epilogue staging) and the narrower tiles get their own stage counts.
+template <int BN, bool B2B = (BN == 16), int TMA = 0, bool SPLIT = false>
 struct Cfg {
-    static constexpr int NACC = (BN > 128 || (B2B && BN > 16)) ? 2 : 4;  // TMEM accumulators = epilogue groups
-    static constexpr int STAGES = TMA == 2 ? (BN > 128 ? 4 : (BN > 64 ? 5 : 6))
-                                           : (BN > 128 ? 3 : (BN > 32 ? 4 : (B2B ? 4 : 6)));  // B2B: room for the gate tiles
+    // TMEM accumulators = epilogue groups.  Split form at BN = 128: 2 groups, so that the 13 warps get 128 registers
+    // each (21 warps get 80, and the exact-mode LSTM cell spills at 80)
+    static constexpr int NACC = (BN > 128 || (B2B && BN > 16) || (SPLIT && BN == 128)) ? 2 : 4;
+    static constexpr int STAGES = SPLIT      ? (BN > 64 ? 2 : (BN > 16 ? 3 : 4))
+                                  : TMA == 2 ? (BN > 128 ? 4 : (BN > 64 ? 5 : 6))
+                                             : (BN > 128 ? 3 : (BN > 32 ? 4 : (B2B ? 4 : 6)));  // B2B: room for the gate tiles
     static constexpr int WARPS = kFirstEpiWarp + 4 * NACC;
     static constexpr int THREADS = WARPS * 32;
     // back-to-back gate (BN == 16, fp16 operands): a second accumulator of 32 columns per group, the ELU tile as an
-    // fp16 A operand (128 rows x 128 B) per group and the 32 x 16 gate weights as a B operand (4 KB)
-    static constexpr int GATE_COLS = B2B ? 2 * BN : 0;
-    static constexpr int ETILE_BYTES = B2B ? NACC * BM * BKB : 0;
-    static constexpr int W2T_BYTES = B2B ? 2 * BN * BKB : 0;
+    // fp16 A operand (128 rows x 128 B) per group and the 32 x 16 gate weights as a B operand (4 KB); the split form
+    // (fp32 operands) keeps the register version of the gate and needs none of them
+    static constexpr bool TC_GATE = B2B && !SPLIT;
+    static constexpr int GATE_COLS = TC_GATE ? 2 * BN : 0;
+    static constexpr int ETILE_BYTES = TC_GATE ? NACC * BM * BKB : 0;
+    static constexpr int W2T_BYTES = TC_GATE ? 2 * BN * BKB : 0;
     static constexpr int TMEM_COLS_RAW = NACC * (BN + GATE_COLS);
     static constexpr uint32_t TMEM_COLS =
         TMEM_COLS_RAW <= 32 ? 32
                             : (TMEM_COLS_RAW <= 64 ? 64 : (TMEM_COLS_RAW <= 128 ? 128 : (TMEM_COLS_RAW <= 256 ? 256 : 512)));
     static constexpr int B_STAGE_BYTES = (TMA == 2 ? BN / 2 : BN) * BKB;
-    static constexpr int STAGE_BYTES = A_STAGE_BYTES + B_STAGE_BYTES;
+    static constexpr int PLANE_BYTES = A_STAGE_BYTES + B_STAGE_BYTES;  // one operand plane: A tile, then W tile
+    static constexpr int STAGE_BYTES = (SPLIT ? 2 : 1) * PLANE_BYTES;     // split: heads, then tails
     static constexpr int TILE_BYTES = STAGES * STAGE_BYTES;
     static constexpr int KOFF_MAX = 512;  // K <= 2048
     static constexpr int OFF_ETILE = TILE_BYTES;               // 1024-aligned (SWIZZLE_128B atoms)
@@ -306,6 +349,7 @@ struct Cfg {
     static_assert(TMEM_COLS_RAW <= 512, "TMEM has 512 columns");
     static_assert(OFF_STG % 16 == 0 && OFF_BIAS % 16 == 0 && OFF_W2 % 16 == 0, "float4 alignment");
     static_assert(BYTES <= 227 * 1024, "shared memory budget");
+    static_assert(!SPLIT || (TMA == 0 && BN <= 128), "the split form gathers fp32 operands into tiles of <= 128 columns");
 };
 
 // coalesced write-out of a staged chunk: W columns (8, 16 or 32) of the warp's 32 rows; consecutive lanes write
@@ -375,7 +419,7 @@ __device__ __forceinline__ void store_chunk(const float* stg, int col0, float* o
 }
 
 // gated 1x1 pair in registers (CRN_ELU.py:240): y[c] = (W2[2c].e + b2[2c]) * sigmoid(W2[2c+1].e + b2[2c+1]), c < C2
-template <int KC>
+template <int KC, bool X>
 __device__ __forceinline__ void small_gate(const float* s_w2, const float* e, int C2, float* y) {
     const float* b2 = s_w2 + 32 * 16;
 #pragma unroll
@@ -392,18 +436,19 @@ __device__ __forceinline__ void small_gate(const float* s_w2, const float* e, in
                 a += x.x * e[4 * q] + x.y * e[4 * q + 1] + x.z * e[4 * q + 2] + x.w * e[4 * q + 3];
                 gt += z.x * e[4 * q] + z.y * e[4 * q + 1] + z.z * e[4 * q + 2] + z.w * e[4 * q + 3];
             }
-            a *= fast_sigmoid(gt);
+            a *= epi_sigmoid<X>(gt);
         }
         y[c] = a;
     }
 }
 
-template <int BN, typename AT, bool B2B = (BN == 16), int TMA = 0>
-__global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
-    gemm_tc_kernel(const GemmParams p, const __grid_constant__ GemmTma tm) {
+// The kernel body of both forms (gemm_tc_kernel, gemm_tc3x_kernel below)
+template <int BN, typename AT, bool B2B, int TMA, bool SPLIT>
+__device__ __forceinline__ void gemm_tc_body(const GemmParams& p, const GemmTma& tm) {
     constexpr int BKE = BKB / (int)sizeof(AT);  // elements per k-block
     constexpr int UE = 16 / (int)sizeof(AT);    // elements per 16-byte gather unit
-    using S = Cfg<BN, B2B, TMA>;
+    using S = Cfg<BN, B2B, TMA, SPLIT>;
+    static_assert(!SPLIT || sizeof(AT) == 4, "the split form reads fp32 operands");
     constexpr int STAGES = S::STAGES;
     constexpr int NACC = S::NACC;
     constexpr bool PAIR = TMA == 2;
@@ -558,6 +603,19 @@ __global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
         const uint32_t dst_gj = (uint32_t)((g >> 3) * 1024 + (g & 7) * 128 + ((j ^ (g & 7)) << 4));
         constexpr int B_ITERS = BN / 16;
         uint32_t ps = 0, pphase = 0;  // stage ring position / phase (the ring runs on across tiles)
+        // split form: this thread's chunks of stage s, once landed, become tf32 heads in place and tf32 tails in the
+        // stage's second plane; then the stage is handed to the tensor core through the async proxy
+        int split_ps = -1;  // stage whose loads are in flight and not split yet
+        auto split_stage = [&](int s) {
+            unsigned char* base = tiles_ptr + s * S::STAGE_BYTES + dst_gj;
+#pragma unroll
+            for (int i = 0; i < BM / 16; ++i) split16(base + i * 2048, base + S::PLANE_BYTES + i * 2048);
+#pragma unroll
+            for (int i = 0; i < B_ITERS; ++i)
+                split16(base + A_STAGE_BYTES + i * 2048, base + S::PLANE_BYTES + A_STAGE_BYTES + i * 2048);
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            mbar_arrive(full_bar(s));
+        };
         const int q16 = 16 / p.Fo, r16 = 16 % p.Fo;
         for (int tile = tfirst; tile < ntiles; tile += tstep) {
             const int m0 = (tile / ntn) * BM;
@@ -610,12 +668,26 @@ __global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
                     wp += wstep;
                 }
                 wptr += BKE;
-                cp_async_mbar_arrive_noinc(full_bar(ps));
+                if (SPLIT) {
+                    // one k-block behind: the previous stage's chunks have landed while this one's loads are in flight
+                    cp_async_commit();
+                    if (split_ps >= 0) {
+                        cp_async_wait<1>();
+                        split_stage(split_ps);
+                    }
+                    split_ps = (int)ps;
+                } else {
+                    cp_async_mbar_arrive_noinc(full_bar(ps));
+                }
                 if (++ps == STAGES) {
                     ps = 0;
                     pphase ^= 1u;
                 }
             }
+        }
+        if (SPLIT && split_ps >= 0) {
+            cp_async_wait<0>();
+            split_stage(split_ps);
         }
     } else if (warp_u == 4) {
         // ============================ MMA issuer ============================
@@ -648,13 +720,22 @@ __global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
                     tc_fence_after();
                     const uint64_t adesc = make_desc(tiles + ms * (uint32_t)S::STAGE_BYTES);
                     const uint64_t bdesc = adesc + (uint64_t)(A_STAGE_BYTES >> 4);
+                    constexpr uint64_t tail = (uint64_t)(S::PLANE_BYTES >> 4);  // split: heads -> tails plane
                     if (elect_one()) {
 #pragma unroll
                         for (int kk = 0; kk < 4; ++kk) {
                             // one MMA consumes 32 bytes of K (8 tf32 / 16 fp16): +2 in the (addr >> 4) field of the atom
                             const uint32_t a1 = kk ? 1u : acc;
-                            if (PAIR) tc_mma_f16_pair(tacc, adesc + (uint64_t)(2 * kk), bdesc + (uint64_t)(2 * kk), idesc_pair, a1);
-                            else tc_mma<AT>(tacc, adesc + (uint64_t)(2 * kk), bdesc + (uint64_t)(2 * kk), idesc, a1);
+                            const uint64_t ad = adesc + (uint64_t)(2 * kk), bd = bdesc + (uint64_t)(2 * kk);
+                            if (PAIR) {
+                                tc_mma_f16_pair(tacc, ad, bd, idesc_pair, a1);
+                            } else if (SPLIT) {  // small terms first: lo.hi + hi.lo, then hi.hi
+                                tc_mma<AT>(tacc, ad + tail, bd, idesc, a1);
+                                tc_mma<AT>(tacc, ad, bd + tail, idesc, 1u);
+                                tc_mma<AT>(tacc, ad, bd, idesc, 1u);
+                            } else {
+                                tc_mma<AT>(tacc, ad, bd, idesc, a1);
+                            }
                         }
                         if (PAIR) tc_commit_pair(empty_bar(ms), 3);  // the stage is free in BOTH CTAs
                         else tc_commit(empty_bar(ms));
@@ -787,9 +868,9 @@ __global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
                     const int mm = m0 + q * 32 + r;
                     if (mm < p.M) {
                         const float* sr = stg + r * SPW;
-                        const float rg = fast_sigmoid(pr[i] + sr[ul] + br);
-                        const float zg = fast_sigmoid(pz[i] + sr[8 + ul] + bz);
-                        const float ng = fast_tanh(pn[i] + rg * (sr[16 + ul] + bn));
+                        const float rg = epi_sigmoid<SPLIT>(pr[i] + sr[ul] + br);
+                        const float zg = epi_sigmoid<SPLIT>(pz[i] + sr[8 + ul] + bz);
+                        const float ng = epi_tanh<SPLIT>(pn[i] + rg * (sr[16 + ul] + bn));
                         const float hn = (1.0f - zg) * ng + zg * ph[i];
                         p.out[(p.b0 + mm) * p.oB + ju] = hn;
                         // fp16 copy = operand of the next step / the next layer's projection
@@ -861,12 +942,12 @@ __global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
                     float cn[8], hv[8];
 #pragma unroll
                     for (int k = 0; k < 8; ++k) {
-                        const float ig = fast_sigmoid(__uint_as_float(v[k]) + sbias[u0 + k]);
-                        const float fg = fast_sigmoid(__uint_as_float(v[8 + k]) + sbias[U + u0 + k]);
-                        const float gg = fast_tanh(__uint_as_float(v[16 + k]) + sbias[2 * U + u0 + k]);
-                        const float og = fast_sigmoid(__uint_as_float(v[24 + k]) + sbias[3 * U + u0 + k]);
+                        const float ig = epi_sigmoid<SPLIT>(__uint_as_float(v[k]) + sbias[u0 + k]);
+                        const float fg = epi_sigmoid<SPLIT>(__uint_as_float(v[8 + k]) + sbias[U + u0 + k]);
+                        const float gg = epi_tanh<SPLIT>(__uint_as_float(v[16 + k]) + sbias[2 * U + u0 + k]);
+                        const float og = epi_sigmoid<SPLIT>(__uint_as_float(v[24 + k]) + sbias[3 * U + u0 + k]);
                         cn[k] = fmaf(fg, pc[k], ig * gg);
-                        hv[k] = og * fast_tanh(cn[k]);
+                        hv[k] = og * epi_tanh<SPLIT>(cn[k]);
                     }
                     if (ok && crs) {
 #pragma unroll
@@ -992,9 +1073,9 @@ __global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
                 tc_fence_before();
                 mbar_arrive(tempty_bar(acc));
 #pragma unroll
-                for (int i = 0; i < 16; ++i) e[i] = fast_elu(__uint_as_float(vr[i]) + sbias[i]);
-                if (p.C2 <= 8) small_gate<8>(s_w2, e, p.C2, y);
-                else small_gate<16>(s_w2, e, p.C2, y);
+                for (int i = 0; i < 16; ++i) e[i] = epi_elu<SPLIT>(__uint_as_float(vr[i]) + sbias[i]);
+                if (p.C2 <= 8) small_gate<8, SPLIT>(s_w2, e, p.C2, y);
+                else small_gate<16, SPLIT>(s_w2, e, p.C2, y);
                 if (row_ok) {
 #pragma unroll
                     for (int i = 0; i < 16; ++i) {
@@ -1038,7 +1119,7 @@ __global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
                             for (int i = 0; i < CH; ++i) v[i] = fmaxf(v[i], 0.f);
                         } else if (p.epi != EPI_BIAS) {
 #pragma unroll
-                            for (int i = 0; i < CH; ++i) v[i] = fast_elu(v[i]);
+                            for (int i = 0; i < CH; ++i) v[i] = epi_elu<SPLIT>(v[i]);
                         }
 #pragma unroll
                         for (int i = 0; i < CH; i += 4)
@@ -1068,15 +1149,15 @@ __global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
                         float w[CO];
                         if (p.epi == EPI_GATE_STATS) {
 #pragma unroll
-                            for (int i = 0; i < CO; ++i) w[i] = v[2 * i] * fast_sigmoid(v[2 * i + 1]);
+                            for (int i = 0; i < CO; ++i) w[i] = v[2 * i] * epi_sigmoid<SPLIT>(v[2 * i + 1]);
                         } else {
 #pragma unroll
                             for (int i = 0; i < CO; ++i) w[i] = v[2 * i];
 #pragma unroll
                             for (int i = 0; i < CO; i += 4)
                                 *reinterpret_cast<float4*>(srow + CO + i) =
-                                    make_float4(fast_elu(v[2 * i + 1]), fast_elu(v[2 * i + 3]), fast_elu(v[2 * i + 5]),
-                                                fast_elu(v[2 * i + 7]));
+                                    make_float4(epi_elu<SPLIT>(v[2 * i + 1]), epi_elu<SPLIT>(v[2 * i + 3]),
+                                                epi_elu<SPLIT>(v[2 * i + 5]), epi_elu<SPLIT>(v[2 * i + 7]));
                         }
 #pragma unroll
                         for (int i = 0; i < CO; i += 4)
@@ -1122,16 +1203,33 @@ __global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
     }
 }
 
-template <int BN, typename AT, bool B2B = (BN == 16)>
+template <int BN, typename AT, bool B2B = (BN == 16), int TMA = 0>
+__global__ void __launch_bounds__(Cfg<BN, B2B, TMA>::THREADS, 1)
+    gemm_tc_kernel(const GemmParams p, const __grid_constant__ GemmTma tm) {
+    gemm_tc_body<BN, AT, B2B, TMA, false>(p, tm);
+}
+// 3xTF32 form: gathered fp32 operands split into tf32 heads and tails, three MMAs per K = 8 step, exact-mode epilogues
+template <int BN, bool B2B = (BN == 16)>
+__global__ void __launch_bounds__(Cfg<BN, B2B, 0, true>::THREADS, 1)
+    gemm_tc3x_kernel(const GemmParams p, const __grid_constant__ GemmTma tm) {
+    gemm_tc_body<BN, float, B2B, 0, true>(p, tm);
+}
+
+template <int BN, typename AT, bool B2B = (BN == 16), bool SPLIT = false>
 int launch_tc(const GemmParams& p, cudaStream_t st) {
-    using S = Cfg<BN, B2B>;
-    SE_DYN_SMEM((gemm_tc_kernel<BN, AT, B2B, 0>), S::BYTES);
+    using S = Cfg<BN, B2B, 0, SPLIT>;
     int g_num_sms = 0;
     if (num_sms_current_device(&g_num_sms)) return 1;
     const int ntiles = ((p.M + BM - 1) / BM) * ((p.epi == EPI_GRU ? p.N : p.Npad) / BN);
     const int grid = ntiles < g_num_sms ? ntiles : g_num_sms;  // persistent: one CTA per SM
     static const GemmTma no_tma{};
-    gemm_tc_kernel<BN, AT, B2B, 0><<<grid, S::THREADS, S::BYTES, st>>>(p, no_tma);
+    if constexpr (SPLIT) {
+        SE_DYN_SMEM((gemm_tc3x_kernel<BN, B2B>), S::BYTES);
+        gemm_tc3x_kernel<BN, B2B><<<grid, S::THREADS, S::BYTES, st>>>(p, no_tma);
+    } else {
+        SE_DYN_SMEM((gemm_tc_kernel<BN, AT, B2B, 0>), S::BYTES);
+        gemm_tc_kernel<BN, AT, B2B, 0><<<grid, S::THREADS, S::BYTES, st>>>(p, no_tma);
+    }
     SE_CUDA_OK(cudaGetLastError());
     return 0;
 }
@@ -1178,6 +1276,21 @@ int launch_tc_tma(const GemmParams& p, const GemmTma& tm_in, cudaStream_t st) {
     cfg.numAttrs = 1;
     SE_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, __half, false, 2>, p, tm));
     return 0;
+}
+
+// split form: fp32 operands; tiles of at most 128 columns (a 256-column GEMM runs as twice as many 128-column tiles,
+// an LSTM on 32-unit tiles)
+int launch_split(const GemmParams& p, cudaStream_t st) {
+    SE_REQUIRE(!p.a_half, "gemm_tc: the 3xTF32 form reads fp32 operands");
+    SE_REQUIRE(p.epi != EPI_LSTM || p.lstm_units != 64, "gemm_tc: the 3xTF32 form runs LSTM steps on 32-unit tiles");
+    if (p.epi == EPI_GRU) return launch_tc<96, float, false, true>(p, st);
+    if (p.epi == EPI_LSTM) return launch_tc<128, float, false, true>(p, st);
+    switch (gemm_tf32_tile_n(p.N)) {
+        case 16: return launch_tc<16, float, true, true>(p, st);
+        case 32: return launch_tc<32, float, false, true>(p, st);
+        case 64: return launch_tc<64, float, false, true>(p, st);
+        default: return launch_tc<128, float, false, true>(p, st);
+    }
 }
 
 template <typename AT>
@@ -1362,9 +1475,10 @@ int gemm_tf32_tile_n(int N) {
     return 256;
 }
 
-int launch_gemm_tf32(const GemmParams& p, cudaStream_t st) {
+int launch_gemm_tf32(const GemmParams& p, cudaStream_t st, bool split) {
     SE_REQUIRE(gemm_tf32_supported(p), "gemm_tc: unsupported shape");
     if (p.M <= 0) return 0;
+    if (split) return launch_split(p, st);
     return p.a_half ? launch_elem<__half>(p, st) : launch_elem<float>(p, st);
 }
 

@@ -145,7 +145,9 @@ bool gemm_tma_supported(const GemmParams& p);
 int gemm_profile_read(unsigned long long* out8, int reset);  // diagnostic cycle counters of the TMA GEMM roles
 
 int launch_gemm_fp32(const GemmParams& p, cudaStream_t st);
-int launch_gemm_tf32(const GemmParams& p, cudaStream_t st);  // tcgen05 path (gemm_tc.cu)
+// tcgen05 path (gemm_tc.cu); split: the 3xTF32 form (fp32 operands as tf32 head + tail, fp32-accurate products and
+// exact-mode epilogues: SE_PRECISION_3XTF32)
+int launch_gemm_tf32(const GemmParams& p, cudaStream_t st, bool split);
 bool gemm_tf32_supported(const GemmParams& p);
 int gemm_tf32_tile_n(int N);  // output-tile width (BN) the tcgen05 kernel uses for N logical columns
 int gemm_tma_tile_n(const GemmParams& p);  // ... and the TMA path for this GEMM (may split 256-column tiles)

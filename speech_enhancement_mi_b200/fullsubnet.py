@@ -73,12 +73,13 @@ class FullSubNet(BaseModel):
                  sample_rate=16000, segment_length=400, win_length=20, hop_length=10, n_fft=320, max_streams=None,
                  device=None, precision=None):
         super().__init__()
-        # extra (not in the reference): "tf32" = tcgen05 on fp32 storage; "fp16" = sub-band LSTM operands stored as
-        # fp16 with fp32 accumulation / cell state -- the reference runs this model under fp16 autocast on CUDA
-        # (fullsubnet.py:943)
+        # extra (not in the reference): "tf32" = tcgen05 on fp32 storage; "3xtf32" = tcgen05 on split fp32 operands
+        # (tf32 head + tail, three products) with exact-mode LSTM cells, accurate to fp32; "fp16" = sub-band LSTM
+        # operands stored as fp16 with fp32 accumulation / cell state -- the reference runs this model under fp16
+        # autocast on CUDA (fullsubnet.py:943)
         self.precision = precision or os.environ.get("SE_B200_FSN_PRECISION", "tf32")
-        if self.precision not in ("tf32", "fp16"):
-            raise ValueError("precision must be 'tf32' or 'fp16'")
+        if self.precision not in ("tf32", "3xtf32", "fp16"):
+            raise ValueError("precision must be 'tf32', '3xtf32' or 'fp16'")
         assert sequence_model in ("GRU", "LSTM"), f"{self.__class__.__name__} only support GRU and LSTM."
         if sequence_model != "LSTM" or fb_output_activate_function != "ReLU" or sb_output_activate_function:
             raise NotImplementedError("the B200 path builds the configuration of config.yaml:153-172 "
@@ -137,7 +138,8 @@ class FullSubNet(BaseModel):
         if self._ctx is None:
             cfg = SeFsnConfig(self.num_freqs, self.num_mics, self.fb_model_hidden_size, self.sb_model_hidden_size,
                               self.num_layers, self.sb_num_neighbors, self.fb_num_neighbors, need,
-                              _native.SE_PRECISION_FP16 if self.precision == "fp16" else _native.SE_PRECISION_TF32)
+                              {"tf32": _native.SE_PRECISION_TF32, "3xtf32": _native.SE_PRECISION_3XTF32,
+                               "fp16": _native.SE_PRECISION_FP16}[self.precision])
             ctx = C.c_void_p()
             check(lib().se_fsn_create(C.byref(ctx), dev, C.byref(cfg)), "se_fsn_create")
             self._ctx, self._ctx_device, self._ctx_capacity, self._fresh = ctx, dev, need, True
