@@ -83,7 +83,7 @@ struct Act {  // zero-bordered channels-last activation buffer [maxB][Tp][Fp][C]
 };
 
 enum OpKind { OP_GEMM, OP_NORM, OP_GRU_PW, OP_PRECONV, OP_GRU_SEQ, OP_DECONV_LAST, OP_SKIP_SMALL, OP_GRU_TC, OP_PRECONV_TC,
-              OP_PRECONV3, OP_ENC_MMA, OP_DEC_MMA, OP_GRU_WAVE, OP_ENC_TC };
+              OP_PRECONV3, OP_ENC_MMA, OP_DEC_MMA, OP_GRU_WAVE, OP_ENC_TC, OP_SKIP_BLEND };
 enum Stage { ST_STFT = 0, ST_PRECONV, ST_ENCODER, ST_GRU, ST_DECODER, ST_MASK, ST_ROLL, ST_COUNT };
 const char* kStageNames[ST_COUNT] = {"stft", "preconv", "encoder", "gru", "decoder", "mask_istft", "roll"};
 
@@ -105,6 +105,7 @@ struct Op {
     Preconv3Params p3;
     EncMmaParams em;
     DecMmaParams dm;
+    SkipBlendParams sb;
     int em_cin = 0, em_cout = 0;  // channel counts of the mma.sync block kernels (encoder / decoder)
     int small_c = 0;  // channel count of the two small-layer kernels
     // TMA operand delivery (gemm_tc.cu): geometry of the tensor the A operand is gathered from, [B][Tp][Fp][C] at `tma_base`
@@ -934,10 +935,44 @@ struct Builder {
             push_norm(ST_DECODER, n, w_off, b_off, wr_off, br_off);
             rec.op_norm = (int)c->ops.size() - 1;
         }
-        // small-channel levels (fp16 mode): the three ops above become ONE launch (back_mma.cu); their packed weights and
-        // report entries are reused
-        if (c->dec_mma && skip->C == Cout_real && Cop == Cout_real &&
-            dec_mma_supported(Cin, Cout_real, in.Tp, in.Fp, Fin, Fs)) {
+        // 32- / 64-channel levels (fp16 inference): the skip pair and the blend above become ONE launch (skip_blend_tc.cu)
+        // over the same packed weights and affines; the transposed conv stays the GEMM before it
+        if (c->half && !c->train && skip->C == Cout_real && Cop == Cout_real && skip_blend_supported(Cout_real, Fs, Fy)) {
+            const Op o_norm = c->ops.back();
+            const OpFix f_norm = fix.back();
+            c->ops.pop_back();
+            fix.pop_back();
+            const Op o_skip = c->ops.back();
+            const OpFix f_skip = fix.back();
+            c->ops.pop_back();
+            fix.pop_back();
+            Op op{};
+            op.kind = OP_SKIP_BLEND;
+            op.stage = ST_DECODER;
+            op.sb = SkipBlendParams{};
+            op.sb.t_org = skip->padT0;
+            op.sb.f_org = skip->padF0;
+            op.sb.Fs = Fs;
+            op.sb.Kp = o_skip.g.K;
+            op.sb.y = reinterpret_cast<const __half*>(y);
+            op.sb.Fy = Fy;
+            op.sb.stats = o_norm.n.stats;
+            op.sb.out = reinterpret_cast<__half*>(dst);
+            op.sb.oB = dB;
+            op.sb.oT = dT;
+            op.sb.oF = dF;
+            op.sb.student = c->student;
+            op.em_cout = Cout_real;
+            op.label = name + ".skip+gln+blend";
+            op.alg_flops = o_skip.alg_flops;
+            op.alg_bytes = 4.0 * T * Fy * Cout_real + 4.0 * 2 * T * Fs * Cout_real;  // y and skip tensor in, block output out
+            c->ops.push_back(op);
+            tma_src(skip->base, skip->C, skip->Fp, skip->Tp, skip->sT, skip->sB, 1, skip->padT0, skip->padF0);
+            fix.push_back({f_skip.w_off, f_skip.b_off, -1, f_norm.nw_off, f_norm.nb_off, f_norm.nwr_off, f_norm.nbr_off});
+        } else if (c->dec_mma && skip->C == Cout_real && Cop == Cout_real &&
+                   dec_mma_supported(Cin, Cout_real, in.Tp, in.Fp, Fin, Fs)) {
+            // small-channel levels (fp16 mode): the three ops above become ONE launch (back_mma.cu); their packed weights
+            // and report entries are reused
             const Op o_norm = c->ops.back();
             const OpFix f_norm = fix.back();
             c->ops.pop_back();
@@ -1734,6 +1769,15 @@ int build_ctx(se_ctx* c) {
             }
         } else if (op.kind == OP_PRECONV3) {
             for (int l = 0; l < 3; ++l) op.p3.w[l] = c->warena + c->pre3_w_off[l];
+        } else if (op.kind == OP_SKIP_BLEND) {
+            op.sb.w = reinterpret_cast<const __half*>(c->warena_h) + f.w_off;
+            op.sb.bias = c->warena + f.b_off;
+            op.sb.nw = c->warena + f.nw_off;
+            op.sb.nb = c->warena + f.nb_off;
+            op.sb.nwr = c->warena + f.nwr_off;
+            op.sb.nbr = c->warena + f.nbr_off;
+            if (make_skip_blend_maps(&op.sb, op.tma_base, op.tma_C, op.tma_Fp, op.tma_Tp, op.tma_sT, op.tma_sB, c->maxB))
+                return 1;
         } else if (op.kind == OP_DEC_MMA) {
             op.dm.w = c->warena + f.w_off;
             op.dm.bias = c->warena + f.b_off;
@@ -1904,6 +1948,11 @@ int launch_op(const se_ctx* c, const Op& op, int B, cudaStream_t st, int s0 = 0)
             dm.b0 = 0;
             dm.B = B;
             return launch_dec_mma(dm, op.em_cin, op.em_cout, st);
+        }
+        case OP_SKIP_BLEND: {
+            SkipBlendParams sb = op.sb;
+            sb.B = B;
+            return launch_skip_blend(sb, op.em_cout, st);
         }
         case OP_GRU_WAVE: {
             GruWaveParams gw = op.gw;

@@ -10,18 +10,9 @@ namespace {
 
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.f / (1.f + expf(-x)); }
 
-// mean / inverse denominator of GlobalLayerNorm from the accumulated (sum, sum of squares) in double
-// teacher: (x-mean)/(sqrt(var+1e-8)+1e-8)  (CRN_ELU.py:51);  student: (x-mean)/(sqrt(var)+1e-8) (distillation_crn.py:51)
 __device__ __forceinline__ void gln_coeffs(const double* stats, int b, double count, int student, float& mean,
                                            float& inv) {
-    const double s = stats[2 * b], ss = stats[2 * b + 1];
-    const double mu = s / count;
-    double var = ss / count - mu * mu;
-    if (var < 0.0) var = 0.0;
-    const float varf = (float)var;
-    const float den = student ? (sqrtf(varf) + 1e-8f) : (sqrtf(varf + 1e-8f) + 1e-8f);
-    mean = (float)mu;
-    inv = 1.0f / den;
+    gln_mean_inv(stats[2 * b], stats[2 * b + 1], count, student, mean, inv);
 }
 
 __device__ __forceinline__ float4 load4(const float* base, long long idx, bool is_half) {

@@ -1457,6 +1457,24 @@ int make_tma_3d_f16(TmaDesc* out, const void* base, int d0, int d1, int d2, long
     return 0;
 }
 
+int make_tma_4d_f16(TmaDesc* out, const void* base, const long long dims[4], const long long strides[3], const int box[4],
+                    int swizzle_bytes) {
+    EncodeTiledFn enc = encode_tiled_fn();
+    SE_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is not available from this driver");
+    SE_REQUIRE((swizzle_bytes == 64 || swizzle_bytes == 128) && box[0] * 2 == swizzle_bytes,
+               "make_tma_4d_f16: the box must span one swizzle row");
+    const cuuint64_t d[4] = {(cuuint64_t)dims[0], (cuuint64_t)dims[1], (cuuint64_t)dims[2], (cuuint64_t)dims[3]};
+    const cuuint64_t st[3] = {(cuuint64_t)strides[0], (cuuint64_t)strides[1], (cuuint64_t)strides[2]};
+    const cuuint32_t bx[4] = {(cuuint32_t)box[0], (cuuint32_t)box[1], (cuuint32_t)box[2], (cuuint32_t)box[3]};
+    const cuuint32_t estr[4] = {1, 1, 1, 1};
+    const CUresult r = enc(reinterpret_cast<CUtensorMap*>(out), CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(base),
+                           d, st, bx, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                           swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    SE_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled (4-D) failed with " + std::to_string((int)r));
+    return 0;
+}
+
 int gemm_profile_read(unsigned long long* out8, int reset) {
     SE_CUDA_OK(cudaDeviceSynchronize());
     if (out8) SE_CUDA_OK(cudaMemcpyFromSymbol(out8, g_gemm_prof, 8 * sizeof(unsigned long long)));

@@ -106,13 +106,7 @@ __device__ __forceinline__ void block_gln(float psum, float psq, double count, i
             a += s_red[w];
             q += s_red[NWARPS + w];
         }
-        const double mu = a / count;
-        double var = q / count - mu * mu;
-        if (var < 0.0) var = 0.0;
-        const float varf = (float)var;
-        const float den = student ? (sqrtf(varf) + 1e-8f) : (sqrtf(varf + 1e-8f) + 1e-8f);
-        s_co[0] = (float)mu;
-        s_co[1] = 1.0f / den;
+        gln_mean_inv(a, q, count, student, s_co[0], s_co[1]);
     }
     __syncthreads();
 }

@@ -21,6 +21,19 @@ struct NvtxRange {
 
 constexpr int kFramesPerChunk = 21;  // T = 1 + K/hop for K=3200, hop=160 (reference: torch.stft center=True)
 
+// GlobalLayerNorm mean and inverse denominator of one stream from its accumulated sum and sum of squares (double):
+// teacher (x-mean)/(sqrt(var+1e-8)+1e-8) (CRN_ELU.py:51), student (x-mean)/(sqrt(var)+1e-8) (distillation_crn.py:51)
+__host__ __device__ __forceinline__ void gln_mean_inv(double s, double ss, double count, int student, float& mean,
+                                                      float& inv) {
+    const double mu = s / count;
+    double var = ss / count - mu * mu;
+    if (var < 0.0) var = 0.0;
+    const float varf = (float)var;
+    const float den = student ? (sqrtf(varf) + 1e-8f) : (sqrtf(varf + 1e-8f) + 1e-8f);
+    mean = (float)mu;
+    inv = 1.0f / den;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // error plumbing
 // ---------------------------------------------------------------------------------------------------------------
@@ -508,6 +521,34 @@ int gru_profile_read(unsigned long long* out16, int reset);  // diagnostic cycle
 // 3-D tiled tensor map over fp16 data: dims (d0 fastest), strides of d1 / d2 in elements, box, SWIZZLE_128B
 int make_tma_3d_f16(TmaDesc* out, const void* base, int d0, int d1, int d2, long long s1, long long s2, int b0, int b1,
                     int b2);
+// 4-D tiled tensor map over fp16 data: dims (d0 fastest), byte strides of d1 .. d3, box; swizzle_bytes 64 or 128 (the
+// box's d0 extent in bytes)
+int make_tma_4d_f16(TmaDesc* out, const void* base, const long long dims[4], const long long strides[3], const int box[4],
+                    int swizzle_bytes);
+
+// gated skip path of the 32- / 64-channel decoder levels as one tcgen05 launch (skip_blend_tc.cu; fp16 inference):
+// out = m elu(residual(skip)) + (1 - m) GLN(y), m = sigmoid(GLN(residualmask(skip)))
+struct SkipBlendParams {
+    TmaDesc skip;            // the padded skip buffer, one box = one stream's interior (make_skip_blend_maps)
+    TmaDesc ymap;            // y, one box = one stream
+    int t_org, f_org;        // tensor coordinates of the interior's (frame 0, bin 0)
+    int Fs;                  // skip bins = output bins
+    const __half* w;         // the skip pair's packed fp16 weights [2C][Kp], rows interleaved (residualmask c, residual c)
+    int Kp;
+    const float* bias;       // [2C], same interleaving
+    const __half* y;         // [B][T][Fy][C] elu(deconv) of the level
+    int Fy;
+    const double* stats;     // [B][2] sum / sum of squares of y
+    const float *nw, *nb;    // norm affine [C]
+    const float *nwr, *nbr;  // residualnorm affine [C]
+    __half* out;             // block output, element strides below
+    long long oB, oT, oF;
+    int student, B;
+};
+bool skip_blend_supported(int C, int Fs, int Fy);
+int make_skip_blend_maps(SkipBlendParams* p, const void* skip_base, int C, int Fp, int Tp, long long sT, long long sB,
+                         int nB);  // p->Fs, p->Fy, p->y set
+int launch_skip_blend(const SkipBlendParams& p, int C, cudaStream_t st);
 
 // persistent small-batch GRU recurrence (gru_seq.cu): one cooperative launch per layer for all chunks and steps
 struct GruSeqParams {

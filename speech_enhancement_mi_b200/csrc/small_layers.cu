@@ -219,12 +219,14 @@ __device__ __forceinline__ uint2 ld_u64(const __half* q) { return __ldg(reinterp
 // grid (gx, B): the warps of a stream's blocks stride over its groups of 16 positions.  Fragment roles (g = lane / 4,
 // t = lane % 4): A rows g, g + 8 = positions, B column g = output channel of the n-tile, C columns 2t, 2t + 1.
 // n-tiles [0, C/8) are the mask channels, [C/8, C/4) the residual channels.  Lane t supplies the CPL = C/4 consecutive
-// channels CPL t .. CPL t + CPL - 1 of its rows (one 8 / 16 / 2 x 16 byte load per row); k-step s consumes elements
+// channels CPL t .. CPL t + CPL - 1 of its rows (one 4 / 8 byte load per row); k-step s consumes elements
 // 4s .. 4s+3 of that chunk.  NSPLIT > 1 splits the n-tiles over neighbouring warps that read the same rows; measured for
 // C = 64 (NSPLIT = 2, 64 registers of B fragments): 0.148 ms against 0.094 ms of the tcgen05 GEMM, whose 128-wide tile is
-// full at that width -- so 64 channels stay on the GEMM path and the dispatch below stops at 32 (0.099 -> 0.078 ms).
+// full at that width.  In fp16 inference 32 and 64 channels run fused with the blend (skip_blend_tc.cu); the dispatch
+// below serves 8 and 16.
 template <int C, int NSPLIT, int GQ>
 __global__ void __launch_bounds__(256) skip_small_mma_kernel(SkipSmallParams p) {
+    static_assert(C == 8 || C == 16, "skip_small_mma: 8 or 16 channels (one 4- or 8-byte A load per row)");
     constexpr int NT = C / 4, HT = NT / 2;          // n-tiles, n-tiles per kind
     constexpr int KS = C >= 16 ? C / 16 : 1;        // k-steps
     constexpr int CPL = C >= 16 ? C / 4 : 2;        // channels per lane and row
@@ -284,16 +286,7 @@ __global__ void __launch_bounds__(256) skip_small_mma_kernel(SkipSmallParams p) 
                     f = Fs - 1;
                 }
                 const __half* src = in + (tt * sT + f * sF);
-                if (C >= 32) {
-#pragma unroll
-                    for (int u = 0; u < CPL / 8; ++u) {
-                        const uint4 v = __ldg(reinterpret_cast<const uint4*>(src) + u);
-                        a[q][2 * u][h] = v.x;
-                        a[q][2 * u][2 + h] = v.y;
-                        a[q][2 * u + 1][h] = v.z;
-                        a[q][2 * u + 1][2 + h] = v.w;
-                    }
-                } else if (C == 16) {
+                if (C == 16) {
                     const uint2 u = ld_u64(src);
                     a[q][0][h] = u.x;
                     a[q][0][2 + h] = u.y;
@@ -440,7 +433,7 @@ __global__ void __launch_bounds__(256) deconv_last_mma_kernel(DeconvLastParams p
 }  // namespace
 
 bool deconv_last_supported(int Cin) { return Cin == 8 || Cin == 16; }
-bool skip_small_supported(int C) { return C == 8 || C == 16 || C == 32; }
+bool skip_small_supported(int C) { return C == 8 || C == 16; }
 
 int launch_deconv_last(const DeconvLastParams& p, int Cin, cudaStream_t st) {
     if (p.B <= 0) return 0;
@@ -465,10 +458,9 @@ int launch_skip_small(const SkipSmallParams& p, int C, cudaStream_t st) {
     const dim3 grid(cc ? (T * p.Fs + 255) / 256 : (C <= 16 ? 2 : 1), p.B);
     if (cc && C == 16) skip_small_kernel<16><<<grid, 256, 0, st>>>(p);
     else if (cc && C == 8) skip_small_kernel<8><<<grid, 256, 0, st>>>(p);
-    else if (C == 32) skip_small_mma_kernel<32, 1, 1><<<grid, 256, 0, st>>>(p);
     else if (C == 16) skip_small_mma_kernel<16, 1, 2><<<grid, 256, 0, st>>>(p);
     else if (C == 8) skip_small_mma_kernel<8, 1, 2><<<grid, 256, 0, st>>>(p);
-    else SE_REQUIRE(false, "skip_small: channels must be 8, 16 or 32");
+    else SE_REQUIRE(false, "skip_small: channels must be 8 or 16");
     SE_CUDA_OK(cudaGetLastError());
     return 0;
 }

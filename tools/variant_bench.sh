@@ -12,7 +12,7 @@ try:
     d = json.loads(open(f"gpurun_out/vb_{v}.json").read().strip().splitlines()[-1])
     k = {x["name"]: round(x["ms"] * 1000, 1) for x in d["kernels"]}
     names = ["convlist.2.conv+elu+gate", "convlist.3.conv+elu", "convlist.3.gate1x1", "gru.l0.input_proj", "gru.l1.input_proj", "gru.fc+elu",
-             "deconvlist.0.deconv+elu", "deconvlist.0.skip1x1", "deconvlist.1.deconv+elu", "deconvlist.1.skip1x1"]
+             "deconvlist.0.deconv+elu", "deconvlist.0.skip+gln+blend", "deconvlist.1.deconv+elu", "deconvlist.1.skip+gln+blend"]
     print(v, round(d["ms_per_step"], 3), [k.get(n) for n in names])
 except Exception as e:
     print(v, "failed", e)
