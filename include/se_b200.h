@@ -140,12 +140,21 @@ int se_fsn_num_params(const se_fsn* ctx);
 const char* se_fsn_param_name(const se_fsn* ctx, int index);
 int64_t se_fsn_param_numel(const se_fsn* ctx, int index);
 int se_fsn_bind_weights(se_fsn* ctx, const float* const* ptrs, int n, void* stream);
-/* replaces: FullSubNet.reset_state (fullsubnet.py:826-832): zero LSTM states, reset both CumLayerNorms */
+/* replaces: FullSubNet.reset_state (fullsubnet.py:826-832): zero LSTM states, reset both CumLayerNorms; also zeroes
+ * the overlap-add carry of se_fsn_process_chunk */
 int se_fsn_reset_state(se_fsn* ctx, int first, int count, void* stream);
 /* replaces: FullSubNet.forward on one chunk (fullsubnet.py:769-824), T = 21 frames:
  *   x [B, 2M, F, T] (M real planes then M imaginary planes, fullsubnet.py:835-844) -> compressed cIRM [B, 2, F, T];
  *   advances the LSTM states fh / sh and the CumLayerNorm running means of streams [0, B). */
 int se_fsn_forward_chunk(se_fsn* ctx, const float* x, float* out, int B, void* stream);
+/* true-streaming FullSubNet step (not in the reference; the chunk loop of fullsubnet.py:932-957 for ONE chunk):
+ *   in  : in[b*in_stream_stride + m*in_mic_stride + n], n < 3200, streams = rows [0, B) of the state arena
+ *   out : 1600 samples per stream at out[b*out_stream_stride + n] =
+ *         (first half of this chunk's iSTFT + carried second half of the previous chunk's) / 2
+ * Advances the LSTM states, both CumLayerNorms and the carry of streams [0, B).  No host synchronisation.
+ * STFT, network, mask, iSTFT and overlap-add run as one CUDA-graph replay per call (captured once per B). */
+int se_fsn_process_chunk(se_fsn* ctx, const float* in, int64_t in_stream_stride, int64_t in_mic_stride,
+                         float* out, int64_t out_stream_stride, int B, void* stream);
 /* replaces: the layout half of FullSubNet.stft_trans / preprocessing (fullsubnet.py:835-844, 880-886): spectrum
  * [R, M, F, T, 2] (se_stft_trans) -> x [R, 2M, F, T] (M real planes, then M imaginary planes) and / or the mic-0 pair
  * x0 [R, 2, F, T]; either output may be NULL */

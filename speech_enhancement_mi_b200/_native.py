@@ -81,6 +81,7 @@ SIGNATURES = {
     "se_fsn_bind_weights": (_I, [_P, C.POINTER(_P), _I, _P]),
     "se_fsn_reset_state": (_I, [_P, _I, _I, _P]),
     "se_fsn_forward_chunk": (_I, [_P, _P, _P, _I, _P]),
+    "se_fsn_process_chunk": (_I, [_P, _P, _L, _L, _P, _L, _I, _P]),
     "se_fsn_apply_mask": (_I, [_P, _P, _P, _I, _I, _I, _P]),
     "se_fsn_planes": (_I, [_P, _I, _I, _I, _I, _P, _P, _P]),
     "se_fsn_realtime_process": (_I, [_P, _P, _P, _I, _L, _I, _I, _P, _P, _P, _P, _P]),

@@ -28,6 +28,8 @@ using namespace se;
 namespace {
 
 constexpr int T = kFramesPerChunk;
+constexpr int KCHUNK = 3200;         // samples per chunk (config.yaml:172 segment_length)
+constexpr int PHOP = KCHUNK / 2;     // samples a streaming step returns
 inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 struct FsnParam {
@@ -92,6 +94,13 @@ struct se_fsn {
           *rt_chunks = nullptr, *rt_pline = nullptr, *rt_fbout = nullptr;
     size_t rt_rows = 0, rt_rows_train = 0, rt_xin_rows = 0;
     IoDesc* rt_io = nullptr;
+    // se_fsn_process_chunk: the overlap-add carry [maxB][K/2] is stream state (allocated with the context, zeroed by
+    // se_fsn_reset_state); the step's scratch is allocated for maxB streams on the first call, and its graphs (one per
+    // B, each setting its own cells) are kept apart from `graphs`, which holds the bare network
+    float* carry = nullptr;
+    float *st_spec = nullptr, *st_xin = nullptr, *st_x0 = nullptr, *st_crm = nullptr, *st_enh = nullptr;
+    IoDesc* st_io = nullptr;
+    std::map<int, cudaGraphExec_t> step_graphs;
     const float* cur_x = nullptr;  // indirection cell for graph replay
     const float** x_cell = nullptr;
     float** out_cell = nullptr;
@@ -471,6 +480,7 @@ int build(se_fsn* c) {
     if (dev_alloc(c, &c->sums, (size_t)4 * B)) return 1;
     if (dev_alloc(c, &c->cstate, (size_t)4 * B)) return 1;
     if (dev_alloc(c, &c->cstep, (size_t)2 * B)) return 1;
+    if (dev_alloc(c, &c->carry, (size_t)B * PHOP)) return 1;
     if (dev_alloc(c, &c->x_cell, 1)) return 1;
     if (dev_alloc(c, &c->out_cell, 1)) return 1;
 
@@ -626,13 +636,40 @@ __global__ void fsn_planes_kernel(const float* spec, int M, int F, float* x, flo
     }
 }
 
-int run_chunk_graph(se_fsn* c, int B, cudaStream_t st) {
-    auto it = c->graphs.find(B);
-    if (it == c->graphs.end()) {
+// The streaming step of se_fsn_process_chunk for streams [0, B): framing + STFT of the chunk the IoDesc cell st_io
+// describes, network input and mic-0 pair, the chunk network on them, decompress_cIRM + complex mask (the arithmetic of
+// se_fsn_realtime_process), iSTFT and the overlap-add with the carried half, written where st_io points.
+int enqueue_step(se_fsn* c, int B, cudaStream_t st) {
+    StftParams sp{};
+    sp.io = c->st_io;
+    sp.B = B;
+    sp.M = c->M;
+    sp.spec_ref = c->st_spec;
+    if (launch_stft_features(sp, st)) return 1;
+    const long long total = (long long)B * c->M * c->F * T;
+    fsn_planes_kernel<<<(int)((total + 255) / 256), 256, 0, st>>>(c->st_spec, c->M, c->F, c->st_xin, c->st_x0, total);
+    fsn_set_cells<<<1, 1, 0, st>>>(c->x_cell, c->st_xin, c->out_cell, c->st_crm);
+    SE_CUDA_OK(cudaGetLastError());
+    if (enqueue(c, B, st)) return 1;
+    if (se_fsn_apply_mask(c->st_crm, c->st_x0, c->st_enh, B, c->F, T, st)) return 1;
+    MaskIstftParams mp{};
+    mp.io = c->st_io;
+    mp.B = B;
+    mp.spec_in = c->st_enh;
+    mp.carry = c->carry;
+    return launch_mask_istft(mp, st);
+}
+
+// replays enq(c, B) from `graphs`, capturing it first on the context's private stream (so that the caller's stream is
+// never put into capture mode)
+int run_graph(se_fsn* c, std::map<int, cudaGraphExec_t>& graphs, int (*enq)(se_fsn*, int, cudaStream_t), int B,
+              cudaStream_t st) {
+    auto it = graphs.find(B);
+    if (it == graphs.end()) {
         if (!c->own_stream) SE_CUDA_OK(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
         cudaGraph_t graph = nullptr;
         SE_CUDA_OK(cudaStreamBeginCapture(c->own_stream, cudaStreamCaptureModeThreadLocal));
-        const int rc = enqueue(c, B, c->own_stream);
+        const int rc = enq(c, B, c->own_stream);
         cudaError_t e = cudaStreamEndCapture(c->own_stream, &graph);
         if (rc) {
             if (graph) cudaGraphDestroy(graph);
@@ -642,11 +679,13 @@ int run_chunk_graph(se_fsn* c, int B, cudaStream_t st) {
         cudaGraphExec_t exec = nullptr;
         SE_CUDA_OK(cudaGraphInstantiate(&exec, graph, 0));
         SE_CUDA_OK(cudaGraphDestroy(graph));
-        it = c->graphs.emplace(B, exec).first;
+        it = graphs.emplace(B, exec).first;
     }
     SE_CUDA_OK(cudaGraphLaunch(it->second, st));
     return 0;
 }
+
+int run_chunk_graph(se_fsn* c, int B, cudaStream_t st) { return run_graph(c, c->graphs, enqueue, B, st); }
 
 template <typename Tp>
 int regrow(se_fsn* c, Tp** buf, size_t count) {  // scratch: freed and re-allocated larger (registered for destroy)
@@ -695,6 +734,7 @@ int se_fsn_destroy(se_fsn* c) {
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     for (auto& kv : c->graphs) cudaGraphExecDestroy(kv.second);
+    for (auto& kv : c->step_graphs) cudaGraphExecDestroy(kv.second);
     if (c->own_stream) cudaStreamDestroy(c->own_stream);
     for (void* p : c->allocs) cudaFree(p);
     delete c;
@@ -756,6 +796,8 @@ int se_fsn_reset_state(se_fsn* c, int first, int count, void* stream) {
     }
     SE_CUDA_OK(cudaMemsetAsync(c->cstate + 4 * (size_t)first, 0, 4 * (size_t)count * sizeof(float), st));
     SE_CUDA_OK(cudaMemsetAsync(c->cstep + 2 * (size_t)first, 0, 2 * (size_t)count * sizeof(int), st));
+    // overlap-add carry of se_fsn_process_chunk
+    SE_CUDA_OK(cudaMemsetAsync(c->carry + (size_t)PHOP * first, 0, (size_t)PHOP * count * sizeof(float), st));
     return 0;
 }
 
@@ -769,6 +811,30 @@ int se_fsn_forward_chunk(se_fsn* c, const float* x, float* out, int B, void* str
     cudaStream_t st = (cudaStream_t)stream;
     fsn_set_cells<<<1, 1, 0, st>>>(c->x_cell, x, c->out_cell, out);
     return run_chunk_graph(c, B, st);
+}
+
+int se_fsn_process_chunk(se_fsn* c, const float* in, int64_t in_stream_stride, int64_t in_mic_stride, float* out,
+                         int64_t out_stream_stride, int B, void* stream) {
+    NvtxRange nvtx_range("se.fsn_chunk_step");
+    SE_REQUIRE(c != nullptr && c->weights_bound, "se_fsn_process_chunk: context without weights");
+    SE_REQUIRE(in != nullptr && out != nullptr, "se_fsn_process_chunk: null buffer");
+    SE_REQUIRE(B >= 0 && B <= c->maxB, "se_fsn_process_chunk: B exceeds max_streams");
+    SE_REQUIRE(c->M <= 3, "se_fsn_process_chunk: the framing kernel serves at most 3 microphones");
+    if (B == 0) return 0;
+    SE_CUDA_OK(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!c->st_io) {  // the step's scratch, for the context's capacity: a graph captured for one B keeps its pointers
+        const size_t per = (size_t)c->F * T, R = c->maxB;
+        if (dev_alloc(c, &c->st_spec, R * c->M * per * 2)) return 1;
+        if (dev_alloc(c, &c->st_xin, R * 2 * c->M * per)) return 1;
+        if (dev_alloc(c, &c->st_x0, R * 2 * per)) return 1;
+        if (dev_alloc(c, &c->st_crm, R * 2 * per)) return 1;
+        if (dev_alloc(c, &c->st_enh, R * 2 * per)) return 1;
+        if (dev_alloc(c, &c->st_io, 1)) return 1;
+    }
+    IoDesc io{in, in_stream_stride, in_mic_stride, 0, KCHUNK, out, out_stream_stride, PHOP};
+    if (launch_set_io(c->st_io, io, st)) return 1;
+    return run_graph(c, c->step_graphs, enqueue_step, B, st);
 }
 
 int se_fsn_realtime_process(se_fsn* c, const float* mixture, const float* source, int B, int64_t L, int flag, int train,

@@ -2,11 +2,14 @@
 the reference's constructor kwargs (config.yaml:153-172), ``state_dict`` keys (``fb_model.*`` / ``sb_model.*``) and
 methods, the arithmetic running in the sm_100a kernels behind include/se_b200.h (se_fsn_*).
 
-Reference: fullsubnet.py:299-331 (unfold), :685-961 (FullSubNet).  Only the chunked loop the trainers and predictors
-use (``train=False``: train_fullsubnet.py:138,151; predict_fullsubnet.py:75) is built; ``train=True`` (all chunks
-concatenated into one forward) raises NotImplementedError; ``compute_loss`` is forward only (no autograd graph).  The reference runs this loop under fp16
-autocast on CUDA (fullsubnet.py:943) and in fp32 on the CPU; this path uses TF32 tensor cores with fp32 accumulation
-and fp32 cell state, checked against the fp32 CPU run.  No PyTorch / CPU compute fallback.
+Reference: fullsubnet.py:299-331 (unfold), :685-961 (FullSubNet).  ``realtime_process`` runs the chunked loop the
+trainers and predictors use (``train=False``: train_fullsubnet.py:138,151; predict_fullsubnet.py:75) and, with
+``train=True``, all chunks as one forward (both CumLayerNorms see the whole utterance), forward only: there is no
+backward, and ``compute_loss`` has no autograd graph either.  ``process_chunk`` / ``process_chunk_host`` (not in the
+reference) are the serving form of the loop: one chunk per call, the overlap-add carry kept on the device.  The
+reference runs this loop under fp16 autocast on CUDA (fullsubnet.py:943) and in fp32 on the CPU; this path uses TF32
+tensor cores with fp32 accumulation and fp32 cell state (or the ``precision`` modes below), checked against the fp32
+CPU run.  No PyTorch / CPU compute fallback.
 """
 from __future__ import annotations
 
@@ -17,7 +20,7 @@ import torch
 import torch.nn as nn
 
 from . import utility
-from . import _native
+from . import _host_pipeline, _native
 from ._native import SeFsnConfig, check, lib
 
 EPS = 1e-8
@@ -186,6 +189,40 @@ class FullSubNet(BaseModel):
             check(lib().se_fsn_forward_chunk(ctx, xd.data_ptr(), out.data_ptr(), B, _stream(dev)), "se_fsn_forward_chunk")
         self._fresh = False
         return out.to(noisy_complex.device)
+
+    def process_chunk(self, chunk, out=None):
+        """True-streaming step (not in the reference; the chunk loop of fullsubnet.py:932-957 for one chunk): chunk
+        [B, M, K] on a CUDA device, any strides -> K/2 enhanced samples per stream [B, K/2] (or into ``out``, whose rows
+        may be strided), overlap-added with the carried half of the previous chunk.  Advances the LSTM states, both
+        CumLayerNorms and the carry of streams [0, B) in one CUDA-graph replay (se_fsn_process_chunk); reset_state()
+        starts every stream afresh."""
+        if not torch.is_tensor(chunk) or not chunk.is_cuda:
+            raise ValueError("process_chunk expects a CUDA tensor")
+        if chunk.dim() != 3 or chunk.shape[1] != self.num_mics or chunk.shape[2] != self.segment_length:
+            raise ValueError(f"process_chunk expects [B, {self.num_mics}, {self.segment_length}], "
+                             f"got {tuple(chunk.shape)}")
+        B, _, K = chunk.shape
+        if chunk.dtype != torch.float32 or chunk.stride(2) != 1:
+            chunk = chunk.to(torch.float32).contiguous()
+        dev = self._pick_device(chunk)
+        if out is None:
+            out = torch.empty((B, K // 2), dtype=torch.float32, device=chunk.device)
+        elif (out.device != chunk.device or out.dtype != torch.float32 or tuple(out.shape) != (B, K // 2)
+              or out.stride(1) != 1):
+            raise ValueError(f"out must be a float32 [{B}, {K // 2}] tensor with unit sample stride on {chunk.device}")
+        ctx = self._ensure_ctx(B, dev, keep_state=True)
+        with torch.cuda.device(dev):
+            check(lib().se_fsn_process_chunk(ctx, chunk.data_ptr(), chunk.stride(0), chunk.stride(1), out.data_ptr(),
+                                             out.stride(0), B, _stream(dev)), "se_fsn_process_chunk")
+        self._fresh = False
+        return out
+
+    def process_chunk_host(self, host_chunk, host_out):
+        """process_chunk with pinned HOST buffers for a serving loop that keeps audio in host memory: host_chunk
+        [B, M, K] -> host_out [B, K/2].  The copies run on side streams over double-buffered device staging, so that the
+        copies of neighbouring steps overlap the compute.  Returns a CUDA event that completes when ``host_out`` holds
+        this chunk's result (call ``.synchronize()`` before reading it).  State semantics are those of process_chunk."""
+        return _host_pipeline.process_chunk_host(self, host_chunk, host_out)
 
     def _spectrum(self, x, dev):
         R, M, K = x.shape
