@@ -80,8 +80,22 @@ int se_crn_bind_weights(se_ctx* ctx, const float* const* ptrs, int n, void* stre
 /* ---- per-stream state (CRN_ELU.py:158,228 buffers + GRU h; reset: CRN_ELU.py:408-415) ------------------------ */
 /* zero the causal-conv buffers, GRU state and overlap-add carry of streams [first, first+count) */
 int se_crn_state_reset(se_ctx* ctx, int first, int count, void* stream);
-/* bytes of carried state per stream (SURVEY.md section 8(a) a12) */
+/* bytes of carried state per stream (SURVEY.md section 8(a) a12): exactly the size of one export record
+ * (0 for a training context, which has no streaming state to export) */
 int64_t se_crn_state_bytes_per_stream(const se_ctx* ctx);
+/* Export / import of the carried state of chosen rows (compaction, migration between contexts or GPUs, checkpoints).
+ * A record holds everything the next step of a stream reads (DESIGN.md section 3), se_crn_state_bytes_per_stream bytes,
+ * its layout fixed by the model, configuration, precision and front path, never by max_streams or the device.
+ *   export: record i of dst_dev <- row rows_host[i] (rows may repeat); the context's state is only read
+ *   import: row rows_host[i] <- record i of src_dev (rows must be distinct); `layout` is se_crn_state_layout of the
+ *           exporting context and must equal this context's
+ * rows_host[i] in [0, max_streams); dst / src are 16-byte aligned device buffers of n records.  Both calls are ordered on
+ * `stream` with the steps, do not synchronise the host and keep captured step graphs valid (import writes in place).
+ * Training contexts reject both. */
+uint64_t se_crn_state_layout(const se_ctx* ctx);
+int se_crn_state_export(se_ctx* ctx, const int32_t* rows_host, int n, void* dst_dev, void* stream);
+int se_crn_state_import(se_ctx* ctx, const int32_t* rows_host, int n, const void* src_dev, uint64_t layout,
+                        void* stream);
 
 /* ---- the fused hot path: one chunk step for B streams --------------------------------------------------------
  * replaces one iteration of the loop CRN_ELU.py:485-489 plus its share of preprocessing/postprocessing
@@ -143,6 +157,13 @@ int se_fsn_bind_weights(se_fsn* ctx, const float* const* ptrs, int n, void* stre
 /* replaces: FullSubNet.reset_state (fullsubnet.py:826-832): zero LSTM states, reset both CumLayerNorms; also zeroes
  * the overlap-add carry of se_fsn_process_chunk */
 int se_fsn_reset_state(se_fsn* ctx, int first, int count, void* stream);
+/* export / import of the carried state of chosen rows, as se_crn_state_export / se_crn_state_import: both LSTM layers'
+ * h and c of the full-band and every sub-band sequence, both CumLayerNorms and the overlap-add carry */
+int64_t se_fsn_state_bytes_per_stream(const se_fsn* ctx);
+uint64_t se_fsn_state_layout(const se_fsn* ctx);
+int se_fsn_state_export(se_fsn* ctx, const int32_t* rows_host, int n, void* dst_dev, void* stream);
+int se_fsn_state_import(se_fsn* ctx, const int32_t* rows_host, int n, const void* src_dev, uint64_t layout,
+                        void* stream);
 /* replaces: FullSubNet.forward on one chunk (fullsubnet.py:769-824), T = 21 frames:
  *   x [B, 2M, F, T] (M real planes then M imaginary planes, fullsubnet.py:835-844) -> compressed cIRM [B, 2, F, T];
  *   advances the LSTM states fh / sh and the CumLayerNorm running means of streams [0, B). */

@@ -14,8 +14,9 @@ import os
 import torch
 import torch.nn as nn
 
-from . import _host_pipeline, _native
+from . import _host_pipeline, _native, stream_state
 from ._native import SeCrnConfig, check, lib
+from .stream_state import StreamState  # noqa: F401  (the type export_state returns)
 
 EPS = 1e-8  # CRN_ELU.py:11
 
@@ -553,6 +554,37 @@ class TemporalCRN(nn.Module):
         neighbouring steps overlap the compute.  Returns a CUDA event that completes when ``host_out`` holds this
         chunk's result (call ``.synchronize()`` before reading it).  State semantics are those of process_chunk."""
         return _host_pipeline.process_chunk_host(self, host_chunk, host_out)
+
+    def export_state(self, rows):
+        """Carried state of streams ``rows`` (ints or an int tensor; repeats allowed) -> ``StreamState`` on the
+        context's device, one record per row (not in the reference).  Runs on the current torch stream of that device
+        and leaves the streams untouched.  With ``import_state`` this moves live streams: compaction of the row prefix
+        the step runs on, migration to a context with more rows or to another GPU, checkpoints (``.cpu()``)."""
+        if self._state_owner == "chunk-batch":
+            raise RuntimeError("export_state: the state was last advanced by the chunk-batched realtime_process, which "
+                               "keeps it in the training context; stream with process_chunk to export it")
+        if self._ctx is None:
+            raise RuntimeError("export_state: no streaming context yet (nothing has been processed)")
+        dev = self._ctx_device
+        with torch.cuda.device(dev):
+            return stream_state.export_records(
+                self._ctx, dev, rows, lib().se_crn_state_bytes_per_stream(self._ctx), lib().se_crn_state_layout(self._ctx),
+                lib().se_crn_state_export, self._stream_ptr(dev), "se_crn_state_export")
+
+    def import_state(self, state, rows):
+        """Write the records of ``state`` (from ``export_state`` of a model with the same configuration and precision)
+        into streams ``rows`` (distinct), on the current torch stream of the context's device.  Creates the streaming
+        context if there is none, with room for max(max_streams, max(rows) + 1) streams, on the device the records are
+        on (CPU records: the model's device).  Captured step graphs stay valid: the state is written in place."""
+        rows = stream_state.row_list(rows)
+        dev = self._pick_device(state.data) if self._ctx is None else self._ctx_device
+        ctx = self._ensure_ctx(max(rows, default=-1) + 1, dev, keep_state=True)
+        with torch.cuda.device(dev):
+            stream_state.import_records(
+                ctx, dev, state, rows, lib().se_crn_state_bytes_per_stream(ctx), lib().se_crn_state_layout(ctx),
+                lib().se_crn_state_import, self._stream_ptr(dev), "se_crn_state_import")
+        self._state_owner = "stream"
+        self._fresh = False
 
     def compute_loss(self, source, pred_source, length):
         """CRN_ELU.py:513-535: loss = 0.7 * stoi_loss + 0.3 * (-SI-SNR); NaN => zero-filled; prints sisnr."""

@@ -48,6 +48,7 @@ _P = C.c_void_p
 _I = C.c_int
 _L = C.c_int64
 _PI = C.POINTER(C.c_int)
+_PI32 = C.POINTER(C.c_int32)
 
 # name -> (restype, argtypes); must list every symbol of include/se_b200.h (tests/test_abi.py checks this)
 SIGNATURES = {
@@ -61,6 +62,9 @@ SIGNATURES = {
     "se_crn_bind_weights": (_I, [_P, C.POINTER(_P), _I, _P]),
     "se_crn_state_reset": (_I, [_P, _I, _I, _P]),
     "se_crn_state_bytes_per_stream": (_L, [_P]),
+    "se_crn_state_layout": (C.c_uint64, [_P]),
+    "se_crn_state_export": (_I, [_P, _PI32, _I, _P, _P]),
+    "se_crn_state_import": (_I, [_P, _PI32, _I, _P, C.c_uint64, _P]),
     "se_crn_process_chunk": (_I, [_P, _P, _L, _L, _P, _L, _I, _P]),
     "se_crn_realtime_process": (_I, [_P, _P, _I, _L, _I, _P, _P]),
     "se_crn_realtime_process_host": (_I, [_P, _P, _I, _L, _I, _P]),
@@ -80,6 +84,10 @@ SIGNATURES = {
     "se_fsn_param_numel": (_L, [_P, _I]),
     "se_fsn_bind_weights": (_I, [_P, C.POINTER(_P), _I, _P]),
     "se_fsn_reset_state": (_I, [_P, _I, _I, _P]),
+    "se_fsn_state_bytes_per_stream": (_L, [_P]),
+    "se_fsn_state_layout": (C.c_uint64, [_P]),
+    "se_fsn_state_export": (_I, [_P, _PI32, _I, _P, _P]),
+    "se_fsn_state_import": (_I, [_P, _PI32, _I, _P, C.c_uint64, _P]),
     "se_fsn_forward_chunk": (_I, [_P, _P, _P, _I, _P]),
     "se_fsn_process_chunk": (_I, [_P, _P, _L, _L, _P, _L, _I, _P]),
     "se_fsn_apply_mask": (_I, [_P, _P, _P, _I, _I, _I, _P]),

@@ -8,6 +8,7 @@
 //     look-ahead inside the chunk) and one zero row on each side of F (stride-2 phase split, taps {0,2,4} / {1,3}).
 // The carried state of a stream is therefore the leading frames of its conv-input buffers, slot 0 of the two GRU
 // hidden sequences and the K/2 overlap-add carry; "roll" moves the trailing frames to the front after each chunk.
+// se_crn_state_export / _import gather and scatter exactly that state of chosen rows (state_tab, state_io.cu).
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <math.h>
@@ -215,7 +216,8 @@ struct se_ctx {
     RollTable roll{};
     RollTable zero_tab{};
     int64_t roll_floats = 0;   // floats moved per stream by the roll kernel
-    int64_t state_floats = 0;  // carried state per stream (allocated extents, incl. zero borders of the GEMM-path buffers)
+    StateTable state_tab;       // what a stream carries between steps (se_crn_state_export / _import; state_io.cu)
+    uint64_t state_layout = 0;  // hash of the record layout
 
     IoDesc* io_dev = nullptr;
     bool use_graph = true;
@@ -1819,7 +1821,6 @@ int build_ctx(se_ctx* c) {
         RollEntry e{base, sB, src, 0, count};
         c->roll.e[c->roll.n++] = e;
         c->zero_tab.e[c->zero_tab.n++] = e;
-        c->state_floats += count;
         c->roll_floats += count;
     };
     if (c->train)
@@ -1827,17 +1828,14 @@ int build_ctx(se_ctx* c) {
     if (c->front_mma) {  // rolled by the kernel itself; the borders of the feature buffer are never written
         RollEntry e{reinterpret_cast<float*>(c->pre_state), pre_state_sB / 2, 0, 0, (int)(pre_state_sB / 2)};
         c->zero_tab.e[c->zero_tab.n++] = e;
-        c->state_floats += 3 * 5 * 4 * NBIN;
     }
     for (int i = 0; i < 3 && c->preconv_tc && !c->front_mma; ++i) {  // rolled by the kernel itself; a reset clears the whole slab
         RollEntry e{reinterpret_cast<float*>(c->pre_h[i]), pre_h_sB / 2, 0, 0, (int)(pre_h_sB / 2)};
         c->zero_tab.e[c->zero_tab.n++] = e;
-        c->state_floats += 5 * 4 * NBIN;
     }
     for (const PreBuf& pb : c->pre_in) {  // rolled by the preconv kernel itself; a reset clears the whole slab
         RollEntry e{pb.base, pb.sB, 0, 0, (int)pb.sB};
         c->zero_tab.e[c->zero_tab.n++] = e;
-        c->state_floats += 5 * 4 * NBIN;
     }
     const int fpe = 4 / c->esz;  // operand elements per float: the roll / zero kernels move 4-byte units
     for (const Act& a : c->enc_in)
@@ -1851,7 +1849,6 @@ int build_ctx(se_ctx* c) {
     {
         RollEntry e{c->carry, PHOP, 0, 0, PHOP};
         c->zero_tab.e[c->zero_tab.n++] = e;
-        c->state_floats += PHOP;
     }
     if (c->train) {
         SE_REQUIRE(c->roll.n == 3 + c->L + 2, "internal: training state table");
@@ -1860,6 +1857,44 @@ int build_ctx(se_ctx* c) {
             if (dev_alloc(c, &p, (size_t)c->roll.e[e].count * maxB)) return 1;
             c->carry_store.push_back(p);
         }
+    }
+    // export / import: exactly what the next step reads, where it sits between steps.  The front kernels roll their own
+    // inputs when they load them (frames 21..24 -> 0..3), launch_roll moves the other entries at the end of the step, so
+    // between steps every carried frame is a LEADING frame and slot 0 of hseq is h_T.
+    if (!c->train) {
+        StateTable& t = c->state_tab;
+        t.desc = "crn variant=" + std::to_string(g.variant) + " precision=" + std::to_string(g.precision) +
+                 " inputs=" + std::to_string(g.num_inputs) + " freqs=" + std::to_string(g.num_freqs) + " channels=";
+        for (int i = 0; i < c->L; ++i) t.desc += std::to_string(g.num_channels[i]) + ",";
+        t.desc += " hidden=" + std::to_string(g.hidden) + " layers=" + std::to_string(g.num_layers) + " kernel=" +
+                  std::to_string(g.kernel_size) + " segment=" + std::to_string(g.segment_length) + " front=" +
+                  (c->front_mma ? "mma" : c->preconv_tc ? "tc" : "planar") + " half=" + std::to_string(c->half);
+        if (c->front_mma) {  // [3 layers][4 frames][224 positions][8 halves]: all of it is carried
+            if (state_table_add(t, "pre_state", 2, c->pre_state, pre_state_sB * 2, pre_state_sB * 2)) return 1;
+        }
+        for (int i = 0; i < 3 && c->preconv_tc && !c->front_mma; ++i)  // frames 0..3 of [25][272][8] halves
+            if (state_table_add(t, "pre_h" + std::to_string(i), 2, c->pre_h[i], pre_h_sB * 2,
+                                4LL * PRECONV_TC_POS * 8 * 2))
+                return 1;
+        for (int i = 0; i < (int)c->pre_in.size(); ++i) {  // frames 0..3 of each of the 5 channel planes [25][Fpp]
+            const PreBuf& pb = c->pre_in[i];
+            if (state_table_add(t, "pre_in" + std::to_string(i), 4, pb.base, pb.sB * 4, 4LL * pb.Fpp * 4, 5, pb.sC * 4))
+                return 1;
+        }
+        for (int i = 0; i < 2 * c->L; ++i) {  // the decoder inputs have no leading frames (padT0 = 0): look-ahead only
+            const Act& a = i < c->L ? c->enc_in[i] : c->dec_in[i - c->L];
+            if (a.padT0 > 0 && state_table_add(t, (i < c->L ? "enc_in" : "dec_in") + std::to_string(i % c->L), c->esz,
+                                               a.base, a.sB * c->esz, a.padT0 * a.sT * c->esz))
+                return 1;
+        }
+        for (int l = 0; l < 2; ++l)
+            if (state_table_add(t, "hseq" + std::to_string(l), c->esz, c->hseq[l], (long long)(T + 1) * H * c->esz,
+                                (long long)H * c->esz))
+                return 1;
+        for (int l = 0; l < 2 && c->half; ++l)  // the fp32 master copy the fp16 recurrence continues from
+            if (state_table_add(t, "h32_" + std::to_string(l), 4, c->h32[l], (long long)H * 4, (long long)H * 4)) return 1;
+        if (state_table_add(t, "carry", 4, c->carry, PHOP * 4, PHOP * 4)) return 1;
+        c->state_layout = state_layout_hash(t);
     }
     if (init_fft_tables()) return 1;
     return 0;
@@ -2674,7 +2709,34 @@ int se_crn_state_reset(se_ctx* c, int first, int count, void* stream) {
 
 int64_t se_crn_state_bytes_per_stream(const se_ctx* c) {
     if (!c) return -1;
-    return c->state_floats * 4;
+    return c->state_tab.record_bytes;
+}
+
+uint64_t se_crn_state_layout(const se_ctx* c) { return c ? c->state_layout : 0; }
+
+int se_crn_state_export(se_ctx* c, const int32_t* rows_host, int n, void* dst_dev, void* stream) {
+    NvtxRange nvtx_range("se.state_export");
+    SE_REQUIRE(c != nullptr, "null context");
+    SE_REQUIRE(!c->train, "se_crn_state_export: a training context carries no per-stream streaming state");
+    if (state_rows_check(rows_host, n, c->maxB, false, "se_crn_state_export")) return 2;
+    SE_REQUIRE(n == 0 || (dst_dev != nullptr && reinterpret_cast<uintptr_t>(dst_dev) % 16 == 0),
+               "se_crn_state_export: dst must be a 16-byte aligned device buffer");
+    SE_CUDA_OK(cudaSetDevice(c->device));
+    return launch_state_pack(c->state_tab, rows_host, n, dst_dev, (cudaStream_t)stream);
+}
+
+int se_crn_state_import(se_ctx* c, const int32_t* rows_host, int n, const void* src_dev, uint64_t layout, void* stream) {
+    NvtxRange nvtx_range("se.state_import");
+    SE_REQUIRE(c != nullptr, "null context");
+    SE_REQUIRE(!c->train, "se_crn_state_import: a training context carries no per-stream streaming state");
+    SE_REQUIRE(layout == c->state_layout,
+               "se_crn_state_import: record layout mismatch (records from another model, configuration, precision or "
+               "front path; this context:" + c->state_tab.desc + ")");
+    if (state_rows_check(rows_host, n, c->maxB, true, "se_crn_state_import")) return 2;
+    SE_REQUIRE(n == 0 || (src_dev != nullptr && reinterpret_cast<uintptr_t>(src_dev) % 16 == 0),
+               "se_crn_state_import: src must be a 16-byte aligned device buffer");
+    SE_CUDA_OK(cudaSetDevice(c->device));
+    return launch_state_unpack(c->state_tab, rows_host, n, src_dev, (cudaStream_t)stream);
 }
 
 int se_crn_process_chunk(se_ctx* c, const float* in, int64_t in_stream_stride, int64_t in_mic_stride, float* out,

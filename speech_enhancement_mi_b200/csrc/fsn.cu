@@ -9,6 +9,7 @@
 // through the koff table, W = [W_ih | W_hh] with rows re-ordered to [i|f|g|o] per 32-unit tile, bias = b_ih + b_hh, and
 // the cell update fused in the epilogue -- the input projection is never materialised.  Per-sequence record (fp32):
 //   [ x: T x Kin_pad | h(layer 0): (T+1) x H | h(layer 1): (T+1) x H ]      slot 0 of an h history = carried state
+// (se_fsn_state_export / _import gather and scatter the carried state of chosen rows: state_tab, state_io.cu)
 // The reflect-padded neighbour gather is expanded once per chunk into the x part of the sub-band records (540 KB per
 // stream and chunk, against 15.4 GFLOP of LSTM work per stream and chunk).
 #include <cuda_fp16.h>
@@ -98,6 +99,8 @@ struct se_fsn {
     // se_fsn_reset_state); the step's scratch is allocated for maxB streams on the first call, and its graphs (one per
     // B, each setting its own cells) are kept apart from `graphs`, which holds the bare network
     float* carry = nullptr;
+    StateTable state_tab;       // what a stream carries between steps (se_fsn_state_export / _import; state_io.cu)
+    uint64_t state_layout = 0;  // hash of the record layout
     float *st_spec = nullptr, *st_xin = nullptr, *st_x0 = nullptr, *st_crm = nullptr, *st_enh = nullptr;
     IoDesc* st_io = nullptr;
     std::map<int, cudaGraphExec_t> step_graphs;
@@ -483,6 +486,28 @@ int build(se_fsn* c) {
     if (dev_alloc(c, &c->carry, (size_t)B * PHOP)) return 1;
     if (dev_alloc(c, &c->x_cell, 1)) return 1;
     if (dev_alloc(c, &c->out_cell, 1)) return 1;
+    {  // export / import (state_io.cu): h_T in slot 0 of both records (after fsn_roll_kernel), the cell states, both
+       // CumLayerNorms and the step carry.  `sums` is not state: every step zeroes it before it accumulates.
+        StateTable& t = c->state_tab;
+        t.desc = "fsn freqs=" + std::to_string(F) + " mics=" + std::to_string(c->M) + " fb_hidden=" + std::to_string(Hf) +
+                 " sb_hidden=" + std::to_string(Hs) + " layers=" + std::to_string(g.num_layers) + " sb_neighbors=" +
+                 std::to_string(g.sb_num_neighbors) + " fb_neighbors=" + std::to_string(g.fb_num_neighbors) +
+                 " precision=" + std::to_string(g.precision);
+        const long long rF = c->recF * 4, rS = c->recS * c->sesz;
+        if (state_table_add(t, "fb_h0", 4, c->fbrec + c->f_h0, rF, Hf * 4LL) ||
+            state_table_add(t, "fb_h1", 4, c->fbrec + c->f_h1, rF, Hf * 4LL) ||
+            state_table_add(t, "sb_h0", c->sesz, reinterpret_cast<char*>(c->sbrec) + c->s_h0 * c->sesz, F * rS,
+                            (long long)Hs * c->sesz, F, rS) ||
+            state_table_add(t, "sb_h1", c->sesz, reinterpret_cast<char*>(c->sbrec) + c->s_h1 * c->sesz, F * rS,
+                            (long long)Hs * c->sesz, F, rS) ||
+            // cell states, unit-major [layer][H][maxB (* F)]: one column (F columns) per stream in each of 2H unit rows
+            state_table_add(t, "fb_c", 4, c->fbc, 4, 4, 2 * Hf, (long long)B * 4) ||
+            state_table_add(t, "sb_c", 4, c->sbc, F * 4LL, F * 4LL, 2 * Hs, (long long)B * F * 4) ||
+            state_table_add(t, "cstate", 4, c->cstate, 16, 16) || state_table_add(t, "cstep", 4, c->cstep, 8, 8) ||
+            state_table_add(t, "carry", 4, c->carry, PHOP * 4LL, PHOP * 4LL))
+            return 1;
+        c->state_layout = state_layout_hash(t);
+    }
 
     const long long recF = c->recF, recS = c->recS;
     const int Kf = c->Kf, Ks = c->Ks;
@@ -799,6 +824,33 @@ int se_fsn_reset_state(se_fsn* c, int first, int count, void* stream) {
     // overlap-add carry of se_fsn_process_chunk
     SE_CUDA_OK(cudaMemsetAsync(c->carry + (size_t)PHOP * first, 0, (size_t)PHOP * count * sizeof(float), st));
     return 0;
+}
+
+int64_t se_fsn_state_bytes_per_stream(const se_fsn* c) { return c ? c->state_tab.record_bytes : -1; }
+
+uint64_t se_fsn_state_layout(const se_fsn* c) { return c ? c->state_layout : 0; }
+
+int se_fsn_state_export(se_fsn* c, const int32_t* rows_host, int n, void* dst_dev, void* stream) {
+    NvtxRange nvtx_range("se.fsn_state_export");
+    SE_REQUIRE(c != nullptr, "null context");
+    if (state_rows_check(rows_host, n, c->maxB, false, "se_fsn_state_export")) return 2;
+    SE_REQUIRE(n == 0 || (dst_dev != nullptr && reinterpret_cast<uintptr_t>(dst_dev) % 16 == 0),
+               "se_fsn_state_export: dst must be a 16-byte aligned device buffer");
+    SE_CUDA_OK(cudaSetDevice(c->device));
+    return launch_state_pack(c->state_tab, rows_host, n, dst_dev, (cudaStream_t)stream);
+}
+
+int se_fsn_state_import(se_fsn* c, const int32_t* rows_host, int n, const void* src_dev, uint64_t layout, void* stream) {
+    NvtxRange nvtx_range("se.fsn_state_import");
+    SE_REQUIRE(c != nullptr, "null context");
+    SE_REQUIRE(layout == c->state_layout,
+               "se_fsn_state_import: record layout mismatch (records from another model, configuration or precision; "
+               "this context:" + c->state_tab.desc + ")");
+    if (state_rows_check(rows_host, n, c->maxB, true, "se_fsn_state_import")) return 2;
+    SE_REQUIRE(n == 0 || (src_dev != nullptr && reinterpret_cast<uintptr_t>(src_dev) % 16 == 0),
+               "se_fsn_state_import: src must be a 16-byte aligned device buffer");
+    SE_CUDA_OK(cudaSetDevice(c->device));
+    return launch_state_unpack(c->state_tab, rows_host, n, src_dev, (cudaStream_t)stream);
 }
 
 int se_fsn_forward_chunk(se_fsn* c, const float* x, float* out, int B, void* stream) {

@@ -601,4 +601,38 @@ int launch_mask_bwd(const MaskBwdParams& p, cudaStream_t st);
 int launch_arena_gather(float* arena, const int* map, const float* theta, long long n, cudaStream_t st);
 int launch_arena_scatter_add(const float* garena, const int* map, float* grad, long long n, cudaStream_t st);
 
+// ---------------------------------------------------------------------------------------------------------------
+// per-stream state export / import (state_io.cu)
+// ---------------------------------------------------------------------------------------------------------------
+// One entry of a context's carried state.  The state of row r is `count` runs of `run` bytes, the u-th at
+// base + r * row_stride + u * unit_stride (count = 1: one contiguous run; count > 1 with a unit_stride that grows with
+// max_streams: the "unit-major" form of the FullSubNet cell states [layer][H][maxB (* F)]).  In a record the entry
+// occupies `run * count` bytes at rec_off, padded to a multiple of 16 with zeros.
+struct StateEntry {
+    char* base;
+    long long row_stride, unit_stride;
+    int run, count;
+    int rec_off;
+    int vec;  // bytes per access: 16 where base, strides and run allow it, else 4
+};
+constexpr int kMaxStateEntries = 24;
+struct StateTable {
+    StateEntry e[kMaxStateEntries];
+    int n = 0;
+    int first_block[kMaxStateEntries + 1];  // filled by the launcher: blocks [first_block[i], first_block[i+1]) serve entry i
+    int record_bytes = 0;                   // multiple of 16
+    std::string desc;                       // what fixes the record's bytes; hashed into the layout (host only)
+};
+// appends an entry (run, row_stride, unit_stride in bytes; multiples of 4) and describes it as `name` with elements of
+// `esz` bytes in t.desc
+int state_table_add(StateTable& t, const std::string& name, int esz, void* base, long long row_stride, long long run,
+                    int count = 1, long long unit_stride = 0);
+// FNV-1a 64 of t.desc: equal layouts <=> byte-compatible records
+uint64_t state_layout_hash(const StateTable& t);
+// host checks of a row list: rows[i] in [0, max_streams), and distinct if `unique`
+int state_rows_check(const int32_t* rows, int n, int max_streams, bool unique, const char* what);
+// record i <-> entries of row rows[i]; records are t.record_bytes apart at rec
+int launch_state_pack(const StateTable& t, const int32_t* rows, int n, void* rec, cudaStream_t st);
+int launch_state_unpack(const StateTable& t, const int32_t* rows, int n, const void* rec, cudaStream_t st);
+
 }  // namespace se

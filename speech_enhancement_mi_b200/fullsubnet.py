@@ -20,8 +20,9 @@ import torch
 import torch.nn as nn
 
 from . import utility
-from . import _host_pipeline, _native
+from . import _host_pipeline, _native, stream_state
 from ._native import SeFsnConfig, check, lib
+from .stream_state import StreamState  # noqa: F401  (the type export_state returns)
 
 EPS = 1e-8
 
@@ -223,6 +224,31 @@ class FullSubNet(BaseModel):
         copies of neighbouring steps overlap the compute.  Returns a CUDA event that completes when ``host_out`` holds
         this chunk's result (call ``.synchronize()`` before reading it).  State semantics are those of process_chunk."""
         return _host_pipeline.process_chunk_host(self, host_chunk, host_out)
+
+    def export_state(self, rows):
+        """Carried state of streams ``rows`` (ints or an int tensor; repeats allowed) -> ``StreamState`` on the
+        context's device (not in the reference): both LSTM layers' h and c of the full-band and every sub-band sequence,
+        both CumLayerNorms and the process_chunk carry.  Runs on the current torch stream of that device and leaves the
+        streams untouched; see ``TemporalCRN.export_state`` for what it serves."""
+        if self._ctx is None:
+            raise RuntimeError("export_state: no streaming context yet (nothing has been processed)")
+        dev = self._ctx_device
+        with torch.cuda.device(dev):
+            return stream_state.export_records(
+                self._ctx, dev, rows, lib().se_fsn_state_bytes_per_stream(self._ctx), lib().se_fsn_state_layout(self._ctx),
+                lib().se_fsn_state_export, _stream(dev), "se_fsn_state_export")
+
+    def import_state(self, state, rows):
+        """Write the records of ``state`` into streams ``rows`` (distinct), as ``TemporalCRN.import_state``: creates
+        the context if there is none, with room for max(max_streams, max(rows) + 1) streams."""
+        rows = stream_state.row_list(rows)
+        dev = self._pick_device(state.data) if self._ctx is None else self._ctx_device
+        ctx = self._ensure_ctx(max(rows, default=-1) + 1, dev, keep_state=True)
+        with torch.cuda.device(dev):
+            stream_state.import_records(
+                ctx, dev, state, rows, lib().se_fsn_state_bytes_per_stream(ctx), lib().se_fsn_state_layout(ctx),
+                lib().se_fsn_state_import, _stream(dev), "se_fsn_state_import")
+        self._fresh = False
 
     def _spectrum(self, x, dev):
         R, M, K = x.shape
