@@ -233,6 +233,14 @@ int se_crn_train_tap_shape(const se_ctx* ctx, int tap, int* C, int* F, int* T);
 int se_crn_train_tap(se_ctx* ctx, int tap, float* out, void* stream);
 int se_crn_train_backward_taps(se_ctx* ctx, const float* dpred, const float* const* dtaps, int n_taps, float* grad_flat,
                                void* stream);
+/* se_crn_train_backward_taps, plus d loss / d mixture of the last se_crn_train_forward (the mixture as an autograd input
+ * of realtime_process; the carried conv buffers and GRU state are detached as in CRN_ELU.py:185,243, so a sample's
+ * gradient comes only from the one or two chunks whose own STFT reads it):
+ *   mixture  [B, M, L], the signal that forward read (its 3-mic spectrum is recomputed)
+ *   dmixture [B, M, L], overwritten; may be NULL (then this is se_crn_train_backward_taps)
+ *   grad_flat may be NULL: parameter-gradient GEMMs are skipped (input gradient only, frozen model) */
+int se_crn_train_backward_input(se_ctx* ctx, const float* mixture, const float* dpred, const float* const* dtaps,
+                                int n_taps, float* grad_flat, float* dmixture, void* stream);
 /* replaces: compute_loss (CRN_ELU.py:513-535) with its backward: source, pred [B,L], length [B] (int32, device) ->
  * out3 (device) = {stoi_loss, cal_si_snr} = {-mean STOI-like score, mean SI-SNR dB} and their gradients w.r.t. pred
  * (d_stoi, d_sisnr: [B,L] each, device).  The caller forms loss = 0.7 * stoi + 0.3 * (-sisnr). */

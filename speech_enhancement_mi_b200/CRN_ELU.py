@@ -90,12 +90,31 @@ class SequenceModel(nn.Module):
 # autograd plumbing of the training micro-step (train.py:195-198).  No arithmetic happens in PyTorch: the two graph
 # nodes below only hand device pointers to se_crn_train_forward / se_crn_train_backward and se_loss_terms_grad.
 # ----------------------------------------------------------------------------------------------------------------
+def _save_mixture(ctx, model, mixture):
+    """Keep the device copy of the mixture the forward reads when its gradient is wanted (the backward recomputes the
+    mixture's 3-mic spectrum from it); returns that copy."""
+    xd = model._to_device(mixture, model._pick_device(mixture))
+    ctx.mixture_meta = (mixture.device, mixture.dtype) if ctx.needs_input_grad[1] else None
+    ctx.save_for_backward(xd if ctx.needs_input_grad[1] else None)
+    return xd
+
+
+def _grads_out(ctx, flat, offsets, dmix):
+    """(None, d mixture, None, *parameter gradients) for the autograd.Function inputs (model, mixture, flag, *params)."""
+    grads = [None] * len(ctx.shapes) if flat is None else \
+        [flat[o:o + s.numel()].view(s) for o, s in zip(offsets, ctx.shapes)]
+    if dmix is not None:
+        device, dtype = ctx.mixture_meta
+        dmix = dmix.to(device=device, dtype=dtype)
+    return (None, dmix, None, *grads)
+
+
 class _RealtimeTrainFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, model, mixture, flag, *params):
         ctx.model = model
         ctx.shapes = [p.shape for p in params]
-        pred = model._train_forward(mixture, flag)
+        pred = model._train_forward(_save_mixture(ctx, model, mixture), flag)
         ctx.fwd_gen = model._fwd_gen  # the training context keeps the activations of its LAST forward only
         return pred
 
@@ -105,9 +124,10 @@ class _RealtimeTrainFn(torch.autograd.Function):
             raise RuntimeError("backward() of a realtime_process result whose activations are gone: another forward ran "
                                "on the model's training context in between (call backward before the next "
                                "realtime_process, as train.py:195-198 does)")
-        flat, offsets = ctx.model._train_backward(dpred)
-        grads = [flat[o:o + s.numel()].view(s) for o, s in zip(offsets, ctx.shapes)]
-        return (None, None, None, *grads)
+        mixture, = ctx.saved_tensors
+        flat, offsets, dmix = ctx.model._train_backward(dpred, mixture=mixture,
+                                                        params=any(ctx.needs_input_grad[3:]))
+        return _grads_out(ctx, flat, offsets, dmix)
 
 
 class _LossTermsFn(torch.autograd.Function):
@@ -454,21 +474,33 @@ class TemporalCRN(nn.Module):
         self._last_chunk_streams = B * n_chunks
         return pred
 
-    def _train_backward(self, dpred, dtaps=None):
+    def _train_backward(self, dpred, dtaps=None, mixture=None, params=True):
+        """-> (flat parameter gradient or None when ``params`` is False, offsets, d mixture or None).  ``mixture``: the
+        device copy of the signal the last _train_forward read; given, d loss / d mixture is computed as well."""
         dev = self._tctx_device
         with torch.cuda.device(dev):
             dp = dpred.detach().to(device=f"cuda:{dev}", dtype=torch.float32).contiguous()
-            flat = torch.empty(lib().se_crn_num_theta(self._tctx), dtype=torch.float32, device=dp.device)
-            if dtaps is None:
-                check(lib().se_crn_train_backward(self._tctx, dp.data_ptr(), flat.data_ptr(), self._stream_ptr(dev)),
-                      "se_crn_train_backward")
-            else:  # gradients of the distillation loss injected at the feature taps (distillation_crn.py:560-565)
+            flat = torch.empty(lib().se_crn_num_theta(self._tctx), dtype=torch.float32, device=dp.device) \
+                if params else None
+            keep = arr = None
+            if dtaps is not None:  # gradients of the distillation loss injected at the feature taps (distillation_crn.py:560-565)
                 keep = [None if g is None else g.detach().to(device=dp.device, dtype=torch.float32).contiguous()
                         for g in dtaps]
                 arr = (C.c_void_p * len(keep))(*[None if g is None else g.data_ptr() for g in keep])
+            if mixture is not None:
+                dmix = torch.empty_like(mixture)
+                check(lib().se_crn_train_backward_input(self._tctx, mixture.data_ptr(), dp.data_ptr(), arr,
+                                                        len(keep) if keep else 0,
+                                                        None if flat is None else flat.data_ptr(), dmix.data_ptr(),
+                                                        self._stream_ptr(dev)), "se_crn_train_backward_input")
+                return flat, self._t_offsets, dmix
+            if dtaps is None:
+                check(lib().se_crn_train_backward(self._tctx, dp.data_ptr(), flat.data_ptr(), self._stream_ptr(dev)),
+                      "se_crn_train_backward")
+            else:
                 check(lib().se_crn_train_backward_taps(self._tctx, dp.data_ptr(), arr, len(keep), flat.data_ptr(),
                                                        self._stream_ptr(dev)), "se_crn_train_backward_taps")
-        return flat, self._t_offsets
+        return flat, self._t_offsets, None
 
     def _train_taps(self):
         """The pre-activation feature taps of the last _train_forward, each [chunks*B, C, F, T]
@@ -491,16 +523,23 @@ class TemporalCRN(nn.Module):
         network, mask, iSTFT and both overlap-adds happen on the device; with CPU tensors (predict.py:48,59-62) the
         host<->device copies are inside the native call as well.
 
-        Under autograd in train mode (train.py:195) the result carries a graph node whose backward is the native
-        backward pass; the forward then runs batched over all chunks (se_crn_train_forward)."""
+        Under autograd in train mode (train.py:195), or in either mode when the mixture requires grad, the result carries
+        a graph node whose backward is the native backward pass (parameters and / or d loss / d mixture, with the
+        carried state detached as in the reference); the forward then runs batched over all chunks
+        (se_crn_train_forward)."""
         B, Cm, L = mixture.shape
         if Cm != self.num_inputs:
             raise ValueError(f"mixture must be [B, {self.num_inputs}, L]")
-        if self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+        if torch.is_grad_enabled() and (mixture.requires_grad or (
+                self.training and any(p.requires_grad for p in self.parameters()))):
             dev = self._pick_device(mixture)
             _, n_chunks = _native.chunk_grid(L + (0 if flag else self.segment_length // 2), self.segment_length)
             self._ensure_train_ctx(self._train_capacity(B, n_chunks), dev, keep_state=bool(flag))
-            return _RealtimeTrainFn.apply(self, mixture, bool(flag), *self._train_params())
+            pred = _RealtimeTrainFn.apply(self, mixture, bool(flag), *self._train_params())
+            if not self.training:  # eval mode: a flag=True continuation finds the state in the training context
+                self._state_owner = "chunk-batch"
+                self._fresh = False
+            return pred
         dev = self._pick_device(mixture)
         # Few streams, many chunks (a file, predict.py:92): the carried state of a chunk is just the tail of the previous
         # chunk's layer inputs (CRN_ELU.py:243), so every layer can run ONCE over all chunks of all streams and only the

@@ -108,6 +108,7 @@ SIGNATURES = {
     "se_crn_train_tap_shape": (_I, [_P, _I, _P, _P, _P]),
     "se_crn_train_tap": (_I, [_P, _I, _P, _P]),
     "se_crn_train_backward_taps": (_I, [_P, _P, _P, _I, _P, _P]),
+    "se_crn_train_backward_input": (_I, [_P, _P, _P, _P, _I, _P, _P, _P]),
     "se_loss_terms_grad": (_I, [_P, _P, _P, _I, _L, _P, _P, _P, _P]),
     "se_axpby_dev": (_I, [_P, _P, _P, _P, _P, _L, _P]),
     "se_clip_adam_step": (_I, [_P, _P, _P, _P, _L, C.c_float, C.c_float, C.c_float, C.c_float, _I, C.c_float,

@@ -281,6 +281,8 @@ struct se_ctx {
     float* sc[4] = {nullptr, nullptr, nullptr, nullptr};  // scratch, 2 * tmp_floats * maxB each
     double* red = nullptr;                                 // [maxB][2]
     float *chunks = nullptr, *dchunks = nullptr, *dspec = nullptr;
+    float* dnoisy = nullptr;  // d loss / d mic-0 spectrum through the mask multiply (input gradient only)
+    bool t_wgrad = true;      // this backward computes parameter gradients (false: d mixture of a frozen model only)
     std::vector<std::pair<void*, size_t>> twins;  // zeroed at the start of every backward
     std::vector<float*> carry_store;              // per state entry: [maxB][count] state kept between flag=True pieces
     int t_nb = 0, t_N = 0, t_front = 0;
@@ -1181,6 +1183,7 @@ int build_ctx(se_ctx* c) {
         if (dev_alloc(c, &c->chunks, (size_t)KCHUNK * maxB)) return 1;
         if (dev_alloc(c, &c->dchunks, (size_t)KCHUNK * maxB)) return 1;
         if (dev_alloc(c, &c->dspec, (size_t)T * NBIN * 2 * maxB)) return 1;
+        if (dev_alloc(c, &c->dnoisy, (size_t)T * NBIN * 2 * maxB)) return 1;
     }
     if (dev_alloc(c, &c->gh, (size_t)3 * H * maxB)) return 1;
     for (int l = 0; l < 2; ++l)
@@ -2370,6 +2373,7 @@ float* garena_of(const se_ctx* c, const void* w) {
 int dense_bwd(se_ctx* c, const Op& op, int B, const float* G, StridedRows gs, float* dA, cudaStream_t st) {
     GemmParams g = op.g;
     g.M = B * op.rows_per_stream;
+    if (!c->t_wgrad) return dA != nullptr ? launch_dgrad(g, G, gs, dA, st, c->bwd_mode) : 0;
     // weight and data gradient read the same G and write disjoint buffers: side by side on two branches, joined before
     // anything downstream may overwrite G (at one piece per rank most of these launches leave SMs idle)
     if (dA != nullptr && c->pipe_stream && c->bwd_overlap) {
@@ -2415,9 +2419,13 @@ int gln_bwd(se_ctx* c, const NormApplyParams& n, int B, int F, const float* y, c
     return launch_gln_bwd(p, st);
 }
 
-int train_backward(se_ctx* c, const float* dpred, const float* const* dtaps, float* grad_flat, cudaStream_t st) {
+// grad_flat == nullptr: no parameter gradient (weight-gradient GEMMs and the arena scatter skipped).  dmixture != nullptr:
+// also d loss / d mixture [nb][3][t_L]; `mixture` is the signal the forward read (its 3-mic spectrum is recomputed).
+int train_backward(se_ctx* c, const float* dpred, const float* const* dtaps, float* grad_flat, const float* mixture,
+                   float* dmixture, cudaStream_t st) {
     SE_REQUIRE(c->t_have_fwd, "se_crn_train_backward: no forward pass to differentiate");
     const int nb = c->t_nb, N = c->t_N, Bp = N * nb, H = c->H, L = c->L, feat = c->feat;
+    c->t_wgrad = grad_flat != nullptr;
     SE_CUDA_OK(cudaMemsetAsync(c->garena, 0, c->warena_floats * sizeof(float), st));
     for (auto& tw : c->twins) SE_CUDA_OK(cudaMemsetAsync(tw.first, 0, tw.second, st));
     float *s0 = c->sc[0], *s1 = c->sc[1], *s2 = c->sc[2], *s3 = c->sc[3];
@@ -2444,6 +2452,7 @@ int train_backward(se_ctx* c, const float* dpred, const float* const* dtaps, flo
         mb.b = c->b_last;
         mb.noisy = c->noisy;
         mb.g = s0;  // [Bp][T][201][2]
+        mb.dnoisy = dmixture != nullptr ? c->dnoisy : nullptr;
         if (launch_mask_bwd(mb, st)) return 1;
     }
     // ---- decoder, last block first --------------------------------------------------------------------------------
@@ -2572,7 +2581,7 @@ int train_backward(se_ctx* c, const float* dpred, const float* const* dtaps, flo
                     return 1;
             }
             gh.out = nullptr;
-            if (launch_wgrad(gh, c->dgh, g3, garena_of(c, gh.W), garena_of(c, gh.bias), st, c->bwd_mode)) return 1;
+            if (c->t_wgrad && launch_wgrad(gh, c->dgh, g3, garena_of(c, gh.W), garena_of(c, gh.bias), st, c->bwd_mode)) return 1;
             if (dense_bwd(c, iop, Bp, c->dgi, g3, l == 1 ? c->dH[0] + H : c->dxg, st)) return 1;
         }
     }
@@ -2606,8 +2615,48 @@ int train_backward(se_ctx* c, const float* dpred, const float* const* dtaps, flo
         if (launch_elu_bwd(s2, r.e, rows * C, st)) return 1;
         if (i == (int)c->conv_recs.size() - 1 && inject_tap(c, dtaps, 0, s2, Bp, st)) return 1;
         const StridedRows g1{(long long)T * r.Fo * C, (long long)r.Fo * C, C};
-        if (dense_bwd(c, cop, Bp, s2, g1, r.need_dgrad ? r.in->dbase : nullptr, st)) return 1;
+        // the first pre-convolution's data gradient lands in the twin of the features (beside its residual path)
+        const bool dgrad = r.need_dgrad || dmixture != nullptr;
+        if (dense_bwd(c, cop, Bp, s2, g1, dgrad ? r.in->dbase : nullptr, st)) return 1;
     }
+    // ---- features -> spectrum -> chunk -> mixture (CRN_ELU.py:369-373,417-424, utility.py:312-370) -------------------
+    // Only the interior frames of the feature twin count: the leading state frames are the previous chunk's features,
+    // detached in the reference (CRN_ELU.py:243), so no gradient crosses chunk state.
+    if (dmixture != nullptr) {
+        IoDesc io{mixture, 3 * c->t_L, c->t_L, -(long long)PHOP - c->t_front, c->t_L, nullptr, 0, 0};
+        if (launch_set_io(c->io_dev, io, st)) return 1;
+        StftParams sp{};
+        sp.io = c->io_dev;
+        sp.B = Bp;
+        sp.M = 3;
+        sp.spec_ref = s0;  // the 3-mic spectrum the forward's features were computed from, [Bp][3][F][T][2]
+        sp.nb = nb;
+        sp.hop_chunk = PHOP;
+        if (launch_stft_features(sp, st)) return 1;
+        const Act& a = c->pre_act[0];
+        FeatBwdParams fb{};
+        fb.B = Bp;
+        fb.student = c->student;
+        fb.dfeat = a.dinterior();
+        fb.fB = a.sB;
+        fb.fC = 1;
+        fb.fT = a.sT;
+        fb.fF = a.sF;
+        fb.dnoisy = c->dnoisy;
+        fb.spec = s0;
+        fb.dspec = s1;
+        if (launch_features_bwd(fb, st)) return 1;
+        MaskIstftParams mp{};  // per (stream, mic) row: the adjoint of framing + window + real DFT -> d chunk [Bp][3][K]
+        mp.B = Bp * 3;
+        mp.spec_in = s1;
+        mp.out_chunk = s2;
+        mp.adjoint = 1;
+        if (launch_mask_istft(mp, st)) return 1;
+        // chunk n of utterance i read mixture[i][m][n*P + j - P - front]: rows (n*nb + i)*3 + m gathered like the output
+        // overlap-add (utterance-mic rows i*3 + m), weight 1, pads and gap dropped
+        if (launch_over_add_cm(s2, 3 * nb, N, KCHUNK, c->t_front, c->t_L, dmixture, st, 1.f)) return 1;
+    }
+    if (grad_flat == nullptr) return 0;
     // ---- packed-arena gradients -> flat vector in the reference layout (registry order) --------------------------------
     SE_CUDA_OK(cudaMemsetAsync(grad_flat, 0, (size_t)c->n_theta * sizeof(float), st));
     return launch_arena_scatter_add(c->garena, c->wmap, grad_flat, (long long)c->warena_floats, st);
@@ -3107,7 +3156,7 @@ int se_crn_train_backward(se_ctx* c, const float* dpred, float* grad_flat, void*
     NvtxRange nvtx_range("se.train_backward");
     if (check_ready(c, 0, true)) return 1;
     SE_REQUIRE(dpred != nullptr && grad_flat != nullptr, "se_crn_train_backward: null buffer");
-    return train_backward(c, dpred, nullptr, grad_flat, (cudaStream_t)stream);
+    return train_backward(c, dpred, nullptr, grad_flat, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 int se_crn_train_num_taps(const se_ctx* c) { return (c && c->train) ? c->L + 1 : 0; }
@@ -3135,7 +3184,18 @@ int se_crn_train_backward_taps(se_ctx* c, const float* dpred, const float* const
     if (check_ready(c, 0, true)) return 1;
     SE_REQUIRE(dpred != nullptr && grad_flat != nullptr, "se_crn_train_backward_taps: null buffer");
     SE_REQUIRE(dtaps == nullptr || n_taps == c->L + 1, "se_crn_train_backward_taps: one gradient slot per feature tap");
-    return train_backward(c, dpred, dtaps, grad_flat, (cudaStream_t)stream);
+    return train_backward(c, dpred, dtaps, grad_flat, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+int se_crn_train_backward_input(se_ctx* c, const float* mixture, const float* dpred, const float* const* dtaps, int n_taps,
+                                float* grad_flat, float* dmixture, void* stream) {
+    NvtxRange nvtx_range("se.train_backward_input");
+    if (check_ready(c, 0, true)) return 1;
+    SE_REQUIRE(dpred != nullptr, "se_crn_train_backward_input: null dpred");
+    SE_REQUIRE(grad_flat != nullptr || dmixture != nullptr, "se_crn_train_backward_input: nothing to compute");
+    SE_REQUIRE(dmixture == nullptr || mixture != nullptr, "se_crn_train_backward_input: d mixture needs the mixture");
+    SE_REQUIRE(dtaps == nullptr || n_taps == c->L + 1, "se_crn_train_backward_input: one gradient slot per feature tap");
+    return train_backward(c, dpred, dtaps, grad_flat, mixture, dmixture, (cudaStream_t)stream);
 }
 
 int se_crn_launches_per_chunk(const se_ctx* c) { return c ? count_launches(c) : 0; }

@@ -438,6 +438,11 @@ __global__ void __launch_bounds__(256, 3) mask_istft_kernel(MaskIstftParams p) {
             float2 e;
             if (p.spec_in != nullptr) {
                 e = reinterpret_cast<const float2*>(p.spec_in)[((long long)b * NBIN + k) * T + t];
+                if (p.adjoint) {  // sum_k Re(D_k e^{+2 pi i k n / N}) = C2R inverse of (N D_0, N/2 D_1 .. N/2 D_199, N D_200)
+                    const float sc = (k == 0 || k == NBIN - 1) ? (float)NFFT : (float)(NFFT / 2);
+                    e.x *= sc;
+                    e.y *= sc;
+                }
             } else {
                 const float2 y = sy[o];  // element (t0 + fr, k) of the stream = o-th of the staged group
                 const float2 x = sx[o];
@@ -555,7 +560,8 @@ __global__ void __launch_bounds__(256, 3) mask_istft_kernel(MaskIstftParams p) {
     // ---- envelope division, trim n_fft/2, chunk-level 50 % overlap-add with the carried half ---------------------
     constexpr int P = K / 2;
     if (p.out_chunk != nullptr) {
-        for (int n = tid; n < K; n += blockDim.x) p.out_chunk[(long long)b * K + n] = s.ola[NFFT / 2 + n] / c_env[n];
+        for (int n = tid; n < K; n += blockDim.x)
+            p.out_chunk[(long long)b * K + n] = p.adjoint ? s.ola[NFFT / 2 + n] : s.ola[NFFT / 2 + n] / c_env[n];
     }
     if (p.carry != nullptr) {
         float* out = p.io->out + b * p.io->out_stream_stride;
@@ -576,7 +582,7 @@ __global__ void __launch_bounds__(256, 3) mask_istft_kernel(MaskIstftParams p) {
 // over_add / iSTFT / mask (the adjoint of the iSTFT is the STFT of dchunk / envelope scaled by c_k / n_fft)
 // ------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) over_add_cm_kernel(const float* __restrict__ chunks, int nb, int N, int front,
-                                                          long long L, float* __restrict__ pred) {
+                                                          long long L, float scale, float* __restrict__ pred) {
     constexpr int P = K / 2;
     const long long total = (long long)nb * L;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
@@ -587,7 +593,7 @@ __global__ void __launch_bounds__(256) over_add_cm_kernel(const float* __restric
         float a = 0.f, b = 0.f;
         if (n1 >= 1 && n1 - 1 < N) a = chunks[((long long)(n1 - 1) * nb + u) * K + (q - (long long)(n1 - 1) * P)];
         if (n1 < N) b = chunks[((long long)n1 * nb + u) * K + (q - (long long)n1 * P)];
-        pred[i] = (a + b) / 2;
+        pred[i] = (a + b) * scale;
     }
 }
 
@@ -639,6 +645,56 @@ __global__ void __launch_bounds__(256) mask_bwd_kernel(MaskBwdParams p) {
         const float dmr = d.x * x.x + d.y * x.y;   // E = M * X (complex): dM = dE * conj(X)
         const float dmi = -d.x * x.y + d.y * x.x;
         reinterpret_cast<float2*>(p.g)[i] = make_float2(dmr * decompress_cirm_grad(m0), dmi * decompress_cirm_grad(m1));
+        if (p.dnoisy != nullptr) {  // E = M * X: dX = dE * conj(M), M the decompressed mask
+            const float mr = decompress_cirm(m0), mi = decompress_cirm(m1);
+            reinterpret_cast<float2*>(p.dnoisy)[i] = make_float2(d.x * mr + d.y * mi, -d.x * mi + d.y * mr);
+        }
+    }
+}
+
+// Adjoint of the input features (CRN_ELU.py:369-373; student phase distillation_crn.py:340), following torch's autograd
+// of the reference expressions: mag_m = sqrt(re^2 + im^2 + 1e-10), ipd_m = angle_0 - angle_m (m = 1, 2); the mic-0
+// spectrum also receives `dnoisy` (the mask multiply).  One thread per (stream, bin, frame), frames fastest.
+__global__ void __launch_bounds__(256) features_bwd_kernel(FeatBwdParams p) {
+    const long long per = (long long)NBIN * T;
+    const long long total = per * p.B;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
+         i += (long long)gridDim.x * blockDim.x) {
+        const int b = (int)(i / per);
+        const int r = (int)(i - b * per);
+        const int k = r / T, t = r - k * T;
+        const float* g = p.dfeat + b * p.fB + t * p.fT + k * p.fF;
+        const float g3 = g[3 * p.fC], g4 = g[4 * p.fC];
+        const float dang[3] = {g3 + g4, -g3, -g4};
+        const float2* spec = reinterpret_cast<const float2*>(p.spec) + (long long)b * 3 * per;
+        float2* dspec = reinterpret_cast<float2*>(p.dspec) + (long long)b * 3 * per;
+#pragma unroll
+        for (int m = 0; m < 3; ++m) {
+            const float2 v = spec[m * per + r];
+            const float re = v.x, im = v.y;
+            const float gm = g[m * p.fC] / sqrtf(re * re + im * im + 1e-10f);
+            float dre = gm * re, dim = gm * im;
+            if (p.student) {  // arctan(u), u = im / (re + 1e-8) + 1e-8
+                const float den = re + 1e-8f;
+                const float u = im / den + 1e-8f;
+                const float du = dang[m] / (1.f + u * u);
+                dim += du / den;
+                dre += -du * im / (den * den);
+            } else {  // atan2(im, re): (re, -im) / |X|^2, exactly 0 at re = im = 0 as torch.atan2's backward
+                const float r2 = re * re + im * im;
+                if (r2 > 0.f) {
+                    const float rc = 1.f / r2;
+                    dim += dang[m] * re * rc;
+                    dre += -dang[m] * im * rc;
+                }
+            }
+            if (m == 0) {
+                const float2 dn = reinterpret_cast<const float2*>(p.dnoisy)[((long long)b * T + t) * NBIN + k];
+                dre += dn.x;
+                dim += dn.y;
+            }
+            dspec[m * per + r] = make_float2(dre, dim);
+        }
     }
 }
 
@@ -710,12 +766,13 @@ int launch_mask_istft(const MaskIstftParams& p, cudaStream_t st) {
     return 0;
 }
 
-int launch_over_add_cm(const float* chunks, int nb, int N, int Kc, int front, long long L, float* pred, cudaStream_t st) {
+int launch_over_add_cm(const float* chunks, int nb, int N, int Kc, int front, long long L, float* pred, cudaStream_t st,
+                       float scale) {
     SE_REQUIRE(Kc == K, "over_add_cm: chunk length must be 3200");
     const long long total = (long long)nb * L;
     if (total <= 0) return 0;
     long long g = (total + 255) / 256;
-    over_add_cm_kernel<<<(int)(g > 2368 ? 2368 : g), 256, 0, st>>>(chunks, nb, N, front, L, pred);
+    over_add_cm_kernel<<<(int)(g > 2368 ? 2368 : g), 256, 0, st>>>(chunks, nb, N, front, L, scale, pred);
     SE_CUDA_OK(cudaGetLastError());
     return 0;
 }
@@ -727,6 +784,15 @@ int launch_over_add_cm_bwd(const float* dpred, int nb, int N, int Kc, int front,
     if (total <= 0) return 0;
     long long g = (total + 255) / 256;
     over_add_cm_bwd_kernel<<<(int)(g > 2368 ? 2368 : g), 256, 0, st>>>(dpred, nb, N, front, L, dchunks);
+    SE_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+int launch_features_bwd(const FeatBwdParams& p, cudaStream_t st) {
+    if (p.B <= 0) return 0;
+    const long long total = (long long)p.B * T * NBIN;
+    long long g = (total + 255) / 256;
+    features_bwd_kernel<<<(int)(g > 2368 ? 2368 : g), 256, 0, st>>>(p);
     SE_CUDA_OK(cudaGetLastError());
     return 0;
 }

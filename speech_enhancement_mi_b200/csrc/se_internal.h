@@ -377,6 +377,10 @@ struct MaskIstftParams {
     float* spec_ref;     // optional enhanced spectrum in the reference layout [B][F][T][2] (forward()); skips iSTFT
     const float* spec_in;  // optional: take the enhanced spectrum [B][F][T][2] from here instead (se_istft_trans)
     int fast;  // tensor-core precisions (tf32 / fp16): decompress_cIRM by two lg2.approx instead of an IEEE division + logf
+    // with spec_in: spec_in is d loss / d (STFT of a chunk) and out_chunk receives d loss / d chunk, the adjoint of the
+    // framing + window + real DFT (per frame sum_k Re(D_k e^{+2 pi i k n / N}) times the window, overlap-added, centre pad
+    // dropped, no envelope division)
+    int adjoint;
 };
 int launch_mask_istft(const MaskIstftParams& p, cudaStream_t st);
 int init_fft_tables();  // uploads twiddles / window / envelope to constant memory of the current device
@@ -581,8 +585,10 @@ int launch_gru_seq_bwd(const GruSeqBwdParams& p, cudaStream_t st);
 int launch_copy_rows(float* dst, long long dB, const float* src, long long sB, int count, int nb, cudaStream_t st);
 
 // chunk-major training layout: stream s = n*b + i is chunk n of utterance i
-// pred[i][j] = (chunk_{q/P-1}[..] + chunk_{q/P}[..]) / 2 at q = j + P + front (utility.py:393-403), j < L
-int launch_over_add_cm(const float* chunks, int nb, int N, int K, int front, long long L, float* pred, cudaStream_t st);
+// pred[i][j] = (chunk_{q/P-1}[..] + chunk_{q/P}[..]) * scale at q = j + P + front (utility.py:393-403), j < L
+// (scale 1: the adjoint of the chunk segmentation, d mixture gathered from the one or two chunks that read each sample)
+int launch_over_add_cm(const float* chunks, int nb, int N, int K, int front, long long L, float* pred, cudaStream_t st,
+                       float scale = 0.5f);
 // adjoint + envelope: dchunk[s][n] = 0.5 * dpred[i][n0*P + n - P - front] / env[n]  (zero outside [0,L))
 int launch_over_add_cm_bwd(const float* dpred, int nb, int N, int K, int front, long long L, float* dchunks,
                            cudaStream_t st);
@@ -595,8 +601,18 @@ struct MaskBwdParams {
     const float *w, *b;
     const float* noisy;   // [B][T][F][2]
     float* g;             // out: d loss / d GLN(y) [B][T][F][2]
+    float* dnoisy;        // optional out: d loss / d noisy [B][T][F][2] through the mask multiply (CRN_ELU.py:401-405)
 };
 int launch_mask_bwd(const MaskBwdParams& p, cudaStream_t st);
+struct FeatBwdParams {  // adjoint of the input features (CRN_ELU.py:369-373, distillation_crn.py:340)
+    int B, student;
+    const float* dfeat;   // d loss / d features, channel c of (b, t, f) at dfeat[b*fB + c*fC + t*fT + f*fF], c < 5
+    long long fB, fC, fT, fF;
+    const float* dnoisy;  // d loss / d mic-0 spectrum from the mask multiply [B][T][F][2]
+    const float* spec;    // the 3-mic spectrum of the chunk [B][3][F][T][2]
+    float* dspec;         // out: d loss / d spectrum [B][3][F][T][2]
+};
+int launch_features_bwd(const FeatBwdParams& p, cudaStream_t st);
 // arena <-> flat parameter vector (map[pos] = 1 + flat index, 0 = padding)
 int launch_arena_gather(float* arena, const int* map, const float* theta, long long n, cudaStream_t st);
 int launch_arena_scatter_add(const float* garena, const int* map, float* grad, long long n, cudaStream_t st);

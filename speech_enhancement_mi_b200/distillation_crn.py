@@ -22,6 +22,7 @@ import torch.nn as nn
 
 from . import _native
 from .CRN_ELU import TemporalCRN as _TemporalCRN
+from .CRN_ELU import _grads_out, _save_mixture
 
 EPS = 1e-8  # distillation_crn.py:13
 
@@ -33,7 +34,7 @@ class _RealtimeTapsFn(torch.autograd.Function):
     def forward(ctx, model, mixture, flag, *params):
         ctx.model = model
         ctx.shapes = [p.shape for p in params]
-        pred = model._train_forward(mixture, flag)
+        pred = model._train_forward(_save_mixture(ctx, model, mixture), flag)
         taps = model._train_taps()
         ctx.fwd_gen = model._fwd_gen
         return (pred, *taps)
@@ -43,9 +44,10 @@ class _RealtimeTapsFn(torch.autograd.Function):
         if ctx.fwd_gen != ctx.model._fwd_gen:
             raise RuntimeError("backward() of a realtime_process result whose activations are gone: another forward ran "
                                "on the model's training context in between")
-        flat, offsets = ctx.model._train_backward(dpred, dtaps)
-        grads = [flat[o:o + s.numel()].view(s) for o, s in zip(offsets, ctx.shapes)]
-        return (None, None, None, *grads)
+        mixture, = ctx.saved_tensors
+        flat, offsets, dmix = ctx.model._train_backward(dpred, dtaps, mixture=mixture,
+                                                        params=any(ctx.needs_input_grad[3:]))
+        return _grads_out(ctx, flat, offsets, dmix)
 
 
 class TemporalCRN(_TemporalCRN):
@@ -64,7 +66,7 @@ class TemporalCRN(_TemporalCRN):
         dev = self._pick_device(mixture)
         _, n_chunks = _native.chunk_grid(L + (0 if flag else self.segment_length // 2), self.segment_length)
         self._ensure_train_ctx(self._train_capacity(B, n_chunks), dev, keep_state=bool(flag))
-        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+        if torch.is_grad_enabled() and (mixture.requires_grad or any(p.requires_grad for p in self.parameters())):
             pred, *taps = _RealtimeTapsFn.apply(self, mixture, bool(flag), *self._train_params())
             return pred, list(taps)
         with torch.no_grad():
