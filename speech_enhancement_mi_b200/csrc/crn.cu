@@ -94,6 +94,10 @@ struct Op {
     std::string label;      // kernel name for reports (se_crn_kernel_info)
     double alg_flops = 0;   // algorithmic FLOPs (2*MACs of the reference op) per stream and chunk
     double alg_bytes = 0;   // algorithmic HBM bytes per stream and chunk: every operand read once, every result written once
+    // fp16 operand mode: alg_bytes counts 4 bytes per element, se_crn_kernel_info scales it by this factor for the tensors
+    // that really are 2 bytes wide (0.5; 0.75 for the last deconv's fp32 output; 1 for the pre-convolution kernels and
+    // the GRU projections / recurrences, which keep fp32 streams)
+    double f16_bytes = 1;
     GemmParams g;
     int rows_per_stream = 0;
     NormApplyParams n;
@@ -109,12 +113,7 @@ struct Op {
     SkipBlendParams sb;
     int em_cin = 0, em_cout = 0;  // channel counts of the mma.sync block kernels (encoder / decoder)
     int small_c = 0;  // channel count of the two small-layer kernels
-    // TMA operand delivery (gemm_tc.cu): geometry of the tensor the A operand is gathered from, [B][Tp][Fp][C] at `tma_base`
-    // with the row grid starting at (frame t_org, bin f_org) and advancing fstep bins per output bin.  C = 0: not described.
-    const void* tma_base = nullptr;
-    int tma_C = 0, tma_Fp = 0, tma_Tp = 0, tma_fstep = 1, tma_t_org = 0, tma_f_org = 0;
-    long long tma_sT = 0, tma_sB = 0;
-    bool tma_ok = false;
+    bool tma_ok = false;  // TMA operand delivery (gemm_tc.cu) with `tma`
     GemmTma tma{};
     // GRU pointwise
     const float* gi = nullptr;
@@ -161,19 +160,6 @@ struct PreBuf {  // channel-planar preconv input [maxB][5][25][Fpp] (se_internal
     float* interior() const { return base + 4 * Fpp + 2 * d; }  // frame 4 (first new frame), bin 0
 };
 
-struct ParamInfo {
-    std::string name;
-    std::vector<int> shape;
-    int64_t numel() const {
-        int64_t n = 1;
-        for (int s : shape) n *= s;
-        return n;
-    }
-};
-
-using HostParams = std::map<std::string, std::vector<float>>;
-using PackFn = std::function<void(const HostParams&, float*)>;  // fills a host mirror of the packed-weight arena
-
 }  // namespace
 }  // namespace se
 
@@ -189,7 +175,7 @@ struct se_ctx {
     std::vector<int> encF;  // F after each encoder level
     int Fg = 0, Cg = 0, feat = 0, H = 0;
 
-    std::vector<ParamInfo> params;
+    WeightArena wa;  // packed weights, their koff tables and the parameter registry
     std::vector<void*> allocs;
 
     // activations
@@ -203,14 +189,6 @@ struct se_ctx {
     int n_stats = 0;
     int stats_last = -1;  // slot of the last deconv's statistics
     const float *w_last = nullptr, *b_last = nullptr;
-
-    // packed weights
-    float* warena = nullptr;
-    size_t warena_floats = 0;
-    int* karena = nullptr;
-    std::vector<int> khost;
-    std::vector<PackFn> packers;
-    bool weights_bound = false;
 
     std::vector<Op> ops;
     RollTable roll{};
@@ -228,7 +206,6 @@ struct se_ctx {
     int ue = 4;         // elements per 16-byte gather unit
     int kblock = 32;    // elements per k-block
     float* h32[2] = {nullptr, nullptr};  // fp16 mode: fp32 master copy of the GRU state [maxB][H] per layer
-    void* warena_h = nullptr;            // fp16 mode: the weight arena converted to fp16 (same indexing)
     float* E(float* base, long long elems) const {  // element offset into an operand buffer
         return reinterpret_cast<float*>(reinterpret_cast<char*>(base) + elems * esz);
     }
@@ -253,7 +230,6 @@ struct se_ctx {
     bool use_tma = true;  // SE_B200_TMA=0: every tcgen05 GEMM keeps the cp.async gather producers
     __half* feat_h = nullptr;     // features of the chunk [maxB][21][224][8] halves (borders stay zero)
     __half* pre_state = nullptr;  // carried frames of the three pre-convolutions [maxB][3][4][224][8] halves
-    size_t pre3_w_off[3] = {0, 0, 0};
     bool b2b_gate = true;      // SE_B200_B2B=0: 32- / 64-channel gates as separate GEMMs
     bool small_layers = true;  // SE_B200_SMALL_LAYERS=0: keep the two small-channel layers on the GEMM path (A/B switch)
     unsigned tc_mask = 0xffffffffu;  // SE_B200_TC_MASK: bit per Stage that may use the tensor-core GEMM (debug)
@@ -273,8 +249,8 @@ struct se_ctx {
     std::vector<ConvRec> conv_recs;       // preconv 0..2, encoder 0..L-1
     std::vector<DeconvRec> deconv_recs;   // decoder 0..L-1
     GruRec gru_rec;
-    float* garena = nullptr;  // gradient twin of warena
-    int* wmap = nullptr;      // warena position -> 1 + index into the flat parameter vector (0: padding)
+    float* garena = nullptr;  // gradient twin of the weight arena
+    int* wmap = nullptr;      // weight-arena position -> 1 + index into the flat parameter vector (0: padding)
     std::vector<int64_t> param_off;
     int64_t n_theta = 0;
     float *dxg = nullptr, *dH[2] = {nullptr, nullptr}, *dhrec = nullptr, *dgi = nullptr, *dgh = nullptr, *gh_all = nullptr;
@@ -293,31 +269,9 @@ struct se_ctx {
     // staging for the host variant
     float *h_in = nullptr, *h_out = nullptr;
     size_t h_in_floats = 0, h_out_floats = 0;
-
-    size_t reserve_w(size_t n) {
-        size_t off = warena_floats;
-        warena_floats += (n + 3) / 4 * 4;
-        return off;
-    }
-    int reserve_k(const std::vector<int>& v) {  // padded with offset-0 units to whole 32-float k-blocks (weights there: 0)
-        int off = (int)khost.size();
-        khost.insert(khost.end(), v.begin(), v.end());
-        while ((khost.size() - off) % 8) khost.push_back(0);
-        return off;
-    }
 };
 
 namespace {
-
-template <typename Tp>
-int dev_alloc(se_ctx* c, Tp** out, size_t count) {
-    void* p = nullptr;
-    SE_CUDA_OK(cudaMalloc(&p, count * sizeof(Tp)));
-    SE_CUDA_OK(cudaMemset(p, 0, count * sizeof(Tp)));
-    c->allocs.push_back(p);
-    *out = reinterpret_cast<Tp*>(p);
-    return 0;
-}
 
 int make_act(se_ctx* c, Act& a, int C, int F, int Tn, int padT0, int padT1, int padF0, int padF1) {
     a.C = C;
@@ -337,7 +291,7 @@ int make_act(se_ctx* c, Act& a, int C, int F, int Tn, int padT0, int padT1, int 
 
 // ---- parameter registry (order of TemporalCRN.state_dict() without the `net.0` aliases; CRN_ELU.py:335-365) -------
 void register_params(se_ctx* c) {
-    auto add = [&](const std::string& n, std::vector<int> s) { c->params.push_back({n, std::move(s)}); };
+    auto add = [&](const std::string& n, std::vector<int> s) { c->wa.params.push_back({n, std::move(s)}); };
     const se_crn_config& g = c->cfg;
     auto conv_block = [&](const std::string& p, int ci, int co, int kf, int kt) {
         add(p + ".conv.weight", {co, ci, kf, kt});
@@ -392,51 +346,99 @@ PackedW reserve_packed(se_ctx* c, int N, int K) {
     PackedW pw;
     pw.Npad = round_up(N, gemm_tf32_tile_n(N));
     pw.K = round_up(K, c->kblock);
-    pw.w_off = c->reserve_w((size_t)pw.Npad * pw.K);
-    pw.b_off = c->reserve_w(pw.Npad);
+    pw.w_off = c->wa.reserve_w((size_t)pw.Npad * pw.K);
+    pw.b_off = c->wa.reserve_w(pw.Npad);
     return pw;
 }
 
-void fill_gemm_common(se_ctx* c, GemmParams& g, const PackedW& pw, int N, int koff_off) {
-    g.W = nullptr;  // patched after arena allocation (offsets kept in out-of-band vectors)
+void fill_gemm_common(se_ctx* c, GemmParams& g, const PackedW& pw, int N) {
     g.K = pw.K;
     g.N = N;
     g.Npad = pw.Npad;
     g.a_half = c->half ? 1 : 0;
-    (void)koff_off;
 }
-
-}  // namespace
-
-// The program builder keeps arena offsets until the arenas exist; these two vectors remember, per op, where its
-// packed weights / koff table start.
-struct OpFix {
-    size_t w_off, b_off;
-    int k_off;
-    size_t nw_off, nb_off, nwr_off, nbr_off;  // norm affine offsets (SIZE_MAX = unused)
-    size_t w2_off = (size_t)-1, b2_off = (size_t)-1;  // fused gate weights of EPI_ELU_GATE
-};
-
-namespace {
 
 constexpr size_t NONE = (size_t)-1;
 
+// geometry of the tensor a GEMM's A operand is gathered from, [B][Tp][Fp][C] at `base`, with the row grid starting at
+// (frame t_org, bin f_org) and advancing fstep bins per output bin (TMA operand delivery).  C = 0: not described.
+struct TmaSrc {
+    const void* base = nullptr;
+    int C = 0, Fp = 0, Tp = 0;
+    long long sT = 0, sB = 0;
+    int fstep = 1, t_org = 0, f_org = 0;
+};
+
+// points a GEMM op at its packed weights, bias, koff table and (EPI_ELU_GATE) fused gate weights
+int bind_gemm(se_ctx* c, Op& op, const PackedW& pw, int k_off, size_t w2_off, size_t b2_off, const TmaSrc& ts) {
+    const WeightArena& wa = c->wa;
+    op.g.W = (c->half && op.g.a_half) ? static_cast<const void*>(wa.wh + pw.w_off)
+                                      : static_cast<const void*>(wa.w + pw.w_off);
+    op.g.bias = wa.w + pw.b_off;
+    op.g.koff = wa.k + k_off;
+    if (w2_off != NONE) {
+        op.g.W2 = wa.w + w2_off;
+        op.g.bias2 = wa.w + b2_off;
+    }
+    // TMA delivery where every k-block of the gather is 64 contiguous channels of one (frame, bin) tap
+    if (c->use_tma && ts.C > 0 && ts.C % 64 == 0 && op.g.a_half) {
+        GemmParams probe = op.g;
+        probe.M = op.rows_per_stream;
+        const int nkb = op.g.K / 64;
+        std::vector<int> kc(4 * nkb, 0);
+        bool ok = gemm_tma_supported(probe) && op.g.Fo * op.g.Tn == op.rows_per_stream;
+        for (int kb = 0; kb < nkb && ok; ++kb) {
+            const int e = wa.khost[k_off + 8 * kb];
+            for (int j = 1; j < 8; ++j) ok = ok && wa.khost[k_off + 8 * kb + j] == e + 8 * j;
+            kc[4 * kb + 2] = (int)(e / ts.sT);
+            const int rem = (int)(e % ts.sT);
+            kc[4 * kb + 1] = rem / ts.C;
+            kc[4 * kb] = rem % ts.C;
+            ok = ok && kc[4 * kb] % 64 == 0;
+        }
+        // weights beyond the real K are zero, but their k-blocks must still address valid channels: the padding
+        // units of the koff table point at offset 0 (frame 0, bin 0, channel 0), which the loop above maps there
+        if (ok) {
+            int* kdev = nullptr;
+            if (dev_alloc(c, &kdev, kc.size())) return 1;
+            SE_CUDA_OK(cudaMemcpy(kdev, kc.data(), kc.size() * sizeof(int), cudaMemcpyHostToDevice));
+            if (make_gemm_tma(&op.tma, ts.base, ts.C, ts.Fp, ts.Tp, ts.sT, ts.sB, c->maxB, op.g.Fo, ts.fstep, op.g.Tn,
+                              op.g.W, op.g.K, op.g.Npad, gemm_tma_tile_n(op.g)))
+                return 1;
+            op.tma.t_org = ts.t_org;
+            op.tma.f_org = ts.f_org;
+            op.tma.kcoord = reinterpret_cast<const int4*>(kdev);
+            op.tma_ok = true;
+        }
+    }
+    return 0;
+}
+
 struct Builder {
     se_ctx* c;
-    std::vector<OpFix> fix;
     std::string m_label;  // meta of the next pushed op
-    double m_flops = 0, m_bytes = 0;
-    void meta(const std::string& label, double flops, double bytes) {
+    double m_flops = 0, m_bytes = 0, m_f16 = 0.5;
+    void meta(const std::string& label, double flops, double bytes, double f16_bytes = 0.5) {
         m_label = label;
         m_flops = flops;
         m_bytes = bytes;
+        m_f16 = f16_bytes;
     }
-    void take_meta(Op& op) {
+    // appends `op` with the pending meta(); `bind` points it at its packed weights once the arena exists.  Returns its
+    // index in se_ctx::ops.
+    int push(Op op, std::function<int(Op&)> bind = nullptr) {
         op.label = m_label;
         op.alg_flops = m_flops;
         op.alg_bytes = m_bytes;
-        m_label.clear();
-        m_flops = m_bytes = 0;
+        op.f16_bytes = m_f16;
+        meta("", 0, 0);
+        c->ops.push_back(op);
+        const int i = (int)c->ops.size() - 1;
+        if (bind) {
+            se_ctx* cc = c;
+            c->wa.binds.push_back([cc, i, bind] { return bind(cc->ops[i]); });
+        }
+        return i;
     }
 
     // identity koff for a dense K-contiguous operand
@@ -444,35 +446,21 @@ struct Builder {
         const int U = c->ue;
         std::vector<int> v(K / U);
         for (int u = 0; u < K / U; ++u) v[u] = U * u;
-        return c->reserve_k(v);
+        return c->wa.reserve_k(v);
     }
 
-    void push_gemm(int stage, GemmParams g, int rows_per_stream, const PackedW& pw, int k_off, size_t w2_off = NONE,
-                   size_t b2_off = NONE) {
+    // ts: the tensor the A operand is gathered from, for TMA delivery
+    int push_gemm(int stage, GemmParams g, int rows_per_stream, const PackedW& pw, int k_off, TmaSrc ts = {},
+                  size_t w2_off = NONE, size_t b2_off = NONE, OpKind kind = OP_GEMM) {
         Op op{};
-        op.kind = OP_GEMM;
+        op.kind = kind;
         op.stage = stage;
         op.g = g;
         op.rows_per_stream = rows_per_stream;
-        take_meta(op);
-        c->ops.push_back(op);
-        fix.push_back({pw.w_off, pw.b_off, k_off, NONE, NONE, NONE, NONE, w2_off, b2_off});
+        se_ctx* cc = c;
+        return push(op, [=](Op& o) { return bind_gemm(cc, o, pw, k_off, w2_off, b2_off, ts); });
     }
     bool tc_stage(int stage) const { return c->tf32 && ((c->tc_mask >> stage) & 1u); }
-    // describes, for the op pushed last, the tensor its A operand is gathered from (see Op::tma_*)
-    void tma_src(const void* base, int C, int Fp, int Tp, long long sT, long long sB, int fstep = 1, int t_org = 0,
-                 int f_org = 0) {
-        Op& op = c->ops.back();
-        op.tma_base = base;
-        op.tma_C = C;
-        op.tma_Fp = Fp;
-        op.tma_Tp = Tp;
-        op.tma_sT = sT;
-        op.tma_sB = sB;
-        op.tma_fstep = fstep;
-        op.tma_t_org = t_org;
-        op.tma_f_org = f_org;
-    }
     // inference: the per-layer temporaries share four buffers; training: every layer keeps its own (saved for backward)
     float* tmp_buf(float* shared, size_t floats_per_stream) {
         if (!c->train) return shared;
@@ -480,20 +468,25 @@ struct Builder {
         if (dev_alloc(c, &p, floats_per_stream * c->maxB)) c->alloc_failed = true;
         return p;
     }
-    void push_norm(int stage, NormApplyParams n, size_t w_off, size_t b_off, size_t wr_off = NONE,
-                   size_t br_off = NONE) {
+    int push_norm(int stage, NormApplyParams n, size_t w_off, size_t b_off, size_t wr_off = NONE, size_t br_off = NONE) {
         Op op{};
         op.kind = OP_NORM;
         op.stage = stage;
         op.n = n;
         op.n.out_half = c->half ? 1 : 0;  // every normalised tensor is the operand of a following GEMM
         op.n.in_half = c->half ? 1 : 0;   // ... and the pre-norm tensors are stored as fp16 too
-        take_meta(op);
-        c->ops.push_back(op);
-        fix.push_back({NONE, NONE, -1, w_off, b_off, wr_off, br_off});
+        se_ctx* cc = c;
+        return push(op, [=](Op& o) {
+            o.n.w = cc->wa.w + w_off;
+            o.n.b = cc->wa.w + b_off;
+            if (wr_off != NONE) {
+                o.n.wr = cc->wa.w + wr_off;
+                o.n.br = cc->wa.w + br_off;
+            }
+            return 0;
+        });
     }
-    void push_gru_pw(const float* gi, long long giB, const float* gh, const float* hprev, long long hB, float* hout,
-                     int H) {
+    int push_gru_pw(const float* gi, long long giB, const float* gh, const float* hprev, long long hB, float* hout, int H) {
         Op op{};
         op.kind = OP_GRU_PW;
         op.stage = ST_GRU;
@@ -504,19 +497,43 @@ struct Builder {
         op.hB = hB;
         op.hout = hout;
         op.H = H;
-        take_meta(op);
-        c->ops.push_back(op);
-        fix.push_back({NONE, NONE, -1, NONE, NONE, NONE, NONE});
+        return push(op);
     }
 
     // per-channel affine [Cp] (zero beyond the real channels) -> arena
     size_t pack_affine(const std::string& key, int Creal, int Cp) {
-        const size_t off = c->reserve_w(Cp);
-        c->packers.push_back([=](const HostParams& hp, float* arena) {
+        const size_t off = c->wa.reserve_w(Cp);
+        c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
             const std::vector<float>& v = hp.at(key);
             for (int i = 0; i < Cp; ++i) arena[off + i] = i < Creal ? v[i] : 0.f;
         });
         return off;
+    }
+
+    // one pre-convolution block in the PRECONV_W_* layout (se_internal.h) -> arena
+    size_t pack_preconv_block(const std::string& name) {
+        const size_t w_off = c->wa.reserve_w(PRECONV_W_FLOATS);
+        c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
+            const std::vector<float>& w = hp.at(name + ".conv.weight");  // [Co][Ci][KF][KT]
+            float* a = arena + w_off;
+            for (int kt = 0; kt < 5; ++kt)
+                for (int ci = 0; ci < 5; ++ci)
+                    for (int kf = 0; kf < 5; ++kf)
+                        for (int co = 0; co < 5; ++co)
+                            a[(kt * 5 + ci) * 28 + kf * 5 + co] = w[((co * 5 + ci) * 5 + kf) * 5 + kt];
+            for (int co = 0; co < 5; ++co) {
+                a[PRECONV_W_BIAS + co] = hp.at(name + ".conv.bias")[co];
+                for (int k = 0; k < 5; ++k) {
+                    a[PRECONV_W_WT + co * 5 + k] = hp.at(name + ".conv_trans.weight")[co * 5 + k];
+                    a[PRECONV_W_WG + co * 5 + k] = hp.at(name + ".conv_gated.weight")[co * 5 + k];
+                }
+                a[PRECONV_W_BT + co] = hp.at(name + ".conv_trans.bias")[co];
+                a[PRECONV_W_BG + co] = hp.at(name + ".conv_gated.bias")[co];
+                a[PRECONV_W_NW + co] = hp.at(name + ".norm.weight")[co];
+                a[PRECONV_W_NB + co] = hp.at(name + ".norm.bias")[co];
+            }
+        });
+        return w_off;
     }
 
     // ---- causal gated conv block (CRN_ELU.py:230-247) ---------------------------------------------------------
@@ -560,9 +577,9 @@ struct Builder {
                     for (int cu = 0; cu < Cp_in / U; ++cu)
                         koff[((kt * KF + kf) * Cp_in) / U + cu] =
                             (int)(kt * dilT * in.sT + kf * dilF * in.sF + U * cu);
-            const int k_off = c->reserve_k(koff);
+            const int k_off = c->wa.reserve_k(koff);
             PackedW pw = reserve_packed(c, Cout_real, K);
-            c->packers.push_back([=](const HostParams& hp, float* arena) {
+            c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
                 const std::vector<float>& w = hp.at(name + ".conv.weight");  // [Co][Ci][KF][KT]
                 const std::vector<float>& b = hp.at(name + ".conv.bias");
                 for (int n = 0; n < Cout_real; ++n) {
@@ -576,9 +593,9 @@ struct Builder {
             });
             size_t w2_off = NONE, b2_off = NONE;
             if (fuse_gate) {
-                w2_off = c->reserve_w((size_t)2 * Cout_real * w2_pitch);
-                b2_off = c->reserve_w((size_t)2 * Cout_real);
-                c->packers.push_back([=](const HostParams& hp, float* arena) {
+                w2_off = c->wa.reserve_w((size_t)2 * Cout_real * w2_pitch);
+                b2_off = c->wa.reserve_w((size_t)2 * Cout_real);
+                c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
                     const std::vector<float>& wt = hp.at(name + ".conv_trans.weight");
                     const std::vector<float>& bt = hp.at(name + ".conv_trans.bias");
                     const std::vector<float>& wg = hp.at(name + ".conv_gated.weight");
@@ -600,7 +617,7 @@ struct Builder {
             g.sF = (long long)strideF * in.sF;
             g.Tn = T;
             g.Fo = Fo;
-            fill_gemm_common(c, g, pw, Cout_real, k_off);
+            fill_gemm_common(c, g, pw, Cout_real);
             g.epi = fuse_gate ? EPI_ELU_GATE : EPI_ELU;
             g.out = fuse_gate ? tmp_y : tmp_e;
             g.oB = (long long)rows * Cp_out;
@@ -626,9 +643,9 @@ struct Builder {
                 if (use_tc) {  // the two B operands of enc_tc.cu, element for element in its shared-memory order
                     const int CI = Cp_in, CO = Cout_real, HP = CI / 16;
                     const size_t n1 = (size_t)15 * HP * 2 * CO * 8, n2 = (size_t)(CO / 16) * 2 * (2 * CO) * 8;
-                    w1c_off = (c->reserve_w(n1 + 8) + 7) / 8 * 8;  // 16-byte aligned in the fp16 copy of the arena (cp.async)
-                    w2c_off = (c->reserve_w(n2 + 8) + 7) / 8 * 8;
-                    c->packers.push_back([=](const HostParams& hp, float* arena) {
+                    w1c_off = (c->wa.reserve_w(n1 + 8) + 7) / 8 * 8;  // 16-byte aligned in the fp16 copy of the arena (cp.async)
+                    w2c_off = (c->wa.reserve_w(n2 + 8) + 7) / 8 * 8;
+                    c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
                         const std::vector<float>& w = hp.at(name + ".conv.weight");  // [Co][Ci][KF][KT]
                         const std::vector<float>& wt = hp.at(name + ".conv_trans.weight");
                         const std::vector<float>& wg = hp.at(name + ".conv_gated.weight");
@@ -664,26 +681,36 @@ struct Builder {
                 op.em.student = c->student;
                 op.em_cin = Cp_in;
                 op.em_cout = Cout_real;
-                op.label = name + ".conv+elu+gate+gln";
-                op.alg_flops = 2.0 * rows * Cout_real * (KT * KF * Cin_real) + 4.0 * rows * Cout_real * Cout_real;
-                op.alg_bytes = 4.0 * Cin_real * in.Tp * in.F + 4.0 * rows * Cout_real;
-                m_label.clear();
-                m_flops = m_bytes = 0;
-                c->ops.push_back(op);
-                fix.push_back({pw.w_off, pw.b_off, -1, nw_off, nb_off, w1c_off, w2c_off, w2_off, b2_off});
+                meta(name + ".conv+elu+gate+gln",
+                     2.0 * rows * Cout_real * (KT * KF * Cin_real) + 4.0 * rows * Cout_real * Cout_real,
+                     4.0 * Cin_real * in.Tp * in.F + 4.0 * rows * Cout_real);
+                se_ctx* cc = c;
+                push(op, [=](Op& o) {
+                    const WeightArena& wa = cc->wa;
+                    if (use_tc) {
+                        o.em.w1c = wa.wh + w1c_off;
+                        o.em.w2c = wa.wh + w2c_off;
+                    }
+                    o.em.w = wa.w + pw.w_off;
+                    o.em.bias = wa.w + pw.b_off;
+                    o.em.w2 = wa.w + w2_off;
+                    o.em.bias2 = wa.w + b2_off;
+                    o.em.nw = wa.w + nw_off;
+                    o.em.nb = wa.w + nb_off;
+                    return 0;
+                });
                 return;
             }
-            push_gemm(stage, g, rows, pw, k_off, w2_off, b2_off);
-            rec.op_conv = (int)c->ops.size() - 1;
+            rec.op_conv = push_gemm(stage, g, rows, pw, k_off, TmaSrc{in.base, in.C, in.Fp, in.Tp, in.sT, in.sB, strideF},
+                                    w2_off, b2_off);
             c->ops.back().state_entry = state_entry;
-            tma_src(in.base, in.C, in.Fp, in.Tp, in.sT, in.sB, strideF);
         }
         // (2) gated 1x1 pair + statistics -> tmp_y [B][T][Fo][Cp_out]
         if (!fuse_gate) {
             const int K = Cp_out;
             const int k_off = koff_dense(K);
             PackedW pw = reserve_packed(c, 2 * Cout_real, K);
-            c->packers.push_back([=](const HostParams& hp, float* arena) {
+            c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
                 const std::vector<float>& wt = hp.at(name + ".conv_trans.weight");
                 const std::vector<float>& bt = hp.at(name + ".conv_trans.bias");
                 const std::vector<float>& wg = hp.at(name + ".conv_gated.weight");
@@ -704,7 +731,7 @@ struct Builder {
             g.sF = Cp_out;
             g.Tn = T;
             g.Fo = Fo;
-            fill_gemm_common(c, g, pw, 2 * Cout_real, k_off);
+            fill_gemm_common(c, g, pw, 2 * Cout_real);
             g.epi = EPI_GATE_STATS;
             g.out = tmp_y;
             g.oB = g.sB;
@@ -714,9 +741,8 @@ struct Builder {
             g.stats = stats;
             g.out_half = c->half ? 1 : 0;
             meta(name + ".gate1x1", 4.0 * rows * Cout_real * Cout_real, 8.0 * rows * Cout_real);
-            push_gemm(stage, g, rows, pw, k_off);
-            rec.op_gate = (int)c->ops.size() - 1;
-            tma_src(tmp_e, Cp_out, Fo, T, (long long)Fo * Cp_out, (long long)rows * Cp_out);
+            rec.op_gate = push_gemm(stage, g, rows, pw, k_off,
+                                    TmaSrc{tmp_e, Cp_out, Fo, T, (long long)Fo * Cp_out, (long long)rows * Cp_out});
         }
         // (3) GlobalLayerNorm (+ residual) -> destination
         {
@@ -744,251 +770,109 @@ struct Builder {
             const size_t w_off = pack_affine(name + ".norm.weight", Cout_real, Cp_out);
             const size_t b_off = pack_affine(name + ".norm.bias", Cout_real, Cp_out);
             meta(name + ".gln" + (residual ? "+residual" : ""), 0, (residual ? 12.0 : 8.0) * rows * Cout_real);
-            push_norm(stage, n, w_off, b_off);
-            rec.op_norm = (int)c->ops.size() - 1;
+            rec.op_norm = push_norm(stage, n, w_off, b_off);
         }
         if (c->train) c->conv_recs.push_back(rec);
     }
 
     // ---- transposed conv block (CRN_ELU.py:290-307) ---------------------------------------------------------
-    // in: [T + 2d][Fin + 2][Cin]; skip: padded encoder-input buffer whose interior is the skip tensor (or null)
+    // in: [T + 2d][Fin + 2][Cin]; skip: padded encoder-input buffer whose interior is the skip tensor (or null).
+    // The weights of every form are packed first (deconv, skip pair, the four affines); then the form is chosen and
+    // only its ops are pushed.
     void deconv_block(const std::string& name, const Act& in, int Cin, int Cout_real, int KT, int d, const Act* skip,
                       float* dst, long long dB, long long dT, long long dF, int stats_slot, int stats_slot_r,
                       float* dgrad_dst = nullptr) {
         const int Fin = in.F;
         const int Fy = 2 * Fin - 1;
+        const int Fs = skip ? skip->F : Fy;
+        const int rows = T * Fs;
         const int Cop = Cout_real < 4 ? Cout_real : round_up(Cout_real, 4);  // last layer keeps 2 (float2 consumer)
         float* y = skip ? tmp_buf(c->tmp_y, (size_t)T * Fy * Cop) : c->ylast;
+        float* const tmp_rm = skip ? tmp_buf(c->tmp_rm, (size_t)rows * Cop) : nullptr;
+        float* const tmp_rr = skip ? tmp_buf(c->tmp_rr, (size_t)rows * Cop) : nullptr;
+        double* const stats = c->stats + (size_t)stats_slot * 2 * c->maxB;
+        double* const stats_r = skip ? c->stats + (size_t)stats_slot_r * 2 * c->maxB : nullptr;
         DeconvRec rec;
         rec.in = &in;
         rec.skip = skip;
         rec.y = y;
-        rec.Cop = Cop;
-        rec.Fy = Fy;
-        rec.Fs = skip ? skip->F : Fy;
-        rec.gout = dgrad_dst;
-        rec.gs = StridedRows{dB, dT, dF};
-        {
-            // Both output parities in one GEMM.  Output bin phi = 2f' (even) uses taps kf = 0,2,4 and phi = 2f'+1 (odd)
-            // taps kf = 1,3, all on the padded input rows f'+2-j (j = kf/2): the odd half re-uses the rows gathered for
-            // the even half.  Columns: [even channels | odd channels] = 2*Cout contiguous floats of y at bin 2f'.  The
-            // odd half of the last row (phi = 2*Fin-1 = Fy) does not exist: GemmParams::odd_tail masks it.
-            const int nkf = 3;
-            const int Fo = Fin;
-            const int K = KT * nkf * Cin;
-            const int U = c->ue;
-            std::vector<int> koff(K / U);
-            for (int kt = 0; kt < KT; ++kt)
-                for (int j = 0; j < nkf; ++j)
-                    for (int cu = 0; cu < Cin / U; ++cu) {
-                        const long long frame = (long long)(KT - 1 - kt) * d;
-                        koff[((kt * nkf + j) * Cin) / U + cu] = (int)(frame * in.sT + (2 - j) * in.sF + U * cu);
-                    }
-            const int k_off = c->reserve_k(koff);
-            PackedW pw = reserve_packed(c, 2 * Cout_real, K);
-            const int KF = 5;
-            c->packers.push_back([=](const HostParams& hp, float* arena) {
-                const std::vector<float>& w = hp.at(name + ".conv.weight");  // [Ci][Co][KF][KT]
-                const std::vector<float>& b = hp.at(name + ".conv.bias");
-                for (int parity = 0; parity < 2; ++parity)
-                    for (int co = 0; co < Cout_real; ++co) {
-                        const int n = parity * Cout_real + co;
-                        for (int kt = 0; kt < KT; ++kt)
-                            for (int j = 0; j < nkf; ++j) {
-                                const int kf = 2 * j + parity;
-                                if (kf >= KF) continue;  // odd rows have no third tap: weights stay zero
-                                for (int ci = 0; ci < Cin; ++ci)
-                                    arena[pw.w_off + (size_t)n * pw.K + (kt * nkf + j) * Cin + ci] =
-                                        w[((ci * Cout_real + co) * KF + kf) * KT + kt];
-                            }
-                        arena[pw.b_off + n] = b[co];
-                    }
-            });
-            GemmParams g{};
-            g.A = in.base;  // padded row 0, frame 0
-            g.sB = in.sB;
-            g.sT = in.sT;
-            g.sF = in.sF;
-            g.Tn = T;
-            g.Fo = Fo;
-            fill_gemm_common(c, g, pw, 2 * Cout_real, k_off);
-            g.epi = EPI_ELU_STATS;
-            g.out = y;
-            g.oB = (long long)T * Fy * Cop;
-            g.oT = (long long)Fy * Cop;
-            g.oF = 2 * Cop;
-            g.odd_tail = 1;
-            g.out_half = (c->half && skip) ? 1 : 0;  // the last layer's output feeds the mask kernel in fp32
-            g.stats = c->stats + (size_t)stats_slot * 2 * c->maxB;
-            g.vec4 = Cop % 4 == 0;
-            // ConvTranspose2d counted over the T kept frames: even bins 3 taps, odd bins 2 taps
-            meta(name + ".deconv+elu", 2.0 * T * (3.0 * Fin + 2.0 * (Fin - 1)) * KT * Cin * Cout_real,
-                 4.0 * Cin * T * Fin + 4.0 * T * Fy * Cout_real);
-            push_gemm(ST_DECODER, g, T * Fo, pw, k_off);
-            rec.op_deconv = (int)c->ops.size() - 1;
-            tma_src(in.base, in.C, in.Fp, in.Tp, in.sT, in.sB);
-            if (c->half && !c->train && !skip && Cout_real == 2 && KT == 3 && deconv_last_supported(Cin) &&
-                c->small_layers) {
-                Op& op = c->ops.back();  // same packed weights and report entry, served by the direct kernel
-                op.kind = OP_DECONV_LAST;
-                op.small_c = Cin;
-                op.dl = DeconvLastParams{};
-                op.dl.in = reinterpret_cast<const __half*>(in.base);
-                op.dl.sB = in.sB;
-                op.dl.sT = in.sT;
-                op.dl.sF = in.sF;
-                op.dl.Fin = Fin;
-                op.dl.d = d;
-                op.dl.Kp = pw.K;
-                op.dl.y = y;
-                op.dl.stats = g.stats;
-            }
-        }
-        if (!skip) {
-            if (c->train) c->deconv_recs.push_back(rec);
-            return;
-        }
-        const int Fs = skip->F;
-        const int rows = T * Fs;
-        float* const tmp_rm = tmp_buf(c->tmp_rm, (size_t)rows * Cop);
-        float* const tmp_rr = tmp_buf(c->tmp_rr, (size_t)rows * Cop);
         rec.rm = tmp_rm;
         rec.rr = tmp_rr;
-        {  // residual mask / residual 1x1 pair on the skip tensor
-            const int K = skip->C;
-            const int k_off = koff_dense(K);
-            PackedW pw = reserve_packed(c, 2 * Cout_real, K);
-            c->packers.push_back([=](const HostParams& hp, float* arena) {
+        rec.Cop = Cop;
+        rec.Fy = Fy;
+        rec.Fs = Fs;
+        rec.gout = dgrad_dst;
+        rec.gs = StridedRows{dB, dT, dF};
+        // Both output parities in one GEMM.  Output bin phi = 2f' (even) uses taps kf = 0,2,4 and phi = 2f'+1 (odd)
+        // taps kf = 1,3, all on the padded input rows f'+2-j (j = kf/2): the odd half re-uses the rows gathered for
+        // the even half.  Columns: [even channels | odd channels] = 2*Cout contiguous floats of y at bin 2f'.  The
+        // odd half of the last row (phi = 2*Fin-1 = Fy) does not exist: GemmParams::odd_tail masks it.
+        const int nkf = 3;
+        const int K = KT * nkf * Cin;
+        const int U = c->ue;
+        std::vector<int> koff(K / U);
+        for (int kt = 0; kt < KT; ++kt)
+            for (int j = 0; j < nkf; ++j)
+                for (int cu = 0; cu < Cin / U; ++cu) {
+                    const long long frame = (long long)(KT - 1 - kt) * d;
+                    koff[((kt * nkf + j) * Cin) / U + cu] = (int)(frame * in.sT + (2 - j) * in.sF + U * cu);
+                }
+        const int k_off = c->wa.reserve_k(koff);
+        const PackedW pw = reserve_packed(c, 2 * Cout_real, K);
+        c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
+            const int KF = 5;
+            const std::vector<float>& w = hp.at(name + ".conv.weight");  // [Ci][Co][KF][KT]
+            const std::vector<float>& b = hp.at(name + ".conv.bias");
+            for (int parity = 0; parity < 2; ++parity)
+                for (int co = 0; co < Cout_real; ++co) {
+                    const int n = parity * Cout_real + co;
+                    for (int kt = 0; kt < KT; ++kt)
+                        for (int j = 0; j < nkf; ++j) {
+                            const int kf = 2 * j + parity;
+                            if (kf >= KF) continue;  // odd rows have no third tap: weights stay zero
+                            for (int ci = 0; ci < Cin; ++ci)
+                                arena[pw.w_off + (size_t)n * pw.K + (kt * nkf + j) * Cin + ci] =
+                                    w[((ci * Cout_real + co) * KF + kf) * KT + kt];
+                        }
+                    arena[pw.b_off + n] = b[co];
+                }
+        });
+        // ConvTranspose2d counted over the T kept frames: even bins 3 taps, odd bins 2 taps
+        const double deconv_flops = 2.0 * T * (3.0 * Fin + 2.0 * (Fin - 1)) * KT * Cin * Cout_real;
+        const double skip_flops = 4.0 * rows * Cout_real * Cout_real;
+        // residual mask / residual 1x1 pair on the skip tensor, then the affines of both GlobalLayerNorms
+        int k2_off = -1;
+        PackedW pw2{};
+        size_t nw_off = NONE, nb_off = NONE, nwr_off = NONE, nbr_off = NONE;
+        if (skip) {
+            k2_off = koff_dense(skip->C);
+            pw2 = reserve_packed(c, 2 * Cout_real, skip->C);
+            c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
                 const std::vector<float>& wm = hp.at(name + ".residualmask.weight");
                 const std::vector<float>& bm = hp.at(name + ".residualmask.bias");
                 const std::vector<float>& wr = hp.at(name + ".residual.weight");
                 const std::vector<float>& br = hp.at(name + ".residual.bias");
                 for (int co = 0; co < Cout_real; ++co) {
                     for (int ci = 0; ci < Cout_real; ++ci) {
-                        arena[pw.w_off + (size_t)(2 * co) * pw.K + ci] = wm[co * Cout_real + ci];
-                        arena[pw.w_off + (size_t)(2 * co + 1) * pw.K + ci] = wr[co * Cout_real + ci];
+                        arena[pw2.w_off + (size_t)(2 * co) * pw2.K + ci] = wm[co * Cout_real + ci];
+                        arena[pw2.w_off + (size_t)(2 * co + 1) * pw2.K + ci] = wr[co * Cout_real + ci];
                     }
-                    arena[pw.b_off + 2 * co] = bm[co];
-                    arena[pw.b_off + 2 * co + 1] = br[co];
+                    arena[pw2.b_off + 2 * co] = bm[co];
+                    arena[pw2.b_off + 2 * co + 1] = br[co];
                 }
             });
-            GemmParams g{};
-            g.A = skip->interior();
-            g.sB = skip->sB;
-            g.sT = skip->sT;
-            g.sF = skip->sF;
-            g.Tn = T;
-            g.Fo = Fs;
-            fill_gemm_common(c, g, pw, 2 * Cout_real, k_off);
-            g.epi = EPI_SKIP;
-            g.out = tmp_rm;
-            g.oB = (long long)rows * Cop;
-            g.oT = (long long)Fs * Cop;
-            g.oF = Cop;
-            g.out2 = tmp_rr;
-            g.o2B = g.oB;
-            g.o2T = g.oT;
-            g.o2F = g.oF;
-            g.stats = c->stats + (size_t)stats_slot_r * 2 * c->maxB;
-            g.vec4 = 1;
-            g.out_half = c->half ? 1 : 0;
-            meta(name + ".skip1x1", 4.0 * rows * Cout_real * Cout_real, 12.0 * rows * Cout_real);
-            push_gemm(ST_DECODER, g, rows, pw, k_off);
-            rec.op_skip = (int)c->ops.size() - 1;
-            tma_src(skip->base, skip->C, skip->Fp, skip->Tp, skip->sT, skip->sB, 1, skip->padT0, skip->padF0);
-            if (c->half && !c->train && skip->C == Cout_real && skip_small_supported(Cout_real) && c->small_layers) {
-                Op& op = c->ops.back();
-                op.kind = OP_SKIP_SMALL;
-                op.small_c = Cout_real;
-                op.sk = SkipSmallParams{};
-                op.sk.in = reinterpret_cast<const __half*>(skip->interior());
-                op.sk.sB = skip->sB;
-                op.sk.sT = skip->sT;
-                op.sk.sF = skip->sF;
-                op.sk.Fs = Fs;
-                op.sk.Kp = pw.K;
-                op.sk.rm = reinterpret_cast<__half*>(tmp_rm);
-                op.sk.rr = reinterpret_cast<__half*>(tmp_rr);
-                op.sk.stats = g.stats;
-            }
+            nw_off = pack_affine(name + ".norm.weight", Cout_real, Cop);
+            nb_off = pack_affine(name + ".norm.bias", Cout_real, Cop);
+            nwr_off = pack_affine(name + ".residualnorm.weight", Cout_real, Cop);
+            nbr_off = pack_affine(name + ".residualnorm.bias", Cout_real, Cop);
         }
-        {
-            NormApplyParams n{};
-            n.mode = 2;
-            n.T = T;
-            n.F = Fs;
-            n.C = Cop;
-            n.student = c->student;
-            n.y = y;
-            n.Fy = Fy;
-            n.stats = c->stats + (size_t)stats_slot * 2 * c->maxB;
-            n.count = (double)Cout_real * Fy * T;
-            n.rm = tmp_rm;
-            n.rr = tmp_rr;
-            n.stats_r = c->stats + (size_t)stats_slot_r * 2 * c->maxB;
-            n.count_r = (double)Cout_real * Fs * T;
-            n.out = dst;
-            n.oB = dB;
-            n.oT = dT;
-            n.oF = dF;
-            const size_t w_off = pack_affine(name + ".norm.weight", Cout_real, Cop);
-            const size_t b_off = pack_affine(name + ".norm.bias", Cout_real, Cop);
-            const size_t wr_off = pack_affine(name + ".residualnorm.weight", Cout_real, Cop);
-            const size_t br_off = pack_affine(name + ".residualnorm.bias", Cout_real, Cop);
-            meta(name + ".gln+skipblend", 0, 4.0 * T * Cout_real * (Fy + 3.0 * Fs));
-            push_norm(ST_DECODER, n, w_off, b_off, wr_off, br_off);
-            rec.op_norm = (int)c->ops.size() - 1;
-        }
-        // 32- / 64-channel levels (fp16 inference): the skip pair and the blend above become ONE launch (skip_blend_tc.cu)
-        // over the same packed weights and affines; the transposed conv stays the GEMM before it
-        if (c->half && !c->train && skip->C == Cout_real && Cop == Cout_real && skip_blend_supported(Cout_real, Fs, Fy)) {
-            const Op o_norm = c->ops.back();
-            const OpFix f_norm = fix.back();
-            c->ops.pop_back();
-            fix.pop_back();
-            const Op o_skip = c->ops.back();
-            const OpFix f_skip = fix.back();
-            c->ops.pop_back();
-            fix.pop_back();
-            Op op{};
-            op.kind = OP_SKIP_BLEND;
-            op.stage = ST_DECODER;
-            op.sb = SkipBlendParams{};
-            op.sb.t_org = skip->padT0;
-            op.sb.f_org = skip->padF0;
-            op.sb.Fs = Fs;
-            op.sb.Kp = o_skip.g.K;
-            op.sb.y = reinterpret_cast<const __half*>(y);
-            op.sb.Fy = Fy;
-            op.sb.stats = o_norm.n.stats;
-            op.sb.out = reinterpret_cast<__half*>(dst);
-            op.sb.oB = dB;
-            op.sb.oT = dT;
-            op.sb.oF = dF;
-            op.sb.student = c->student;
-            op.em_cout = Cout_real;
-            op.label = name + ".skip+gln+blend";
-            op.alg_flops = o_skip.alg_flops;
-            op.alg_bytes = 4.0 * T * Fy * Cout_real + 4.0 * 2 * T * Fs * Cout_real;  // y and skip tensor in, block output out
-            c->ops.push_back(op);
-            tma_src(skip->base, skip->C, skip->Fp, skip->Tp, skip->sT, skip->sB, 1, skip->padT0, skip->padF0);
-            fix.push_back({f_skip.w_off, f_skip.b_off, -1, f_norm.nw_off, f_norm.nb_off, f_norm.nwr_off, f_norm.nbr_off});
-        } else if (c->dec_mma && skip->C == Cout_real && Cop == Cout_real &&
-                   dec_mma_supported(Cin, Cout_real, in.Tp, in.Fp, Fin, Fs)) {
-            // small-channel levels (fp16 mode): the three ops above become ONE launch (back_mma.cu); their packed weights
-            // and report entries are reused
-            const Op o_norm = c->ops.back();
-            const OpFix f_norm = fix.back();
-            c->ops.pop_back();
-            fix.pop_back();
-            const Op o_skip = c->ops.back();
-            const OpFix f_skip = fix.back();
-            c->ops.pop_back();
-            fix.pop_back();
-            const Op o_dec = c->ops.back();
-            const OpFix f_dec = fix.back();
-            c->ops.pop_back();
-            fix.pop_back();
+        se_ctx* cc = c;
+        const bool fused_skip = skip && skip->C == Cout_real && Cop == Cout_real;
+        // 32- / 64-channel levels (fp16 inference): the skip pair and the blend as ONE launch (skip_blend_tc.cu) after the
+        // transposed-conv GEMM
+        const bool blend = fused_skip && c->half && !c->train && skip_blend_supported(Cout_real, Fs, Fy);
+        if (fused_skip && !blend && c->dec_mma && dec_mma_supported(Cin, Cout_real, in.Tp, in.Fp, Fin, Fs)) {
+            // small-channel levels (fp16 mode): the whole block as ONE launch (back_mma.cu)
             Op op{};
             op.kind = OP_DEC_MMA;
             op.stage = ST_DECODER;
@@ -999,13 +883,13 @@ struct Builder {
             op.dm.Fp = in.Fp;
             op.dm.d = d;
             op.dm.Fin = Fin;
-            op.dm.Kp = o_dec.g.K;
+            op.dm.Kp = pw.K;
             op.dm.skip = reinterpret_cast<const __half*>(skip->interior());
             op.dm.sk_sB = skip->sB;
             op.dm.sk_sT = skip->sT;
             op.dm.sk_sF = skip->sF;
             op.dm.Fs = Fs;
-            op.dm.K2p = o_skip.g.K;
+            op.dm.K2p = pw2.K;
             op.dm.out = reinterpret_cast<__half*>(dst);
             op.dm.oB = dB;
             op.dm.oT = dT;
@@ -1013,12 +897,167 @@ struct Builder {
             op.dm.student = c->student;
             op.em_cin = Cin;
             op.em_cout = Cout_real;
-            op.label = name + ".deconv+skip+blend";
-            op.alg_flops = o_dec.alg_flops + o_skip.alg_flops;
-            op.alg_bytes = 4.0 * Cin * T * Fin + 4.0 * 2 * T * Fs * Cout_real;  // input and skip tensor in, block output out
-            c->ops.push_back(op);
-            fix.push_back({f_dec.w_off, f_dec.b_off, -1, f_norm.nw_off, f_norm.nb_off, f_norm.nwr_off, f_norm.nbr_off,
-                           f_skip.w_off, f_skip.b_off});
+            // input and skip tensor in, block output out
+            meta(name + ".deconv+skip+blend", deconv_flops + skip_flops, 4.0 * Cin * T * Fin + 4.0 * 2 * T * Fs * Cout_real);
+            push(op, [=](Op& o) {
+                const float* w = cc->wa.w;
+                o.dm.w = w + pw.w_off;
+                o.dm.bias = w + pw.b_off;
+                o.dm.w2 = w + pw2.w_off;
+                o.dm.bias2 = w + pw2.b_off;
+                o.dm.nw = w + nw_off;
+                o.dm.nb = w + nb_off;
+                o.dm.nwr = w + nwr_off;
+                o.dm.nbr = w + nbr_off;
+                return 0;
+            });
+            return;
+        }
+        meta(name + ".deconv+elu", deconv_flops, 4.0 * Cin * T * Fin + 4.0 * T * Fy * Cout_real);
+        if (c->half && !c->train && !skip && Cout_real == 2 && KT == 3 && deconv_last_supported(Cin) && c->small_layers) {
+            Op op{};  // the last level on the direct kernel (small_layers.cu): fp16 input, fp32 output
+            op.kind = OP_DECONV_LAST;
+            op.stage = ST_DECODER;
+            op.small_c = Cin;
+            op.dl = DeconvLastParams{};
+            op.dl.in = reinterpret_cast<const __half*>(in.base);
+            op.dl.sB = in.sB;
+            op.dl.sT = in.sT;
+            op.dl.sF = in.sF;
+            op.dl.Fin = Fin;
+            op.dl.d = d;
+            op.dl.Kp = pw.K;
+            op.dl.y = y;
+            op.dl.stats = stats;
+            m_f16 = 0.75;
+            push(op, [=](Op& o) {
+                o.dl.w = cc->wa.w + pw.w_off;
+                o.dl.bias = cc->wa.w + pw.b_off;
+                return 0;
+            });
+        } else {
+            GemmParams g{};
+            g.A = in.base;  // padded row 0, frame 0
+            g.sB = in.sB;
+            g.sT = in.sT;
+            g.sF = in.sF;
+            g.Tn = T;
+            g.Fo = Fin;
+            fill_gemm_common(c, g, pw, 2 * Cout_real);
+            g.epi = EPI_ELU_STATS;
+            g.out = y;
+            g.oB = (long long)T * Fy * Cop;
+            g.oT = (long long)Fy * Cop;
+            g.oF = 2 * Cop;
+            g.odd_tail = 1;
+            g.out_half = (c->half && skip) ? 1 : 0;  // the last layer's output feeds the mask kernel in fp32
+            g.stats = stats;
+            g.vec4 = Cop % 4 == 0;
+            rec.op_deconv = push_gemm(ST_DECODER, g, T * Fin, pw, k_off, TmaSrc{in.base, in.C, in.Fp, in.Tp, in.sT, in.sB});
+        }
+        if (!skip) {
+            if (c->train) c->deconv_recs.push_back(rec);
+            return;
+        }
+        const TmaSrc skip_src{skip->base, skip->C, skip->Fp, skip->Tp, skip->sT, skip->sB, 1, skip->padT0, skip->padF0};
+        if (blend) {
+            Op op{};
+            op.kind = OP_SKIP_BLEND;
+            op.stage = ST_DECODER;
+            op.sb = SkipBlendParams{};
+            op.sb.t_org = skip->padT0;
+            op.sb.f_org = skip->padF0;
+            op.sb.Fs = Fs;
+            op.sb.Kp = pw2.K;
+            op.sb.y = reinterpret_cast<const __half*>(y);
+            op.sb.Fy = Fy;
+            op.sb.stats = stats;
+            op.sb.out = reinterpret_cast<__half*>(dst);
+            op.sb.oB = dB;
+            op.sb.oT = dT;
+            op.sb.oF = dF;
+            op.sb.student = c->student;
+            op.em_cout = Cout_real;
+            // y and skip tensor in, block output out
+            meta(name + ".skip+gln+blend", skip_flops, 4.0 * T * Fy * Cout_real + 4.0 * 2 * T * Fs * Cout_real);
+            push(op, [=](Op& o) {
+                const float* w = cc->wa.w;
+                o.sb.w = cc->wa.wh + pw2.w_off;
+                o.sb.bias = w + pw2.b_off;
+                o.sb.nw = w + nw_off;
+                o.sb.nb = w + nb_off;
+                o.sb.nwr = w + nwr_off;
+                o.sb.nbr = w + nbr_off;
+                return make_skip_blend_maps(&o.sb, skip_src.base, skip_src.C, skip_src.Fp, skip_src.Tp, skip_src.sT,
+                                            skip_src.sB, cc->maxB);
+            });
+            return;
+        }
+        meta(name + ".skip1x1", skip_flops, 12.0 * rows * Cout_real);
+        if (c->half && !c->train && skip->C == Cout_real && skip_small_supported(Cout_real) && c->small_layers) {
+            Op op{};  // the skip pair on the small-channel kernel (small_layers.cu)
+            op.kind = OP_SKIP_SMALL;
+            op.stage = ST_DECODER;
+            op.small_c = Cout_real;
+            op.sk = SkipSmallParams{};
+            op.sk.in = reinterpret_cast<const __half*>(skip->interior());
+            op.sk.sB = skip->sB;
+            op.sk.sT = skip->sT;
+            op.sk.sF = skip->sF;
+            op.sk.Fs = Fs;
+            op.sk.Kp = pw2.K;
+            op.sk.rm = reinterpret_cast<__half*>(tmp_rm);
+            op.sk.rr = reinterpret_cast<__half*>(tmp_rr);
+            op.sk.stats = stats_r;
+            push(op, [=](Op& o) {
+                o.sk.w = cc->wa.w + pw2.w_off;
+                o.sk.bias = cc->wa.w + pw2.b_off;
+                return 0;
+            });
+        } else {
+            GemmParams g{};
+            g.A = skip->interior();
+            g.sB = skip->sB;
+            g.sT = skip->sT;
+            g.sF = skip->sF;
+            g.Tn = T;
+            g.Fo = Fs;
+            fill_gemm_common(c, g, pw2, 2 * Cout_real);
+            g.epi = EPI_SKIP;
+            g.out = tmp_rm;
+            g.oB = (long long)rows * Cop;
+            g.oT = (long long)Fs * Cop;
+            g.oF = Cop;
+            g.out2 = tmp_rr;
+            g.o2B = g.oB;
+            g.o2T = g.oT;
+            g.o2F = g.oF;
+            g.stats = stats_r;
+            g.vec4 = 1;
+            g.out_half = c->half ? 1 : 0;
+            rec.op_skip = push_gemm(ST_DECODER, g, rows, pw2, k2_off, skip_src);
+        }
+        {
+            NormApplyParams n{};
+            n.mode = 2;
+            n.T = T;
+            n.F = Fs;
+            n.C = Cop;
+            n.student = c->student;
+            n.y = y;
+            n.Fy = Fy;
+            n.stats = stats;
+            n.count = (double)Cout_real * Fy * T;
+            n.rm = tmp_rm;
+            n.rr = tmp_rr;
+            n.stats_r = stats_r;
+            n.count_r = (double)Cout_real * Fs * T;
+            n.out = dst;
+            n.oB = dB;
+            n.oT = dT;
+            n.oF = dF;
+            meta(name + ".gln+skipblend", 0, 4.0 * T * Cout_real * (Fy + 3.0 * Fs));
+            rec.op_norm = push_norm(ST_DECODER, n, nw_off, nb_off, nwr_off, nbr_off);
         }
         if (c->train) c->deconv_recs.push_back(rec);
     }
@@ -1200,7 +1239,7 @@ int build_ctx(se_ctx* c) {
     if (dev_alloc(c, &c->gru_counters, (size_t)2 * ((maxB + 127) / 128))) return 1;
 
     // ---- program ----------------------------------------------------------------------------------------------
-    Builder b{c, {}};
+    Builder b{c};
     int slot = 0;
     for (int i = 0; i < 3 && c->train; ++i) {  // training: generic conv blocks with the residual add (CRN_ELU.py:376)
         const Act& in = c->pre_act[i];
@@ -1209,32 +1248,9 @@ int build_ctx(se_ctx* c) {
                      nx.interior(), nx.sB, nx.sT, nx.sF, true, slot++, i, nx.dinterior());
         c->conv_recs.back().need_dgrad = i > 0;
     }
-    auto pack_preconv_block = [&](const std::string& name) -> size_t {  // PRECONV_W_* layout (se_internal.h)
-        const size_t w_off = c->reserve_w(PRECONV_W_FLOATS);
-        c->packers.push_back([=](const HostParams& hp, float* arena) {
-            const std::vector<float>& w = hp.at(name + ".conv.weight");  // [Co][Ci][KF][KT]
-            float* a = arena + w_off;
-            for (int kt = 0; kt < 5; ++kt)
-                for (int ci = 0; ci < 5; ++ci)
-                    for (int kf = 0; kf < 5; ++kf)
-                        for (int co = 0; co < 5; ++co)
-                            a[(kt * 5 + ci) * 28 + kf * 5 + co] = w[((co * 5 + ci) * 5 + kf) * 5 + kt];
-            for (int co = 0; co < 5; ++co) {
-                a[PRECONV_W_BIAS + co] = hp.at(name + ".conv.bias")[co];
-                for (int k = 0; k < 5; ++k) {
-                    a[PRECONV_W_WT + co * 5 + k] = hp.at(name + ".conv_trans.weight")[co * 5 + k];
-                    a[PRECONV_W_WG + co * 5 + k] = hp.at(name + ".conv_gated.weight")[co * 5 + k];
-                }
-                a[PRECONV_W_BT + co] = hp.at(name + ".conv_trans.bias")[co];
-                a[PRECONV_W_BG + co] = hp.at(name + ".conv_gated.bias")[co];
-                a[PRECONV_W_NW + co] = hp.at(name + ".norm.weight")[co];
-                a[PRECONV_W_NB + co] = hp.at(name + ".norm.bias")[co];
-            }
-        });
-        return w_off;
-    };
     if (c->front_mma) {  // fp16 mode: the three pre-convolution blocks in one launch (front_mma.cu)
-        for (int i = 0; i < 3; ++i) c->pre3_w_off[i] = pack_preconv_block("preconvlist." + std::to_string(i));
+        size_t w_off[3];
+        for (int i = 0; i < 3; ++i) w_off[i] = b.pack_preconv_block("preconvlist." + std::to_string(i));
         const Act& nx = c->enc_in[0];
         Op op{};
         op.kind = OP_PRECONV3;
@@ -1249,37 +1265,17 @@ int build_ctx(se_ctx* c) {
         op.p3.oT = nx.sT;
         op.p3.oF = nx.sF;
         op.p3.student = c->student;
-        op.label = "preconvlist.0-2.fused";
-        op.alg_flops = 3 * 2.0 * T * NBIN * 5 * (125 + 10);
         // features in, block output out, 4 carried frames per layer read and written (fp32 sizes, as for every other op)
-        op.alg_bytes = 4.0 * 5 * NBIN * (T + T + 3 * 2 * 4);
-        c->ops.push_back(op);
-        b.fix.push_back({NONE, NONE, -1, NONE, NONE, NONE, NONE});
+        b.meta("preconvlist.0-2.fused", 3 * 2.0 * T * NBIN * 5 * (125 + 10), 4.0 * 5 * NBIN * (T + T + 3 * 2 * 4));
+        b.push(op, [=](Op& o) {
+            for (int l = 0; l < 3; ++l) o.p3.w[l] = c->wa.w + w_off[l];
+            return 0;
+        });
         slot += 3;
     }
     for (int i = 0; i < 3 && c->preconv_tc && !c->front_mma; ++i) {  // fp16 mode: pre-convolutions on the tensor cores (preconv_tc.cu)
         const std::string name = "preconvlist." + std::to_string(i);
-        const size_t w_off = c->reserve_w(PRECONV_W_FLOATS);
-        c->packers.push_back([=](const HostParams& hp, float* arena) {
-            const std::vector<float>& w = hp.at(name + ".conv.weight");  // [Co][Ci][KF][KT]
-            float* a = arena + w_off;
-            for (int kt = 0; kt < 5; ++kt)
-                for (int ci = 0; ci < 5; ++ci)
-                    for (int kf = 0; kf < 5; ++kf)
-                        for (int co = 0; co < 5; ++co)
-                            a[(kt * 5 + ci) * 28 + kf * 5 + co] = w[((co * 5 + ci) * 5 + kf) * 5 + kt];
-            for (int co = 0; co < 5; ++co) {
-                a[PRECONV_W_BIAS + co] = hp.at(name + ".conv.bias")[co];
-                for (int k = 0; k < 5; ++k) {
-                    a[PRECONV_W_WT + co * 5 + k] = hp.at(name + ".conv_trans.weight")[co * 5 + k];
-                    a[PRECONV_W_WG + co * 5 + k] = hp.at(name + ".conv_gated.weight")[co * 5 + k];
-                }
-                a[PRECONV_W_BT + co] = hp.at(name + ".conv_trans.bias")[co];
-                a[PRECONV_W_BG + co] = hp.at(name + ".conv_gated.bias")[co];
-                a[PRECONV_W_NW + co] = hp.at(name + ".norm.weight")[co];
-                a[PRECONV_W_NB + co] = hp.at(name + ".norm.bias")[co];
-            }
-        });
+        const size_t w_off = b.pack_preconv_block(name);
         Op op{};
         op.kind = OP_PRECONV_TC;
         op.stage = ST_PRECONV;
@@ -1299,37 +1295,17 @@ int build_ctx(se_ctx* c) {
             op.pt.oT = nx.sT;
             op.pt.oF = nx.sF;
         }
-        op.label = name + ".fused";
-        op.alg_flops = 2.0 * T * NBIN * 5 * (125 + 10);
-        op.alg_bytes = 2.0 * 8 * NBIN * (PRECONV_TP + T);
-        c->ops.push_back(op);
-        b.fix.push_back({NONE, NONE, -1, w_off, NONE, NONE, NONE});
+        b.meta(name + ".fused", 2.0 * T * NBIN * 5 * (125 + 10), 2.0 * 8 * NBIN * (PRECONV_TP + T), 1);
+        b.push(op, [=](Op& o) {
+            o.pt.w = c->wa.w + w_off;
+            return 0;
+        });
         slot++;
     }
     for (int i = 0; i < 3 && !c->train && !c->preconv_tc; ++i) {  // pre-convolutions: one fused kernel per layer (preconv.cu), exact fp32
         const PreBuf& in = c->pre_in[i];
         const std::string name = "preconvlist." + std::to_string(i);
-        const size_t w_off = c->reserve_w(PRECONV_W_FLOATS);
-        c->packers.push_back([=](const HostParams& hp, float* arena) {
-            const std::vector<float>& w = hp.at(name + ".conv.weight");  // [Co][Ci][KF][KT]
-            float* a = arena + w_off;
-            for (int kt = 0; kt < 5; ++kt)
-                for (int ci = 0; ci < 5; ++ci)
-                    for (int kf = 0; kf < 5; ++kf)
-                        for (int co = 0; co < 5; ++co)
-                            a[(kt * 5 + ci) * 28 + kf * 5 + co] = w[((co * 5 + ci) * 5 + kf) * 5 + kt];
-            for (int co = 0; co < 5; ++co) {
-                a[PRECONV_W_BIAS + co] = hp.at(name + ".conv.bias")[co];
-                for (int k = 0; k < 5; ++k) {
-                    a[PRECONV_W_WT + co * 5 + k] = hp.at(name + ".conv_trans.weight")[co * 5 + k];
-                    a[PRECONV_W_WG + co * 5 + k] = hp.at(name + ".conv_gated.weight")[co * 5 + k];
-                }
-                a[PRECONV_W_BT + co] = hp.at(name + ".conv_trans.bias")[co];
-                a[PRECONV_W_BG + co] = hp.at(name + ".conv_gated.bias")[co];
-                a[PRECONV_W_NW + co] = hp.at(name + ".norm.weight")[co];
-                a[PRECONV_W_NB + co] = hp.at(name + ".norm.bias")[co];
-            }
-        });
+        const size_t w_off = b.pack_preconv_block(name);
         Op op{};
         op.kind = OP_PRECONV;
         op.stage = ST_PRECONV;
@@ -1354,11 +1330,11 @@ int build_ctx(se_ctx* c) {
             op.pc.out_vec8 = 1;
             op.pc.out_half = c->half ? 1 : 0;
         }
-        op.label = name + ".fused";
-        op.alg_flops = 2.0 * T * NBIN * 5 * (125 + 10);
-        op.alg_bytes = 4.0 * 5 * NBIN * (PRECONV_TP + T);
-        c->ops.push_back(op);
-        b.fix.push_back({NONE, NONE, -1, w_off, NONE, NONE, NONE});
+        b.meta(name + ".fused", 2.0 * T * NBIN * 5 * (125 + 10), 4.0 * 5 * NBIN * (PRECONV_TP + T), 1);
+        b.push(op, [=](Op& o) {
+            o.pc.w = c->wa.w + w_off;
+            return 0;
+        });
         slot++;
     }
     for (int i = 0; i < c->L; ++i) {
@@ -1398,7 +1374,7 @@ int build_ctx(se_ctx* c) {
         if (wave && l == 1) {  // W_ih1 in the gate-tile order of the fused cell; no batched projection
             PackedW pw = reserve_packed(c, 3 * H, H);
             wave_pw[1] = pw;
-            c->packers.push_back([=](const HostParams& hp, float* arena) {
+            c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
                 const std::vector<float>& w = hp.at("gru.sequence_model.weight_ih_l1");
                 const std::vector<float>& bi = hp.at("gru.sequence_model.bias_ih_l1");
                 for (int n = 0; n < 3 * H; ++n) {
@@ -1410,7 +1386,7 @@ int build_ctx(se_ctx* c) {
         } else {  // input projection for all T frames at once
             const int k_off = b.koff_dense(Kin);
             PackedW pw = reserve_packed(c, 3 * H, Kin);
-            c->packers.push_back([=](const HostParams& hp, float* arena) {
+            c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
                 const std::vector<float>& w = hp.at("gru.sequence_model.weight_ih_l" + s);
                 const std::vector<float>& bi = hp.at("gru.sequence_model.bias_ih_l" + s);
                 for (int n = 0; n < 3 * H; ++n) {
@@ -1432,23 +1408,22 @@ int build_ctx(se_ctx* c) {
             gp.sF = 0;
             gp.Tn = T;
             gp.Fo = 1;
-            fill_gemm_common(c, gp, pw, 3 * H, k_off);
+            fill_gemm_common(c, gp, pw, 3 * H);
             gp.epi = EPI_BIAS;
             gp.out = c->gi_l[l];
             gp.oB = (long long)T * 3 * H;
             gp.oT = 3 * H;
             gp.oF = 0;
             gp.vec4 = 1;
-            b.meta("gru.l" + s + ".input_proj", 2.0 * T * 3 * H * Kin, 4.0 * T * (Kin + 3 * H));
-            b.push_gemm(ST_GRU, gp, T, pw, k_off);
-            c->gru_rec.op_in[l] = (int)c->ops.size() - 1;
-            if (l == 0) b.tma_src(c->xg, feat, 1, T, feat, (long long)T * feat);
-            else b.tma_src(c->hseq[0], H, 1, T + 1, H, (long long)(T + 1) * H, 1, 1, 0);
+            b.meta("gru.l" + s + ".input_proj", 2.0 * T * 3 * H * Kin, 4.0 * T * (Kin + 3 * H), 1);
+            c->gru_rec.op_in[l] = b.push_gemm(ST_GRU, gp, T, pw, k_off,
+                                              l == 0 ? TmaSrc{c->xg, feat, 1, T, feat, (long long)T * feat}
+                                                     : TmaSrc{c->hseq[0], H, 1, T + 1, H, (long long)(T + 1) * H, 1, 1, 0});
         }
         const int k_off = b.koff_dense(H);
         PackedW pw = reserve_packed(c, 3 * H, H);
         const bool fused = !c->train && (c->half || (c->tf32 && ((c->tc_mask >> ST_GRU) & 1u) && H % 32 == 0));
-        c->packers.push_back([=](const HostParams& hp, float* arena) {
+        c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
             const std::vector<float>& w = hp.at("gru.sequence_model.weight_hh_l" + s);
             const std::vector<float>& bh = hp.at("gru.sequence_model.bias_hh_l" + s);
             for (int n = 0; n < 3 * H; ++n) {
@@ -1466,9 +1441,6 @@ int build_ctx(se_ctx* c) {
                 op.kind = OP_GRU_WAVE;
                 op.stage = ST_GRU;
                 op.rows_per_stream = 1;
-                op.label = "gru.l0+l1.recurrence(wavefront)";
-                op.alg_flops = 2.0 * T * 3 * H * H * 3;          // W_hh0, W_ih1, W_hh1
-                op.alg_bytes = 22.0 * T * H;  // gi0 (fp32) read; h0 history written, read by both layers; h1 written + read (fp16)
                 op.gw = GruWaveParams{};
                 op.gw.Kp = pw.K;
                 op.gw.gi0 = c->gi_l[0];
@@ -1481,23 +1453,32 @@ int build_ctx(se_ctx* c) {
                 op.gw.H = H;
                 op.gw.T = T;
                 op.gw.layers = 2;
-                c->ops.push_back(op);
-                b.fix.push_back({wave_pw[0].w_off, wave_pw[0].b_off, -1, wave_pw[1].w_off, wave_pw[1].b_off,
-                                 wave_pw[2].w_off, wave_pw[2].b_off});
+                // W_hh0, W_ih1, W_hh1; gi0 (fp32) read; h0 history written, read by both layers; h1 written + read (fp16)
+                b.meta("gru.l0+l1.recurrence(wavefront)", 2.0 * T * 3 * H * H * 3, 22.0 * T * H, 1);
+                b.push(op, [=](Op& o) {
+                    const WeightArena& wa = c->wa;
+                    o.gw.Whh0 = wa.wh + wave_pw[0].w_off;
+                    o.gw.bhh0 = wa.w + wave_pw[0].b_off;
+                    o.gw.Wih1 = wa.wh + wave_pw[1].w_off;
+                    o.gw.bih1 = wa.w + wave_pw[1].b_off;
+                    o.gw.Whh1 = wa.wh + wave_pw[2].w_off;
+                    o.gw.bhh1 = wa.w + wave_pw[2].b_off;
+                    o.gw.cstride = (c->maxB + 127) / 128;
+                    o.gw.counters = c->gru_counters;
+                    return make_gru_wave_maps(&o.gw, c->maxB);
+                });
             }
             continue;
         }
         if (persist) {  // the whole recurrence of the layer: one persistent tensor-core kernel (gru_tc_persist.cu)
-            GemmParams gp{};
-            fill_gemm_common(c, gp, pw, 3 * H, k_off);
-            gp.epi = EPI_GRU;
-            b.meta("gru.l" + s + ".recurrence", 2.0 * T * 3 * H * H, 4.0 * T * (3 * H + 2 * H));
-            b.push_gemm(ST_GRU, gp, 1, pw, k_off);
-            Op& op = c->ops.back();
+            Op op{};
+            op.stage = ST_GRU;
+            op.rows_per_stream = 1;
+            op.gru_layer = l;
+            b.meta("gru.l" + s + ".recurrence", 2.0 * T * 3 * H * H, 4.0 * T * (3 * H + 2 * H), 1);
             if (c->gru_wave == 2 && gru_wave_supported(H, 1)) {  // H too large for the wavefront: its one-layer form (measured
                                                                // 151 us vs 146 us per layer at H = 512: opt-in)
                 op.kind = OP_GRU_WAVE;
-                op.gru_layer = l;
                 op.gw = GruWaveParams{};
                 op.gw.Kp = pw.K;
                 op.gw.gi0 = c->gi_l[l];
@@ -1508,10 +1489,16 @@ int build_ctx(se_ctx* c) {
                 op.gw.H = H;
                 op.gw.T = T;
                 op.gw.layers = 1;
+                b.push(op, [=](Op& o) {
+                    o.gw.Whh0 = c->wa.wh + pw.w_off;
+                    o.gw.bhh0 = c->wa.w + pw.b_off;
+                    o.gw.cstride = (c->maxB + 127) / 128;
+                    o.gw.counters = c->gru_counters + (size_t)l * o.gw.cstride;
+                    return make_gru_wave_maps(&o.gw, c->maxB);
+                });
                 continue;
             }
             op.kind = OP_GRU_TC;
-            op.gru_layer = l;
             op.gt = GruTcParams{};
             op.gt.Kp = pw.K;
             op.gt.gi = c->gi_l[l];
@@ -1521,6 +1508,12 @@ int build_ctx(se_ctx* c) {
             op.gt.h32 = c->h32[l];
             op.gt.H = H;
             op.gt.T = T;
+            b.push(op, [=](Op& o) {
+                o.gt.Whh = c->wa.wh + pw.w_off;
+                o.gt.bhh = c->wa.w + pw.b_off;
+                o.gt.counters = c->gru_counters + (size_t)l * ((c->maxB + 127) / 128);
+                return 0;
+            });
         }
         for (int t = 0; t < T && fused && !persist; ++t) {
             GemmParams gp{};
@@ -1528,7 +1521,7 @@ int build_ctx(se_ctx* c) {
             gp.sB = (long long)(T + 1) * H;
             gp.Tn = 1;
             gp.Fo = 1;
-            fill_gemm_common(c, gp, pw, 3 * H, k_off);
+            fill_gemm_common(c, gp, pw, 3 * H);
             gp.epi = EPI_GRU;
             gp.gi = c->gi_l[l] + (long long)t * 3 * H;
             gp.giB = (long long)T * 3 * H;
@@ -1546,7 +1539,7 @@ int build_ctx(se_ctx* c) {
                 gp.hB = (long long)(T + 1) * H;
             }
             gp.H = H;
-            b.meta("gru.l" + s + ".step" + std::to_string(t), 2.0 * 3 * H * H, 4.0 * (3 * H + 2 * H));
+            b.meta("gru.l" + s + ".step" + std::to_string(t), 2.0 * 3 * H * H, 4.0 * (3 * H + 2 * H), 1);
             b.push_gemm(ST_GRU, gp, 1, pw, k_off);
         }
         const bool seq = c->train && gru_seq_supported(H);
@@ -1556,15 +1549,13 @@ int build_ctx(se_ctx* c) {
             gp.sB = (long long)(T + 1) * H;
             gp.Tn = 1;
             gp.Fo = 1;
-            fill_gemm_common(c, gp, pw, 3 * H, k_off);
+            fill_gemm_common(c, gp, pw, 3 * H);
             gp.epi = EPI_BIAS;
             gp.out = c->gh;
             gp.oB = 3 * H;
             b.meta("gru.l" + s + ".recurrence", 2.0 * T * 3 * H * H, 4.0 * T * (3 * H + 2 * H));
-            b.push_gemm(ST_GRU, gp, 1, pw, k_off);
-            c->ops.back().kind = OP_GRU_SEQ;
+            c->gru_rec.op_hh[l] = b.push_gemm(ST_GRU, gp, 1, pw, k_off, {}, NONE, NONE, OP_GRU_SEQ);
             c->ops.back().gru_layer = l;
-            c->gru_rec.op_hh[l] = (int)c->ops.size() - 1;
         }
         for (int t = 0; t < T && !fused && !seq; ++t) {
             GemmParams gp{};
@@ -1574,18 +1565,18 @@ int build_ctx(se_ctx* c) {
             gp.sF = 0;
             gp.Tn = 1;
             gp.Fo = 1;
-            fill_gemm_common(c, gp, pw, 3 * H, k_off);
+            fill_gemm_common(c, gp, pw, 3 * H);
             gp.epi = EPI_BIAS;
             gp.out = c->gh;
             gp.oB = 3 * H;
             gp.oT = 0;
             gp.oF = 0;
-            b.meta("gru.l" + s + ".step" + std::to_string(t) + ".hh", 2.0 * 3 * H * H, 4.0 * (H + 3 * H));
-            b.push_gemm(ST_GRU, gp, 1, pw, k_off);
-            if (t == 0) c->gru_rec.op_hh[l] = (int)c->ops.size() - 1;
+            b.meta("gru.l" + s + ".step" + std::to_string(t) + ".hh", 2.0 * 3 * H * H, 4.0 * (H + 3 * H), 1);
+            const int i = b.push_gemm(ST_GRU, gp, 1, pw, k_off);
+            if (t == 0) c->gru_rec.op_hh[l] = i;
             c->ops.back().chunk_serial = 1;
             c->ops.back().gru_layer = l;
-            b.meta("gru.l" + s + ".step" + std::to_string(t) + ".cell", 0, 4.0 * (6 * H + 2 * H));
+            b.meta("gru.l" + s + ".step" + std::to_string(t) + ".cell", 0, 4.0 * (6 * H + 2 * H), 1);
             b.push_gru_pw(c->gi_l[l] + (long long)t * 3 * H, (long long)T * 3 * H, c->gh, c->hseq[l] + (long long)t * H,
                           (long long)(T + 1) * H, c->hseq[l] + (long long)(t + 1) * H, H);
             c->ops.back().chunk_serial = 1;
@@ -1595,7 +1586,7 @@ int build_ctx(se_ctx* c) {
     {  // fc + ELU + stats, then per-feature GLN into the first decoder input
         const int k_off = b.koff_dense(H);
         PackedW pw = reserve_packed(c, feat, H);
-        c->packers.push_back([=](const HostParams& hp, float* arena) {
+        c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
             const std::vector<float>& w = hp.at("gru.fc_output_layer.weight");
             const std::vector<float>& bb = hp.at("gru.fc_output_layer.bias");
             for (int n = 0; n < feat; ++n) {
@@ -1611,7 +1602,7 @@ int build_ctx(se_ctx* c) {
         gp.sF = 0;
         gp.Tn = T;
         gp.Fo = 1;
-        fill_gemm_common(c, gp, pw, feat, k_off);
+        fill_gemm_common(c, gp, pw, feat);
         gp.epi = EPI_ELU_STATS;
         gp.out = c->fcraw;
         gp.oB = (long long)T * feat;
@@ -1621,9 +1612,8 @@ int build_ctx(se_ctx* c) {
         gp.vec4 = 1;
         gp.out_half = c->half ? 1 : 0;
         b.meta("gru.fc+elu", 2.0 * T * feat * H, 4.0 * T * (H + feat));
-        b.push_gemm(ST_GRU, gp, T, pw, k_off);
-        c->gru_rec.op_fc = (int)c->ops.size() - 1;
-        b.tma_src(c->hseq[1], H, 1, T + 1, H, (long long)(T + 1) * H, 1, 1, 0);
+        c->gru_rec.op_fc =
+            b.push_gemm(ST_GRU, gp, T, pw, k_off, TmaSrc{c->hseq[1], H, 1, T + 1, H, (long long)(T + 1) * H, 1, 1, 0});
 
         const Act& nx = c->dec_in[0];
         NormApplyParams n{};
@@ -1641,8 +1631,8 @@ int build_ctx(se_ctx* c) {
         n.oB = nx.sB;
         n.oT = nx.sT;
         n.oF = nx.sF;
-        const size_t w_off = c->reserve_w(feat), b_off = c->reserve_w(feat);
-        c->packers.push_back([=](const HostParams& hp, float* arena) {
+        const size_t w_off = c->wa.reserve_w(feat), b_off = c->wa.reserve_w(feat);
+        c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
             const std::vector<float>& w = hp.at("gru.norm.weight");
             const std::vector<float>& bb = hp.at("gru.norm.bias");
             for (int n2 = 0; n2 < feat; ++n2) {
@@ -1651,8 +1641,7 @@ int build_ctx(se_ctx* c) {
             }
         });
         b.meta("gru.gln", 0, 8.0 * T * feat);
-        b.push_norm(ST_GRU, n, w_off, b_off);
-        c->gru_rec.op_norm = (int)c->ops.size() - 1;
+        c->gru_rec.op_norm = b.push_norm(ST_GRU, n, w_off, b_off);
     }
     // ---- decoder ----------------------------------------------------------------------------------------------
     size_t wl_off = NONE, bl_off = NONE;
@@ -1678,16 +1667,18 @@ int build_ctx(se_ctx* c) {
     SE_REQUIRE(!c->alloc_failed, "out of device memory while allocating the per-layer training buffers");
 
     // ---- arenas -------------------------------------------------------------------------------------------------
-    if (dev_alloc(c, &c->warena, c->warena_floats)) return 1;
-    if (c->half && dev_alloc(c, reinterpret_cast<char**>(&c->warena_h), c->warena_floats * 2)) return 1;
+    c->wa.half = c->half;
+    if (c->wa.allocate(c->allocs)) return 1;
+    c->w_last = c->wa.w + wl_off;
+    c->b_last = c->wa.w + bl_off;
     if (c->train) {
         // position map of the packed arena: run the packers on index-coded parameters (value = 1 + flat index; every
         // packer only copies values, and 6.2 M indices are exact in fp32)
-        if (dev_alloc(c, &c->garena, c->warena_floats)) return 1;
-        if (dev_alloc(c, &c->wmap, c->warena_floats)) return 1;
+        if (dev_alloc(c, &c->garena, c->wa.floats)) return 1;
+        if (dev_alloc(c, &c->wmap, c->wa.floats)) return 1;
         HostParams hp;
         int64_t off = 0;
-        for (const ParamInfo& pi : c->params) {
+        for (const ParamInfo& pi : c->wa.params) {
             c->param_off.push_back(off);
             std::vector<float> v((size_t)pi.numel());
             for (size_t i = 0; i < v.size(); ++i) v[i] = (float)(off + (int64_t)i + 1);
@@ -1696,128 +1687,11 @@ int build_ctx(se_ctx* c) {
         }
         c->n_theta = off;
         SE_REQUIRE(off < (1 << 24), "internal: parameter count exceeds the exact-integer range of the index coding");
-        std::vector<float> arena(c->warena_floats, 0.f);
-        for (const PackFn& f : c->packers) f(hp, arena.data());
-        std::vector<int> map(c->warena_floats);
+        const std::vector<float> arena = c->wa.pack(hp);
+        std::vector<int> map(arena.size());
         for (size_t i = 0; i < arena.size(); ++i) map[i] = (int)arena[i];
         SE_CUDA_OK(cudaMemcpy(c->wmap, map.data(), map.size() * sizeof(int), cudaMemcpyHostToDevice));
     }
-    if (dev_alloc(c, &c->karena, c->khost.size())) return 1;
-    SE_CUDA_OK(cudaMemcpy(c->karena, c->khost.data(), c->khost.size() * sizeof(int), cudaMemcpyHostToDevice));
-    for (size_t i = 0; i < c->ops.size(); ++i) {
-        Op& op = c->ops[i];
-        const OpFix& f = b.fix[i];
-        if (op.kind == OP_GRU_WAVE) {
-            const __half* wh = reinterpret_cast<const __half*>(c->warena_h);
-            op.gw.Whh0 = wh + f.w_off;
-            op.gw.bhh0 = c->warena + f.b_off;
-            op.gw.cstride = (c->maxB + 127) / 128;
-            op.gw.counters = c->gru_counters;
-            if (op.gw.layers == 2) {
-                op.gw.Wih1 = wh + f.nw_off;
-                op.gw.bih1 = c->warena + f.nb_off;
-                op.gw.Whh1 = wh + f.nwr_off;
-                op.gw.bhh1 = c->warena + f.nbr_off;
-            } else {
-                op.gw.counters += (size_t)op.gru_layer * op.gw.cstride;
-            }
-            if (make_gru_wave_maps(&op.gw, c->maxB)) return 1;
-        } else if (op.kind == OP_GRU_TC) {
-            op.gt.Whh = reinterpret_cast<const __half*>(c->warena_h) + f.w_off;
-            op.gt.bhh = c->warena + f.b_off;
-            op.gt.counters = c->gru_counters + (size_t)op.gru_layer * ((c->maxB + 127) / 128);
-        } else if (op.kind == OP_DECONV_LAST) {
-            op.dl.w = c->warena + f.w_off;
-            op.dl.bias = c->warena + f.b_off;
-        } else if (op.kind == OP_SKIP_SMALL) {
-            op.sk.w = c->warena + f.w_off;
-            op.sk.bias = c->warena + f.b_off;
-        } else if (op.kind == OP_GEMM || op.kind == OP_GRU_SEQ) {
-            op.g.W = (c->half && op.g.a_half) ? static_cast<const void*>(reinterpret_cast<const unsigned short*>(c->warena_h) + f.w_off)
-                                              : static_cast<const void*>(c->warena + f.w_off);
-            op.g.bias = c->warena + f.b_off;
-            op.g.koff = c->karena + f.k_off;
-            if (f.w2_off != NONE) {
-                op.g.W2 = c->warena + f.w2_off;
-                op.g.bias2 = c->warena + f.b2_off;
-            }
-            // TMA delivery where every k-block of the gather is 64 contiguous channels of one (frame, bin) tap
-            if (op.kind == OP_GEMM && c->use_tma && op.tma_C > 0 && op.tma_C % 64 == 0 && op.g.a_half) {
-                GemmParams probe = op.g;
-                probe.M = op.rows_per_stream;
-                const int nkb = op.g.K / 64;
-                std::vector<int> kc(4 * nkb, 0);
-                bool ok = gemm_tma_supported(probe) && op.g.Fo * op.g.Tn == op.rows_per_stream;
-                for (int kb = 0; kb < nkb && ok; ++kb) {
-                    const int e = c->khost[f.k_off + 8 * kb];
-                    for (int j = 1; j < 8; ++j) ok = ok && c->khost[f.k_off + 8 * kb + j] == e + 8 * j;
-                    kc[4 * kb + 2] = (int)(e / op.tma_sT);
-                    const int rem = (int)(e % op.tma_sT);
-                    kc[4 * kb + 1] = rem / op.tma_C;
-                    kc[4 * kb] = rem % op.tma_C;
-                    ok = ok && kc[4 * kb] % 64 == 0;
-                }
-                // weights beyond the real K are zero, but their k-blocks must still address valid channels: the padding
-                // units of the koff table point at offset 0 (frame 0, bin 0, channel 0), which the loop above maps there
-                if (ok) {
-                    int* kdev = nullptr;
-                    if (dev_alloc(c, &kdev, kc.size())) return 1;
-                    SE_CUDA_OK(cudaMemcpy(kdev, kc.data(), kc.size() * sizeof(int), cudaMemcpyHostToDevice));
-                    if (make_gemm_tma(&op.tma, op.tma_base, op.tma_C, op.tma_Fp, op.tma_Tp, op.tma_sT, op.tma_sB, c->maxB,
-                                      op.g.Fo, op.tma_fstep, op.g.Tn, op.g.W, op.g.K, op.g.Npad, gemm_tma_tile_n(op.g)))
-                        return 1;
-                    op.tma.t_org = op.tma_t_org;
-                    op.tma.f_org = op.tma_f_org;
-                    op.tma.kcoord = reinterpret_cast<const int4*>(kdev);
-                    op.tma_ok = true;
-                }
-            }
-        } else if (op.kind == OP_PRECONV3) {
-            for (int l = 0; l < 3; ++l) op.p3.w[l] = c->warena + c->pre3_w_off[l];
-        } else if (op.kind == OP_SKIP_BLEND) {
-            op.sb.w = reinterpret_cast<const __half*>(c->warena_h) + f.w_off;
-            op.sb.bias = c->warena + f.b_off;
-            op.sb.nw = c->warena + f.nw_off;
-            op.sb.nb = c->warena + f.nb_off;
-            op.sb.nwr = c->warena + f.nwr_off;
-            op.sb.nbr = c->warena + f.nbr_off;
-            if (make_skip_blend_maps(&op.sb, op.tma_base, op.tma_C, op.tma_Fp, op.tma_Tp, op.tma_sT, op.tma_sB, c->maxB))
-                return 1;
-        } else if (op.kind == OP_DEC_MMA) {
-            op.dm.w = c->warena + f.w_off;
-            op.dm.bias = c->warena + f.b_off;
-            op.dm.w2 = c->warena + f.w2_off;
-            op.dm.bias2 = c->warena + f.b2_off;
-            op.dm.nw = c->warena + f.nw_off;
-            op.dm.nb = c->warena + f.nb_off;
-            op.dm.nwr = c->warena + f.nwr_off;
-            op.dm.nbr = c->warena + f.nbr_off;
-        } else if (op.kind == OP_ENC_MMA || op.kind == OP_ENC_TC) {
-            if (op.kind == OP_ENC_TC) {
-                op.em.w1c = reinterpret_cast<const __half*>(c->warena_h) + f.nwr_off;
-                op.em.w2c = reinterpret_cast<const __half*>(c->warena_h) + f.nbr_off;
-            }
-            op.em.w = c->warena + f.w_off;
-            op.em.bias = c->warena + f.b_off;
-            op.em.w2 = c->warena + f.w2_off;
-            op.em.bias2 = c->warena + f.b2_off;
-            op.em.nw = c->warena + f.nw_off;
-            op.em.nb = c->warena + f.nb_off;
-        } else if (op.kind == OP_PRECONV_TC) {
-            op.pt.w = c->warena + f.nw_off;
-        } else if (op.kind == OP_PRECONV) {
-            op.pc.w = c->warena + f.nw_off;
-        } else if (op.kind == OP_NORM) {
-            op.n.w = c->warena + f.nw_off;
-            op.n.b = c->warena + f.nb_off;
-            if (f.nwr_off != NONE) {
-                op.n.wr = c->warena + f.nwr_off;
-                op.n.br = c->warena + f.nbr_off;
-            }
-        }
-    }
-    c->w_last = c->warena + wl_off;
-    c->b_last = c->warena + bl_off;
 
     // ---- state tables -------------------------------------------------------------------------------------------
     auto add_state = [&](float* base, long long sB, long long src, int count) {
@@ -2103,33 +1977,14 @@ int count_launches(const se_ctx* c) {
 int run_stream_step(se_ctx* c, const IoDesc& io, int B, cudaStream_t st) {
     if (launch_set_io(c->io_dev, io, st)) return 1;
     if (!c->use_graph) return enqueue_stream_step(c, B, st);
-    auto it = c->graphs.find(B);
-    if (it == c->graphs.end()) {
-        // capture on a private stream so that the caller's stream is not put into capture mode
-        if (!c->own_stream) SE_CUDA_OK(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
-        cudaGraph_t graph = nullptr;
-        SE_CUDA_OK(cudaStreamBeginCapture(c->own_stream, cudaStreamCaptureModeThreadLocal));
-        const int rc = enqueue_stream_step(c, B, c->own_stream);
-        cudaError_t e = cudaStreamEndCapture(c->own_stream, &graph);
-        if (rc) {
-            if (graph) cudaGraphDestroy(graph);
-            return 1;
-        }
-        SE_CUDA_OK(e);
-        cudaGraphExec_t exec = nullptr;
-        SE_CUDA_OK(cudaGraphInstantiate(&exec, graph, 0));
-        SE_CUDA_OK(cudaGraphDestroy(graph));
-        it = c->graphs.emplace(B, exec).first;
-    }
-    SE_CUDA_OK(cudaGraphLaunch(it->second, st));
-    return 0;
+    return replay_graph(c->graphs, &c->own_stream, B, [=](cudaStream_t s) { return enqueue_stream_step(c, B, s); }, st);
 }
 
 int check_ready(se_ctx* c, int B, bool want_train = false) {
     SE_REQUIRE(c != nullptr, "null context");
     SE_REQUIRE(c->train == want_train, want_train ? "this entry point needs a context created with training = 1"
                                                   : "training context: use the se_crn_train_* entry points");
-    SE_REQUIRE(c->weights_bound, "se_crn_bind_weights has not been called");
+    SE_REQUIRE(c->wa.bound, "se_crn_bind_weights has not been called");
     SE_REQUIRE(B >= 0 && B <= c->maxB, "B exceeds max_streams of the context");
     SE_CUDA_OK(cudaSetDevice(c->device));
     return 0;
@@ -2366,7 +2221,7 @@ int inject_tap(const se_ctx* c, const float* const* dtaps, int k, float* s, int 
 }
 
 float* garena_of(const se_ctx* c, const void* w) {
-    return c->garena + (reinterpret_cast<const float*>(w) - c->warena);
+    return c->garena + (reinterpret_cast<const float*>(w) - c->wa.w);
 }
 
 // weight + data gradient of one forward GEMM op.  G: d loss / d (pre-activation output), rows addressed by `gs`.
@@ -2426,7 +2281,7 @@ int train_backward(se_ctx* c, const float* dpred, const float* const* dtaps, flo
     SE_REQUIRE(c->t_have_fwd, "se_crn_train_backward: no forward pass to differentiate");
     const int nb = c->t_nb, N = c->t_N, Bp = N * nb, H = c->H, L = c->L, feat = c->feat;
     c->t_wgrad = grad_flat != nullptr;
-    SE_CUDA_OK(cudaMemsetAsync(c->garena, 0, c->warena_floats * sizeof(float), st));
+    SE_CUDA_OK(cudaMemsetAsync(c->garena, 0, c->wa.floats * sizeof(float), st));
     for (auto& tw : c->twins) SE_CUDA_OK(cudaMemsetAsync(tw.first, 0, tw.second, st));
     float *s0 = c->sc[0], *s1 = c->sc[1], *s2 = c->sc[2], *s3 = c->sc[3];
 
@@ -2659,7 +2514,7 @@ int train_backward(se_ctx* c, const float* dpred, const float* const* dtaps, flo
     if (grad_flat == nullptr) return 0;
     // ---- packed-arena gradients -> flat vector in the reference layout (registry order) --------------------------------
     SE_CUDA_OK(cudaMemsetAsync(grad_flat, 0, (size_t)c->n_theta * sizeof(float), st));
-    return launch_arena_scatter_add(c->garena, c->wmap, grad_flat, (long long)c->warena_floats, st);
+    return launch_arena_scatter_add(c->garena, c->wmap, grad_flat, (long long)c->wa.floats, st);
 }
 
 }  // namespace
@@ -2678,16 +2533,7 @@ int se_ctx_create(se_ctx** out, int device, const se_crn_config* cfg) {
         return 2;
     }
     *out = nullptr;
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) {
-        set_error("se_ctx_create: no CUDA device (this library has no CPU fallback)");
-        return 3;
-    }
-    SE_REQUIRE(device >= 0 && device < n, "se_ctx_create: bad device index");
-    SE_CUDA_OK(cudaSetDevice(device));
-    cudaDeviceProp prop;
-    SE_CUDA_OK(cudaGetDeviceProperties(&prop, device));
-    SE_REQUIRE(prop.major == 10, "se_ctx_create: kernels are built for sm_100a (Blackwell B200) only");
+    if (const int rc = check_create_device(device, "se_ctx_create")) return rc;
     se_ctx* c = new se_ctx();
     c->cfg = *cfg;
     c->device = device;
@@ -2715,38 +2561,18 @@ int se_ctx_destroy(se_ctx* c) {
     return 0;
 }
 
-int se_crn_num_params(const se_ctx* c) { return c ? (int)c->params.size() : 0; }
+int se_crn_num_params(const se_ctx* c) { return c ? (int)c->wa.params.size() : 0; }
 const char* se_crn_param_name(const se_ctx* c, int i) {
-    return (c && i >= 0 && i < (int)c->params.size()) ? c->params[i].name.c_str() : nullptr;
+    return (c && i >= 0 && i < (int)c->wa.params.size()) ? c->wa.params[i].name.c_str() : nullptr;
 }
 int64_t se_crn_param_numel(const se_ctx* c, int i) {
-    return (c && i >= 0 && i < (int)c->params.size()) ? c->params[i].numel() : -1;
+    return (c && i >= 0 && i < (int)c->wa.params.size()) ? c->wa.params[i].numel() : -1;
 }
 
 int se_crn_bind_weights(se_ctx* c, const float* const* ptrs, int n, void* stream) {
     SE_REQUIRE(c != nullptr && ptrs != nullptr, "se_crn_bind_weights: null argument");
-    SE_REQUIRE(n == (int)c->params.size(), "se_crn_bind_weights: wrong number of tensors");
     SE_CUDA_OK(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    SE_CUDA_OK(cudaStreamSynchronize(st));
-    HostParams hp;
-    for (int i = 0; i < n; ++i) {
-        SE_REQUIRE(ptrs[i] != nullptr, "se_crn_bind_weights: null tensor " + c->params[i].name);
-        std::vector<float> v((size_t)c->params[i].numel());
-        SE_CUDA_OK(cudaMemcpy(v.data(), ptrs[i], v.size() * sizeof(float), cudaMemcpyDefault));
-        hp.emplace(c->params[i].name, std::move(v));
-    }
-    std::vector<float> arena(c->warena_floats, 0.f);
-    for (const PackFn& f : c->packers) f(hp, arena.data());
-    SE_CUDA_OK(cudaDeviceSynchronize());  // no step may still read the old weights
-    SE_CUDA_OK(cudaMemcpy(c->warena, arena.data(), arena.size() * sizeof(float), cudaMemcpyHostToDevice));
-    if (c->half) {  // fp16 copy of the whole arena (same indexing): the GEMM weight operands are read from it
-        std::vector<__half> ah(arena.size());
-        for (size_t i = 0; i < arena.size(); ++i) ah[i] = __float2half_rn(arena[i]);
-        SE_CUDA_OK(cudaMemcpy(c->warena_h, ah.data(), ah.size() * sizeof(__half), cudaMemcpyHostToDevice));
-    }
-    c->weights_bound = true;
-    return 0;
+    return c->wa.upload(ptrs, n, (cudaStream_t)stream, "se_crn_bind_weights");
 }
 
 int se_crn_state_reset(se_ctx* c, int first, int count, void* stream) {
@@ -3139,8 +2965,8 @@ int se_crn_bind_weights_flat(se_ctx* c, const float* theta, void* stream) {
     SE_REQUIRE(c != nullptr && theta != nullptr, "se_crn_bind_weights_flat: null argument");
     SE_REQUIRE(c->train, "se_crn_bind_weights_flat needs a context created with training = 1");
     SE_CUDA_OK(cudaSetDevice(c->device));
-    if (launch_arena_gather(c->warena, c->wmap, theta, (long long)c->warena_floats, (cudaStream_t)stream)) return 1;
-    c->weights_bound = true;
+    if (launch_arena_gather(c->wa.w, c->wmap, theta, (long long)c->wa.floats, (cudaStream_t)stream)) return 1;
+    c->wa.bound = true;
     return 0;
 }
 
@@ -3226,11 +3052,7 @@ int se_crn_kernel_info(const se_ctx* c, int index, char* name, int name_cap, dou
         fl = op.alg_flops;
         by = op.alg_bytes;
         stg = op.stage;
-        // the op table counts 4 bytes per element; in fp16 operand mode the tensors of the encoder / decoder / Linear+GLN
-        // ops really are 2 bytes wide (the GRU projections keep their fp32 gi stream, the last deconv its fp32 output)
-        if (c->half && op.kind != OP_PRECONV_TC && op.kind != OP_PRECONV && op.kind != OP_GRU_TC && op.kind != OP_GRU_WAVE &&
-            op.label.find("input_proj") == std::string::npos && op.label.find("step") == std::string::npos)
-            by *= op.kind == OP_DECONV_LAST ? 0.75 : 0.5;
+        if (c->half) by *= op.f16_bytes;
     } else if (index == n + 1) {
         label = "mask+istft+ola";
         by = 4.0 * (2 * 2 * NBIN * T + PHOP + 2 * PHOP);

@@ -33,21 +33,11 @@ constexpr int KCHUNK = 3200;         // samples per chunk (config.yaml:172 segme
 constexpr int PHOP = KCHUNK / 2;     // samples a streaming step returns
 inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
-struct FsnParam {
-    std::string name;
-    std::vector<int> shape;
-    int64_t numel() const {
-        int64_t n = 1;
-        for (int s : shape) n *= s;
-        return n;
-    }
-};
-using HostParams = std::map<std::string, std::vector<float>>;
-
-struct FsnOp {
-    int kind;  // 0 gemm, 1..n elementwise kernels (see enqueue)
+struct FsnGemm {
     GemmParams g;
     int rows_per_stream;
+    bool tma_ok = false;  // TMA descriptors (fp16 LSTM steps) in `tma`
+    GemmTma tma{};
 };
 
 }  // namespace
@@ -60,34 +50,22 @@ struct se_fsn {
     int Ks = 0;                                // sub-band input size (32)
     long long recF = 0, recS = 0;              // record strides (floats)
     long long f_h0 = 0, f_h1 = 0, s_h0 = 0, s_h1 = 0;  // offsets of the h histories inside a record
-    std::vector<FsnParam> params;
+    WeightArena wa;  // packed weights, their koff tables and the parameter registry
     std::vector<void*> allocs;
     float *fbrec = nullptr, *sbrec = nullptr, *fbc = nullptr, *sbc = nullptr, *fbout = nullptr, *pline = nullptr;
     float *crm = nullptr;  // [B*F][T][2]
     double* sums = nullptr;      // [B][4]: sum |X|, weighted sum of the unfolded mic-0 magnitude, (sum, sumsq) of fb_out
     float* cstate = nullptr;     // [B][4]: running mean fb, running mean sb, inv fb, inv sb
     int* cstep = nullptr;        // [B][2]
-    float* warena = nullptr;
-    size_t warena_floats = 0;
     // SE_PRECISION_FP16: the sub-band records (x_t and the h histories, 98.7 % of the FLOPs read them) and the sub-band
     // weights are stored as fp16 (tcgen05 kind::f16, fp32 accumulate; cell state c and all statistics stay fp32)
     bool half = false;
     bool split = false;  // SE_PRECISION_3XTF32: every GEMM in the 3xTF32 form (fp32-accurate products, exact cells)
     bool wide_tiles = true;  // 256-column LSTM tiles where the hidden size allows (SE_B200_FSN_WIDE=0: 128-column tiles)
+    bool use_tma = true;     // TMA operand delivery of the fp16 LSTM steps (SE_B200_FSN_TMA=0: cp.async gather)
     int sesz = 4;   // element size of the sub-band records
     int Ksp = 0;    // sub-band input size padded to whole k-blocks (32 floats / 64 halves)
-    void* warena_h = nullptr;
-    std::vector<int> g_half;  // per gemm: operands are fp16
-    std::vector<GemmTma> g_tma;  // per gemm: TMA descriptors (fp16 LSTM steps), valid where g_tma_ok
-    std::vector<int> g_tma_ok;
-    int* karena = nullptr;
-    std::vector<int> khost;
-    std::vector<std::function<void(const HostParams&, float*)>> packers;
-    std::vector<GemmParams> gemms;   // in launch order, interleaved with the elementwise kernels by enqueue()
-    std::vector<size_t> g_w, g_b;
-    std::vector<int> g_k;
-    std::vector<int> g_rows;
-    bool weights_bound = false;
+    std::vector<FsnGemm> gemms;  // in launch order, interleaved with the elementwise kernels by enqueue()
     std::map<int, cudaGraphExec_t> graphs;
     cudaStream_t own_stream = nullptr;
     // scratch of se_fsn_realtime_process (grown on demand; see there for which buffer scales with what)
@@ -107,31 +85,9 @@ struct se_fsn {
     const float* cur_x = nullptr;  // indirection cell for graph replay
     const float** x_cell = nullptr;
     float** out_cell = nullptr;
-
-    size_t reserve_w(size_t n) {
-        size_t off = warena_floats;
-        warena_floats += (n + 3) / 4 * 4;
-        return off;
-    }
-    int reserve_k(const std::vector<int>& v) {
-        int off = (int)khost.size();
-        khost.insert(khost.end(), v.begin(), v.end());
-        while ((khost.size() - off) % 8) khost.push_back(0);
-        return off;
-    }
 };
 
 namespace {
-
-template <typename Tp>
-int dev_alloc(se_fsn* c, Tp** out, size_t count) {
-    void* p = nullptr;
-    SE_CUDA_OK(cudaMalloc(&p, count * sizeof(Tp)));
-    SE_CUDA_OK(cudaMemset(p, 0, count * sizeof(Tp)));
-    c->allocs.push_back(p);
-    *out = reinterpret_cast<Tp*>(p);
-    return 0;
-}
 
 // ---------------------------------------------------------------------------------------------------------------
 // elementwise kernels
@@ -321,7 +277,7 @@ __global__ void unfold_kernel(const float* in, float* out, int C, int F, int Tn,
 // program
 // ---------------------------------------------------------------------------------------------------------------
 void register_params(se_fsn* c) {
-    auto add = [&](const std::string& n, std::vector<int> s) { c->params.push_back({n, std::move(s)}); };
+    auto add = [&](const std::string& n, std::vector<int> s) { c->wa.params.push_back({n, std::move(s)}); };
     auto seq = [&](const std::string& p, int in, int H, int out) {
         for (int l = 0; l < 2; ++l) {
             const std::string s = std::to_string(l);
@@ -347,9 +303,9 @@ void build_lstm(se_fsn* c, const std::string& prefix, int layer, int Kin, int Ki
     const int U_tile = (H % 64 == 0 && c->wide_tiles && !c->split) ? 64 : 32;
     const int K = Kin_pad + H;
     const int N = 4 * H;
-    const size_t w_off = c->reserve_w((size_t)N * K), b_off = c->reserve_w(N);
+    const size_t w_off = c->wa.reserve_w((size_t)N * K), b_off = c->wa.reserve_w(N);
     const std::string s = std::to_string(layer);
-    c->packers.push_back([=](const HostParams& hp, float* arena) {
+    c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
         const std::vector<float>& wi = hp.at(prefix + ".sequence_model.weight_ih_l" + s);
         const std::vector<float>& wh = hp.at(prefix + ".sequence_model.weight_hh_l" + s);
         const std::vector<float>& bi = hp.at(prefix + ".sequence_model.bias_ih_l" + s);
@@ -387,12 +343,44 @@ void build_lstm(se_fsn* c, const std::string& prefix, int layer, int Kin, int Ki
         g.o2B = H;
         g.c_rows = (long long)c->maxB * rows_per_stream;
         g.H = H;
-        c->gemms.push_back(g);
-        c->g_w.push_back(w_off);
-        c->g_b.push_back(b_off);
-        c->g_k.push_back(c->reserve_k(koff));
-        c->g_rows.push_back(rows_per_stream);
-        c->g_half.push_back(half ? 1 : 0);
+        const int k_off = c->wa.reserve_k(koff);
+        const size_t i = c->gemms.size();
+        c->gemms.push_back({g, rows_per_stream});
+        c->wa.binds.push_back([=] {
+            FsnGemm& e = c->gemms[i];
+            e.g.W = half ? static_cast<const void*>(c->wa.wh + w_off) : static_cast<const void*>(c->wa.w + w_off);
+            e.g.bias = c->wa.w + b_off;
+            e.g.koff = c->wa.k + k_off;
+            // fp16 LSTM steps of the sub-band model: TMA operand delivery + CTA pairs (gemm_tc.cu).  A row of the GEMM is
+            // one (stream, bin) sequence record; every 64-wide k-block of [x_t | h_{t-1}] is contiguous inside the record,
+            // so the A tile of a k-block is ONE 2-D box (64 halves at the block's offset x 128 consecutive records).
+            if (!(c->use_tma && half && e.g.sB % 64 == 0)) return 0;
+            GemmParams probe = e.g;
+            probe.M = rows_per_stream;
+            if (!gemm_tma_supported(probe)) return 0;
+            const int nkb = K / 64;
+            std::vector<int> kc(4 * nkb, 0);
+            bool ok = true;
+            for (int kb = 0; kb < nkb && ok; ++kb) {
+                const int u = c->wa.khost[k_off + 8 * kb];
+                for (int j = 1; j < 8; ++j) ok = ok && c->wa.khost[k_off + 8 * kb + j] == u + 8 * j;
+                ok = ok && u % 8 == 0;
+                kc[4 * kb] = u;
+            }
+            if (!ok) return 0;
+            int* kdev = nullptr;
+            if (dev_alloc(c, &kdev, kc.size())) return 1;
+            SE_CUDA_OK(cudaMemcpy(kdev, kc.data(), kc.size() * sizeof(int), cudaMemcpyHostToDevice));
+            const int nrows = c->maxB * rows_per_stream;
+            if (make_gemm_tma(&e.tma, e.g.A, (int)e.g.sB, 1, 1, e.g.sB, e.g.sB, nrows, 1, 1, 1, e.g.W, e.g.K, e.g.Npad,
+                              gemm_tma_tile_n(e.g)))
+                return 1;
+            e.tma.t_org = 0;
+            e.tma.f_org = 0;
+            e.tma.kcoord = reinterpret_cast<const int4*>(kdev);
+            e.tma_ok = true;
+            return 0;
+        });
     }
 }
 
@@ -401,8 +389,8 @@ void build_fc(se_fsn* c, const std::string& prefix, int H, int N, float* rec, lo
     const int U = half ? 8 : 4;
     const int esz = half ? 2 : 4;
     const int Npad = round_up(N, gemm_tf32_tile_n(N));
-    const size_t w_off = c->reserve_w((size_t)Npad * H), b_off = c->reserve_w(Npad);
-    c->packers.push_back([=](const HostParams& hp, float* arena) {
+    const size_t w_off = c->wa.reserve_w((size_t)Npad * H), b_off = c->wa.reserve_w(Npad);
+    c->wa.packers.push_back([=](const HostParams& hp, float* arena) {
         const std::vector<float>& w = hp.at(prefix + ".fc_output_layer.weight");
         const std::vector<float>& b = hp.at(prefix + ".fc_output_layer.bias");
         for (int n = 0; n < N; ++n) {
@@ -428,12 +416,16 @@ void build_fc(se_fsn* c, const std::string& prefix, int H, int N, float* rec, lo
     g.oT = oT;
     g.vec4 = vec4;
     g.stats = stats;
-    c->gemms.push_back(g);
-    c->g_w.push_back(w_off);
-    c->g_b.push_back(b_off);
-    c->g_k.push_back(c->reserve_k(koff));
-    c->g_rows.push_back(rows_per_stream_T);
-    c->g_half.push_back(half ? 1 : 0);
+    const int k_off = c->wa.reserve_k(koff);
+    const size_t i = c->gemms.size();
+    c->gemms.push_back({g, rows_per_stream_T});
+    c->wa.binds.push_back([=] {
+        GemmParams& e = c->gemms[i].g;
+        e.W = half ? static_cast<const void*>(c->wa.wh + w_off) : static_cast<const void*>(c->wa.w + w_off);
+        e.bias = c->wa.w + b_off;
+        e.koff = c->wa.k + k_off;
+        return 0;
+    });
 }
 
 int build(se_fsn* c) {
@@ -460,6 +452,7 @@ int build(se_fsn* c) {
     c->half = g.precision == SE_PRECISION_FP16;
     c->split = g.precision == SE_PRECISION_3XTF32;
     if (const char* e = getenv("SE_B200_FSN_WIDE")) c->wide_tiles = atoi(e) != 0;
+    if (const char* e = getenv("SE_B200_FSN_TMA")) c->use_tma = atoi(e) != 0;
     c->sesz = c->half ? 2 : 4;
     SE_REQUIRE(round_up(c->Ks, 32) == c->Ks, "FullSubNet: sub-band input size must be a multiple of 32 (31 neighbours + 1)");
     c->Ksp = round_up(c->Ks, c->half ? 64 : 32);
@@ -524,56 +517,16 @@ int build(se_fsn* c) {
                c->sbc + (size_t)B * F * Hs, F, c->half);
     build_fc(c, "sb_model", Hs, 2, c->sbrec, recS, sh1, EPI_BIAS, c->crm, 2LL * T, 2, 0, nullptr, F * T, c->half);
 
-    if (dev_alloc(c, &c->warena, c->warena_floats)) return 1;
-    if (c->half && dev_alloc(c, reinterpret_cast<char**>(&c->warena_h), c->warena_floats * 2)) return 1;
-    if (dev_alloc(c, &c->karena, c->khost.size())) return 1;
-    SE_CUDA_OK(cudaMemcpy(c->karena, c->khost.data(), c->khost.size() * sizeof(int), cudaMemcpyHostToDevice));
-    if (init_fft_tables()) return 1;  // se_fsn_realtime_process frames and transforms on this device
-    c->g_tma.resize(c->gemms.size());
-    c->g_tma_ok.assign(c->gemms.size(), 0);
-    bool use_tma = true;
-    if (const char* e = getenv("SE_B200_FSN_TMA")) use_tma = atoi(e) != 0;
-    for (size_t i = 0; i < c->gemms.size(); ++i) {
-        c->gemms[i].W = c->g_half[i] ? static_cast<const void*>(reinterpret_cast<const __half*>(c->warena_h) + c->g_w[i])
-                                     : static_cast<const void*>(c->warena + c->g_w[i]);
-        c->gemms[i].bias = c->warena + c->g_b[i];
-        c->gemms[i].koff = c->karena + c->g_k[i];
-        // fp16 LSTM steps of the sub-band model: TMA operand delivery + CTA pairs (gemm_tc.cu).  A row of the GEMM is one
-        // (stream, bin) sequence record; every 64-wide k-block of [x_t | h_{t-1}] is contiguous inside the record, so the
-        // A tile of a k-block is ONE 2-D box (64 halves at the block's offset x 128 consecutive records).
-        const GemmParams& g = c->gemms[i];
-        if (!(use_tma && c->g_half[i] && g.epi == EPI_LSTM && g.sB % 64 == 0)) continue;
-        GemmParams probe = g;
-        probe.M = c->g_rows[i];
-        if (!gemm_tma_supported(probe)) continue;
-        const int nkb = g.K / 64;
-        std::vector<int> kc(4 * nkb, 0);
-        bool ok = true;
-        for (int kb = 0; kb < nkb && ok; ++kb) {
-            const int e = c->khost[c->g_k[i] + 8 * kb];
-            for (int j = 1; j < 8; ++j) ok = ok && c->khost[c->g_k[i] + 8 * kb + j] == e + 8 * j;
-            ok = ok && e % 8 == 0;
-            kc[4 * kb] = e;
-        }
-        if (!ok) continue;
-        int* kdev = nullptr;
-        if (dev_alloc(c, &kdev, kc.size())) return 1;
-        SE_CUDA_OK(cudaMemcpy(kdev, kc.data(), kc.size() * sizeof(int), cudaMemcpyHostToDevice));
-        const int nrows = c->maxB * c->g_rows[i];
-        if (make_gemm_tma(&c->g_tma[i], g.A, (int)g.sB, 1, 1, g.sB, g.sB, nrows, 1, 1, 1, g.W, g.K, g.Npad, gemm_tma_tile_n(g)))
-            return 1;
-        c->g_tma[i].t_org = 0;
-        c->g_tma[i].f_org = 0;
-        c->g_tma[i].kcoord = reinterpret_cast<const int4*>(kdev);
-        c->g_tma_ok[i] = 1;
-    }
-    return 0;
+    c->wa.half = c->half;
+    if (c->wa.allocate(c->allocs)) return 1;
+    return init_fft_tables();  // se_fsn_realtime_process frames and transforms on this device
 }
 
 int run_gemm(se_fsn* c, int i, int B, cudaStream_t st) {
-    GemmParams g = c->gemms[i];
-    g.M = B * c->g_rows[i];
-    if (c->g_tma_ok[i]) return launch_gemm_tma(g, c->g_tma[i], st);
+    const FsnGemm& e = c->gemms[i];
+    GemmParams g = e.g;
+    g.M = B * e.rows_per_stream;
+    if (e.tma_ok) return launch_gemm_tma(g, e.tma, st);
     return launch_gemm_tf32(g, st, c->split);
 }
 
@@ -601,8 +554,8 @@ int phase_fullband(se_fsn* c, int B, cudaStream_t st) {  // scale, reflect-padde
     for (int i = 0; i < 2 * T; ++i)
         if (run_gemm(c, gi++, B, st)) return 1;
     {  // fb fc + ReLU; its statistics slot is sums[b][2..3]
-        GemmParams g = c->gemms[gi];
-        g.M = B * c->g_rows[gi];
+        GemmParams g = c->gemms[gi].g;
+        g.M = B * c->gemms[gi].rows_per_stream;
         g.stats = c->sums + 2;
         g.stats_stride = 4;  // sums holds 4 doubles per stream
         if (launch_gemm_tf32(g, st, c->split)) return 1;
@@ -685,32 +638,9 @@ int enqueue_step(se_fsn* c, int B, cudaStream_t st) {
     return launch_mask_istft(mp, st);
 }
 
-// replays enq(c, B) from `graphs`, capturing it first on the context's private stream (so that the caller's stream is
-// never put into capture mode)
-int run_graph(se_fsn* c, std::map<int, cudaGraphExec_t>& graphs, int (*enq)(se_fsn*, int, cudaStream_t), int B,
-              cudaStream_t st) {
-    auto it = graphs.find(B);
-    if (it == graphs.end()) {
-        if (!c->own_stream) SE_CUDA_OK(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
-        cudaGraph_t graph = nullptr;
-        SE_CUDA_OK(cudaStreamBeginCapture(c->own_stream, cudaStreamCaptureModeThreadLocal));
-        const int rc = enq(c, B, c->own_stream);
-        cudaError_t e = cudaStreamEndCapture(c->own_stream, &graph);
-        if (rc) {
-            if (graph) cudaGraphDestroy(graph);
-            return 1;
-        }
-        SE_CUDA_OK(e);
-        cudaGraphExec_t exec = nullptr;
-        SE_CUDA_OK(cudaGraphInstantiate(&exec, graph, 0));
-        SE_CUDA_OK(cudaGraphDestroy(graph));
-        it = graphs.emplace(B, exec).first;
-    }
-    SE_CUDA_OK(cudaGraphLaunch(it->second, st));
-    return 0;
+int run_chunk_graph(se_fsn* c, int B, cudaStream_t st) {
+    return replay_graph(c->graphs, &c->own_stream, B, [=](cudaStream_t s) { return enqueue(c, B, s); }, st);
 }
-
-int run_chunk_graph(se_fsn* c, int B, cudaStream_t st) { return run_graph(c, c->graphs, enqueue, B, st); }
 
 template <typename Tp>
 int regrow(se_fsn* c, Tp** buf, size_t count) {  // scratch: freed and re-allocated larger (registered for destroy)
@@ -733,16 +663,7 @@ int se_fsn_create(se_fsn** out, int device, const se_fsn_config* cfg) {
         return 2;
     }
     *out = nullptr;
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) {
-        set_error("se_fsn_create: no CUDA device (this library has no CPU fallback)");
-        return 3;
-    }
-    SE_REQUIRE(device >= 0 && device < n, "se_fsn_create: bad device index");
-    SE_CUDA_OK(cudaSetDevice(device));
-    cudaDeviceProp prop;
-    SE_CUDA_OK(cudaGetDeviceProperties(&prop, device));
-    SE_REQUIRE(prop.major == 10, "se_fsn_create: kernels are built for sm_100a (Blackwell B200) only");
+    if (const int rc = check_create_device(device, "se_fsn_create")) return rc;
     se_fsn* c = new se_fsn();
     c->cfg = *cfg;
     c->device = device;
@@ -766,37 +687,18 @@ int se_fsn_destroy(se_fsn* c) {
     return 0;
 }
 
-int se_fsn_num_params(const se_fsn* c) { return c ? (int)c->params.size() : 0; }
+int se_fsn_num_params(const se_fsn* c) { return c ? (int)c->wa.params.size() : 0; }
 const char* se_fsn_param_name(const se_fsn* c, int i) {
-    return (c && i >= 0 && i < (int)c->params.size()) ? c->params[i].name.c_str() : nullptr;
+    return (c && i >= 0 && i < (int)c->wa.params.size()) ? c->wa.params[i].name.c_str() : nullptr;
 }
 int64_t se_fsn_param_numel(const se_fsn* c, int i) {
-    return (c && i >= 0 && i < (int)c->params.size()) ? c->params[i].numel() : -1;
+    return (c && i >= 0 && i < (int)c->wa.params.size()) ? c->wa.params[i].numel() : -1;
 }
 
 int se_fsn_bind_weights(se_fsn* c, const float* const* ptrs, int n, void* stream) {
     SE_REQUIRE(c != nullptr && ptrs != nullptr, "se_fsn_bind_weights: null argument");
-    SE_REQUIRE(n == (int)c->params.size(), "se_fsn_bind_weights: wrong number of tensors");
     SE_CUDA_OK(cudaSetDevice(c->device));
-    SE_CUDA_OK(cudaStreamSynchronize((cudaStream_t)stream));
-    HostParams hp;
-    for (int i = 0; i < n; ++i) {
-        SE_REQUIRE(ptrs[i] != nullptr, "se_fsn_bind_weights: null tensor " + c->params[i].name);
-        std::vector<float> v((size_t)c->params[i].numel());
-        SE_CUDA_OK(cudaMemcpy(v.data(), ptrs[i], v.size() * sizeof(float), cudaMemcpyDefault));
-        hp.emplace(c->params[i].name, std::move(v));
-    }
-    std::vector<float> arena(c->warena_floats, 0.f);
-    for (auto& f : c->packers) f(hp, arena.data());
-    SE_CUDA_OK(cudaDeviceSynchronize());
-    SE_CUDA_OK(cudaMemcpy(c->warena, arena.data(), arena.size() * sizeof(float), cudaMemcpyHostToDevice));
-    if (c->half) {  // fp16 copy of the arena (same indexing): the sub-band GEMMs read their weights from it
-        std::vector<__half> ah(arena.size());
-        for (size_t i = 0; i < arena.size(); ++i) ah[i] = __float2half_rn(arena[i]);
-        SE_CUDA_OK(cudaMemcpy(c->warena_h, ah.data(), ah.size() * sizeof(__half), cudaMemcpyHostToDevice));
-    }
-    c->weights_bound = true;
-    return 0;
+    return c->wa.upload(ptrs, n, (cudaStream_t)stream, "se_fsn_bind_weights");
 }
 
 int se_fsn_reset_state(se_fsn* c, int first, int count, void* stream) {
@@ -855,7 +757,7 @@ int se_fsn_state_import(se_fsn* c, const int32_t* rows_host, int n, const void* 
 
 int se_fsn_forward_chunk(se_fsn* c, const float* x, float* out, int B, void* stream) {
     NvtxRange nvtx_range("se.fsn_forward_chunk");
-    SE_REQUIRE(c != nullptr && c->weights_bound, "se_fsn_forward_chunk: context without weights");
+    SE_REQUIRE(c != nullptr && c->wa.bound, "se_fsn_forward_chunk: context without weights");
     SE_REQUIRE(x != nullptr && out != nullptr, "se_fsn_forward_chunk: null buffer");
     SE_REQUIRE(B >= 0 && B <= c->maxB, "se_fsn_forward_chunk: B exceeds max_streams");
     if (B == 0) return 0;
@@ -868,7 +770,7 @@ int se_fsn_forward_chunk(se_fsn* c, const float* x, float* out, int B, void* str
 int se_fsn_process_chunk(se_fsn* c, const float* in, int64_t in_stream_stride, int64_t in_mic_stride, float* out,
                          int64_t out_stream_stride, int B, void* stream) {
     NvtxRange nvtx_range("se.fsn_chunk_step");
-    SE_REQUIRE(c != nullptr && c->weights_bound, "se_fsn_process_chunk: context without weights");
+    SE_REQUIRE(c != nullptr && c->wa.bound, "se_fsn_process_chunk: context without weights");
     SE_REQUIRE(in != nullptr && out != nullptr, "se_fsn_process_chunk: null buffer");
     SE_REQUIRE(B >= 0 && B <= c->maxB, "se_fsn_process_chunk: B exceeds max_streams");
     SE_REQUIRE(c->M <= 3, "se_fsn_process_chunk: the framing kernel serves at most 3 microphones");
@@ -886,13 +788,13 @@ int se_fsn_process_chunk(se_fsn* c, const float* in, int64_t in_stream_stride, i
     }
     IoDesc io{in, in_stream_stride, in_mic_stride, 0, KCHUNK, out, out_stream_stride, PHOP};
     if (launch_set_io(c->st_io, io, st)) return 1;
-    return run_graph(c, c->step_graphs, enqueue_step, B, st);
+    return replay_graph(c->step_graphs, &c->own_stream, B, [=](cudaStream_t s) { return enqueue_step(c, B, s); }, st);
 }
 
 int se_fsn_realtime_process(se_fsn* c, const float* mixture, const float* source, int B, int64_t L, int flag, int train,
                             float* pred, float* crm_out, float* s_out, float* x0_out, void* stream) {
     NvtxRange nvtx_range("se.fsn_realtime_process");
-    SE_REQUIRE(c != nullptr && c->weights_bound, "se_fsn_realtime_process: context without weights");
+    SE_REQUIRE(c != nullptr && c->wa.bound, "se_fsn_realtime_process: context without weights");
     SE_REQUIRE(mixture != nullptr && pred != nullptr && L > 0, "se_fsn_realtime_process: null buffer");
     SE_REQUIRE(B >= 1 && B <= c->maxB, "se_fsn_realtime_process: B exceeds max_streams");
     SE_REQUIRE(c->M <= 3, "se_fsn_realtime_process: the framing kernel serves at most 3 microphones");

@@ -5,7 +5,10 @@
 #include <stdint.h>
 #include <nvtx3/nvToolsExt.h>  // header-only (the tools library is dlopen'ed when a profiler is attached)
 
+#include <functional>
+#include <map>
 #include <string>
+#include <vector>
 
 namespace se {
 
@@ -64,6 +67,71 @@ int num_sms_current_device(int* out);
     do {                                                                               \
         if (se::ensure_dyn_smem(reinterpret_cast<const void*>(kernel), (int)(bytes))) return 1; \
     } while (0)
+
+// ---------------------------------------------------------------------------------------------------------------
+// context plumbing shared by the CRN and FullSubNet contexts (arena.cu)
+// ---------------------------------------------------------------------------------------------------------------
+// zero-filled device buffer of `bytes`, recorded in `allocs` (freed when the owning context is destroyed)
+int dev_alloc_bytes(std::vector<void*>& allocs, void** out, size_t bytes);
+template <typename Owner, typename Tp>
+int dev_alloc(Owner* c, Tp** out, size_t count) {
+    return dev_alloc_bytes(c->allocs, reinterpret_cast<void**>(out), count * sizeof(Tp));
+}
+// the checks of se_*_create before a context is built: 3 = no CUDA device, 2 = bad index or not an sm_100 device,
+// 1 = CUDA error; makes `device` current.  `fn` prefixes the error messages.
+int check_create_device(int device, const char* fn);
+// replays enq(stream) as a CUDA graph captured once per B into `graphs`.  The capture runs on *own (created on first
+// use), so that the caller's stream is never put into capture mode.
+int replay_graph(std::map<int, cudaGraphExec_t>& graphs, cudaStream_t* own, int B,
+                 const std::function<int(cudaStream_t)>& enq, cudaStream_t st);
+
+struct ParamInfo {  // one tensor of the reference model's state_dict
+    std::string name;
+    std::vector<int> shape;
+    int64_t numel() const {
+        int64_t n = 1;
+        for (int s : shape) n *= s;
+        return n;
+    }
+};
+using HostParams = std::map<std::string, std::vector<float>>;
+using PackFn = std::function<void(const HostParams&, float*)>;  // fills a host mirror of the packed-weight arena
+
+// The packed weights of a context.  Building the program reserves regions of the fp32 weight arena (multiples of 4
+// floats, so every region is 16-byte aligned) and of the koff table (gather offsets of 16-byte units), and registers
+// for each region a packer that fills it from the reference parameters.  Each op registers a bind that sets its
+// weight / bias / koff pointers (and builds whatever descriptor depends on them) once allocate() has created the device
+// arenas.  With `half`, an fp16 mirror of the whole weight arena (same indexing) holds the fp16 weight operands.
+struct WeightArena {
+    std::vector<ParamInfo> params;  // registry in the order of the reference state_dict
+    bool half = false;
+    size_t floats = 0;
+    std::vector<int> khost;
+    std::vector<PackFn> packers;
+    std::vector<std::function<int()>> binds;
+    float* w = nullptr;          // device arenas (allocate)
+    __half* wh = nullptr;        // fp16 mirror (half only)
+    int* k = nullptr;
+    bool bound = false;          // weights have been uploaded
+
+    size_t reserve_w(size_t n) {
+        const size_t off = floats;
+        floats += (n + 3) / 4 * 4;
+        return off;
+    }
+    int reserve_k(const std::vector<int>& v) {  // padded with offset-0 units to whole k-blocks of 8 units (weights there: 0)
+        const int off = (int)khost.size();
+        khost.insert(khost.end(), v.begin(), v.end());
+        while ((khost.size() - off) % 8) khost.push_back(0);
+        return off;
+    }
+    std::vector<float> pack(const HostParams& hp) const;  // runs every packer on a zeroed host arena
+    // device arenas, koff upload, then every bind
+    int allocate(std::vector<void*>& allocs);
+    // gathers the `n` tensors of the registry from `ptrs` (host or device), packs them and uploads the arena (and its
+    // fp16 mirror) once no work on `st` or the device still reads the old weights; `fn` prefixes the error messages
+    int upload(const float* const* ptrs, int n, cudaStream_t st, const char* fn);
+};
 
 // ---------------------------------------------------------------------------------------------------------------
 // gathered GEMM:  C[m][n] = sum_k A(m,k) * W[n][k],  m = (b*Tn + t)*Fo + f
